@@ -6,7 +6,7 @@ official approach config (128 steps) + finisher config (36 steps), bundled check
 `build_curriculum_local_eval_suite(seed=700001+5*1009, stage_index=5)`.  One "step" = one full pass of the hot path
 over the suite = 65,536 episodes x 164 env-steps, each with a policy forward.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); episodes shard by index with no data-path collective
 (weak scaling: 65,536 episodes per GPU), one all-reduce of the eval statistics after the timed region.
@@ -48,6 +48,7 @@ ACTOR_FLOPS = 2 * (56 * 64 + 64 * 64 + 64 * 7)   # 16256
 ENV_FLOPS = 1800
 XU_OPS_PER_ENV_STEP = 160     # MUFU-class instructions per env-step of the tensor-core rollout: 128 tanh + 12 sin/cos + ~20 rcp / sqrt / conversions (SASS count)
 THRESHOLD_BAND = 0.01         # parity: an episode is "within tolerance of a threshold" if scaling the decision thresholds by 1 -+ 1 % flips the ORACLE
+DUMP_LIMIT_BYTES = 64_000_000
 
 
 def peaks() -> dict:
@@ -142,6 +143,21 @@ def bench_config(episodes_per_gpu: int, world: int) -> dict:
             "approach_config": "workspace_expansion_dynamic_scale_big", "finisher_config": "dock_workspace_handoff_noop_ft_12env",
             "policies": "bundled approach stage8-11 + finisher checkpoints", "parallelism": f"env-sharded x{world}",
             "l2": "256 MB flush between timed iterations"}
+
+
+def dump_outputs(out_dir: Path, arrays: dict[str, np.ndarray]) -> None:
+    """Per-episode results as ``out_dir/<name>.npy``: float32 stays float32, flags and counters become (exact) float64, so two builds
+    can be compared output for output.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of episodes is written, the same rows
+    of every array; ``episode_index.npy`` holds their indices into the suite."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(arrays["success"])
+    arrays["episode_index"] = np.arange(n, dtype=np.float64)
+    row_bytes = sum(a.nbytes for a in arrays.values()) // n
+    keep = min(n, (DUMP_LIMIT_BYTES - 4096 * len(arrays)) // row_bytes)     # 4 KB per file covers the .npy header
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", a[rows])
 
 
 def cpu_config1(threads_all: int) -> dict:
@@ -408,7 +424,13 @@ def main() -> None:
     ap.add_argument("--skip-step-kernel", action="store_true")
     ap.add_argument("--grad-exchange", default="peer", choices=["peer", "nccl"], help="training leg, N > 1: gradient sum over NVLink peer buffers or NCCL")
     ap.add_argument("--skip-train", action="store_true", help="skip the BASELINE config-5 leg (Stage-10 PPO training, extra key `train`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="write the per-episode results of the last timed step (all ranks' shards) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)
@@ -492,6 +514,12 @@ def main() -> None:
     env_steps = int(out.env_steps.item())
     res = out.to_numpy()
     success = float(res["success"].mean())
+    dumped = res
+    if args.dump_outputs is not None and world > 1:     # the whole suite in episode order: every rank's shard
+        mine = out.raw[:, :n].contiguous()
+        shards = [torch.empty_like(mine) for _ in range(world)]
+        dist.all_gather(shards, mine)
+        dumped = RolloutResult(raw=torch.cat(shards, dim=1), n=n * world, env_steps=out.env_steps).to_numpy()
 
     # ---- end-to-end leg: host buffers, pinned H2D + D2H inside the timed region ----------------------
     pinned = {k: torch.as_tensor(np.ascontiguousarray(getattr(suite, k), dtype=np.float32)).pin_memory() for k in ("initial_q", "goal_q")}
@@ -631,6 +659,8 @@ def main() -> None:
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "success_rate": e2e_success},
             "clocks": clocks.summary(), "gpu_launches": launches, "train": train,
         }
+        if args.dump_outputs is not None:
+            dump_outputs(args.dump_outputs, dumped)
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if world > 1:

@@ -7,16 +7,12 @@ ROOT = Path(__file__).resolve().parents[1]
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
 
-REFERENCE_PKG = Path("/root/reference/hrl_ws/src/hrl_trainer")
-
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the live reference under /root/reference (build container only)")
+    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on a B200 with -m gpu)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = REFERENCE_PKG.exists()
     try:
         import torch
 
@@ -24,8 +20,6 @@ def pytest_collection_modifyitems(config, items):
     except Exception:  # pragma: no cover
         have_gpu = False
     for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
 

@@ -9,10 +9,9 @@ module and in the package namespaces that re-export them -- with this repository
 class (pure reward-function tests) run against the reference's own functions and pass trivially; the ones that step the env exercise
 ``libkin_b200.so``.
 
-It needs a machine with BOTH a B200 and a checkout of the reference.  Neither box of this build has both (the build container has the
-reference and no GPU, the GPU box has no /root/reference, and reference sources must not be copied into the repository), so here it
-is exercised only up to the patching step by ``tests/test_reference_conformance.py``; ``tests/test_gpu_rollout.py::
-test_single_env_adapter_conformance`` restates the env-facing assertions of those files for the GPU box.
+It needs a machine with BOTH a B200 and a checkout of the reference, and reference sources must not be copied into the repository,
+so the test suite does not run it; ``tests/test_gpu_rollout.py::test_single_env_adapter_conformance`` restates the env-facing
+assertions of those files.
 """
 from __future__ import annotations
 
