@@ -68,9 +68,12 @@ __device__ __forceinline__ float norm7(const float* v) {
 
 // ---- FAST flavour (the tensor-core rollout / collection kernels) -----------------------------------------------------
 // Same formulas, cheaper instruction sequences: single-MUFU sqrt / reciprocal (relative error 2^-23, no slow path), a
-// branch-free atan2 (minimax polynomial, |error| < 1e-7 rad), margins from the normalised joint position, and the previous
-// step's pose-error norms carried instead of recomputed.  Differences from the strict flavour are a few ulp (<= 2e-7),
-// far inside the 1e-5 m / 1e-5 rad pose tolerance; the strict kernels (K1, kin_rollout_ffma) do not use it.
+// branch-free atan2 (minimax polynomial, |error| < 5e-7 rad), margins from the normalised joint position, and the previous
+// step's pose-error norms carried instead of recomputed.  Measured FK differences from the strict flavour (B200): with the
+// polynomial sine / cosine (FAST = 1) the same position and Euler angles within 3.2e-7 rad; with the MUFU ones (FAST = 2, the
+// default of the tensor-core rollout) 4.8e-7 m and 8.7e-6 rad (an Euler angle near pitch +-pi/2; 1.4e-6 rad elsewhere on the
+// joint limits) -- inside the 1e-5 m / 1e-5 rad pose tolerance (tests/test_gpu_fast_env_math.py).  The strict kernels (K1,
+// kin_rollout_ffma) do not use it.
 __device__ __forceinline__ float sqrt_approx(float x) {
     float y;
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -90,11 +93,15 @@ template <int FAST>
 __device__ __forceinline__ float norm3_sel(float a, float b, float c) { return sqrt_sel<FAST>(fmaf(a, a, fmaf(b, b, c * c))); }
 
 // atan2 for the Euler extraction: t = min/max in [0, 1], atan(t) = t + t^3 Q(t^2) (Remez fit, max |error| 7.5e-8 in fp32),
-// then the octant / quadrant / sign fixes.  atan2(0, 0) = 0 like the reference's math.atan2.
+// then the octant / quadrant / sign fixes.  |error| < 5e-7 rad (the fit, rcp.approx and the rounding of pi/2 - r, pi - r) for
+// max(|x|, |y|) in [2^-126, 2^126]: the guard of the reciprocal is the smallest normal float, so t is the true ratio for every
+// normal input (rcp.approx flushes a subnormal operand); with both inputs subnormal the octant and sign are still right.
+// atan2(+-0, +0) = +-0 and atan2(+-0, x < 0) = +-pi like math.atan2, but atan2(+-0, -0) = +-0 where math.atan2 gives +-pi:
+// the x < 0 test does not see the sign of a zero.
 __device__ __forceinline__ float atan2_fast(float y, float x) {
     const float ax = fabsf(x), ay = fabsf(y);
     const float mx = fmaxf(ax, ay), mn = fminf(ax, ay);
-    const float t = mn * rcp_approx(fmaxf(mx, 1e-30f));
+    const float t = mn * rcp_approx(fmaxf(mx, 1.17549435e-38f));
     const float s = t * t;
     float p = 0.0026222446467727423f;
     p = fmaf(p, s, -0.015132537111639977f);
@@ -242,6 +249,13 @@ __device__ __forceinline__ void pose_error(const float* curr, const float* goal,
 __device__ __forceinline__ float joint_margin(const KinEnvParams& P, float q, int i) {
     float nearest = fminf(q - P.joint_lower[i], P.joint_upper[i] - q);
     return clampf(2.0f * nearest * P.k_inv_span[i], 0.0f, 1.0f);
+}
+
+// FAST flavour: the normalised joint position 2 (q - lo) / span - 1 of a q inside its limits.  It is >= -1 (q - lo >= 0), but
+// 2 k_inv_span (hi - lo) may round above 1 for limits whose span is not representable (up to 1 + 3e-5 for a short span far from
+// zero): the upper clamp keeps qn <= 1 and so the margin 1 - |qn| >= 0, which the observation relies on without clipping again.
+__device__ __forceinline__ float qnorm(const KinEnvParams& P, float q, int i) {
+    return fminf(fmaf(2.0f * P.k_inv_span[i], q - P.joint_lower[i], -1.0f), 1.0f);
 }
 
 // AKE:432-444 -- thresholds always come from reward_config (ar_*), also in dock mode
@@ -721,7 +735,7 @@ __device__ __forceinline__ void step_core(const KinEnvParams& P, EnvRegs& s, con
         dq_sq = fmaf(dqi, dqi, dq_sq);
         dchg_sq = fmaf(dch, dch, dchg_sq);
         if constexpr (FAST) {   // margin = clip(2 min(q - lo, hi - q) / span, 0, 1) = 1 - |2 (q - lo) / span - 1| for q inside its limits
-            out.qn[i] = fmaf(2.0f * P.k_inv_span[i], qn[i] - P.joint_lower[i], -1.0f);
+            out.qn[i] = qnorm(P, qn[i], i);
             out.margin[i] = 1.0f - fabsf(out.qn[i]);
         } else {
             out.margin[i] = joint_margin(P, qn[i], i);

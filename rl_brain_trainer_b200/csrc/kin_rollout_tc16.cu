@@ -53,34 +53,6 @@ struct Tile16 {
     int step_id;
 };
 
-// Observation of the current state as 18 packed fp16 pairs in X-image column order:
-// dq 0:7 | goal_ori_err 7:10 | goal_pos_err 10:13 | joint_limit_margin 13:20 | prev_action 20:27 | progress 27:29 | q 29:36
-// (observation_builder.py:29-94; values and clamps as kin_core.cuh::build_obs_from).
-__device__ __forceinline__ void obs_pack(const KinEnvParams& P, const EnvRegs& s, const StepOut& so, unsigned* w) {
-    float v[X_DYN];
-#pragma unroll
-    for (int i = 0; i < NJ; ++i) {
-        v[i] = s.dq[i] * P.k_inv_delta_limit[i];
-        v[13 + i] = so.margin[i];
-        v[20 + i] = s.pa[i];
-        v[29 + i] = so.qn[i];
-    }
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        v[7 + k] = so.oe[k] * P.k_inv_ori_err_scale;
-        v[10 + k] = so.pe[k] * P.k_inv_pos_err_scale;
-    }
-    v[27] = (float)s.step * P.k_inv_episode_length;
-    v[28] = (float)s.dwell * P.k_inv_dwell_steps_target;
-#pragma unroll
-    for (int i = 0; i < X_DYN / 2; ++i) w[i] = pack_h2(v[2 * i], v[2 * i + 1]);
-    // margins (columns 14..19) and normalised q (30..35) are inside [0, 1] / [-1, 1] by construction (q is clipped to its limits);
-    // everything else gets the reference's clip to [-1, 1] (progress is non-negative, its clip to [0, 1] is the same upper bound)
-#pragma unroll
-    for (int i = 0; i < X_DYN / 2; ++i)
-        if (!((i >= 7 && i <= 9) || i >= 15)) w[i] = clamp1_h2(w[i]);
-}
-
 // The MMAs of one layer of one tile (one elected lane).  layer 0: X . W0^T (K = 48, bias in column 36); layer 1: H . W1^T + b1
 // (bias: X[:, 32:48] . W0img[:, 48:64]^T); layer 2: H . WO^T + bo (N = 16; bias: X[:, 32:48] . WOB[:, 32:48]^T).
 // AT: the A operands (X, H) live in tensor memory -- x_lo / h_lo are then TMEM addresses (lane 0, first column of the operand) and a
@@ -236,20 +208,6 @@ __device__ __forceinline__ void issuer_phase(IssTile& a, IssTile& b, unsigned w0
 
 __device__ __forceinline__ bool ready_pred16(float pos_thr, float ori_thr, float a_thr, float dq_thr, float pos, float ori, float an, float dqn) {
     return pos_thr > 0.0f && ori_thr > 0.0f && pos <= pos_thr && ori <= ori_thr && (a_thr <= 0.0f || an <= a_thr) && (dq_thr <= 0.0f || dqn <= dq_thr);
-}
-
-// pose error, margins and normalised joint positions of a freshly reset state (what step_core<FAST> leaves behind after a step)
-__device__ __forceinline__ void prime_step_out(const KinEnvParams& P, const EnvRegs& s, StepOut& so) {
-    so.done = 0u;
-    so.pos = s.entry[0];
-    so.ori = s.entry[1];
-    so.dq_l2 = 0.0f;
-    pose_error(s.ee, s.goal, so.pe, so.oe);
-#pragma unroll
-    for (int i = 0; i < NJ; ++i) {
-        so.qn[i] = fmaf(2.0f * P.k_inv_span[i], s.q[i] - P.joint_lower[i], -1.0f);
-        so.margin[i] = 1.0f - fabsf(so.qn[i]);
-    }
 }
 
 // ISS: the CTA's last two warps are issuer warps (<= 14 env warps, the balanced one-wave shape): blockDim.x = 32 (env warps + 2)

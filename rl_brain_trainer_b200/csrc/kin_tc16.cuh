@@ -83,6 +83,49 @@ __device__ __forceinline__ void st_chunk(unsigned char* img, int row, int chunk,
 // and are folded into the layer-1 bias when the weights are staged.
 __device__ __forceinline__ int dyn_col(int k) { return k < 20 ? k : (k < 27 ? k + 10 : (k < 29 ? k + 10 : k + 11)); }
 
+// Observation of the current state as 18 packed fp16 pairs in X-image column order:
+// dq 0:7 | goal_ori_err 7:10 | goal_pos_err 10:13 | joint_limit_margin 13:20 | prev_action 20:27 | progress 27:29 | q 29:36
+// (observation_builder.py:29-94; values and clamps as kin_core.cuh::build_obs_from).
+__device__ __forceinline__ void obs_pack(const KinEnvParams& P, const EnvRegs& s, const StepOut& so, unsigned* w) {
+    float v[X_DYN];
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) {
+        v[i] = s.dq[i] * P.k_inv_delta_limit[i];
+        v[13 + i] = so.margin[i];
+        v[20 + i] = s.pa[i];
+        v[29 + i] = so.qn[i];
+    }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        v[7 + k] = so.oe[k] * P.k_inv_ori_err_scale;
+        v[10 + k] = so.pe[k] * P.k_inv_pos_err_scale;
+    }
+    v[27] = (float)s.step * P.k_inv_episode_length;
+    v[28] = (float)s.dwell * P.k_inv_dwell_steps_target;
+#pragma unroll
+    for (int i = 0; i < X_DYN / 2; ++i) w[i] = pack_h2(v[2 * i], v[2 * i + 1]);
+    // margins (columns 14..19) and normalised q (30..35) are inside [0, 1] / [-1, 1] by construction (q is clipped to its limits
+    // and kin_core.cuh::qnorm clamps the rounding above 1); everything else gets the reference's clip to [-1, 1] (progress is
+    // non-negative, its clip to [0, 1] is the same upper bound)
+#pragma unroll
+    for (int i = 0; i < X_DYN / 2; ++i)
+        if (!((i >= 7 && i <= 9) || i >= 15)) w[i] = clamp1_h2(w[i]);
+}
+
+// pose error, margins and normalised joint positions of a freshly reset state (what step_core<FAST> leaves behind after a step)
+__device__ __forceinline__ void prime_step_out(const KinEnvParams& P, const EnvRegs& s, StepOut& so) {
+    so.done = 0u;
+    so.pos = s.entry[0];
+    so.ori = s.entry[1];
+    so.dq_l2 = 0.0f;
+    pose_error(s.ee, s.goal, so.pe, so.oe);
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) {
+        so.qn[i] = qnorm(P, s.q[i], i);
+        so.margin[i] = 1.0f - fabsf(so.qn[i]);
+    }
+}
+
 // stage one policy's actor as fp16 B-operand images (all threads of the CTA); `mode` selects the mode_flag column
 __device__ __forceinline__ void load_weights(Smem& S, const DevPolicy& p, int mode, int tid, int nthreads) {
     for (int i = tid; i < HID * 64; i += nthreads) {
