@@ -581,6 +581,22 @@ int kin_route_step(void *handle, const KinRouteTable *host_route, float *state, 
                    float *obs, float *reward, uint8_t *done, float *raux, float *rcomp, int sequence_mode,
                    int reset_ready_streak_on_advance, void *stream);
 
+/* Replaces: a VecEnv of RouteKinematicEnv / RouteSequenceKinematicEnv (kinematic_phase1/train_route_curriculum.py) stepping and
+ * auto-resetting -- kin_route_step followed, in the same launch, by the sampled reset of every slot the step finished
+ * (KIN_DONE_TERMINATED or KIN_DONE_TRUNCATED).  reward / done / raux / rcomp describe the step just taken; the finished slots'
+ * done bytes also get KIN_DONE_AUTORESET and their obs rows hold the first observation of the next episode.
+ * Counter convention: state row KIN_ROW_EPISODE counts the episodes a slot has finished.  A finished slot draws
+ * episode = row + 1, resets exactly as kin_route_reset_sampled(host_reset, seed, counter = episode) would, and stores episode back
+ * into the row; so the counter lives on the device and a CUDA graph can replay the call unchanged.  A sampled reset of the whole
+ * batch with counter 0 plus a zeroed KIN_ROW_EPISODE row starts the sequence: later resets of a slot use counters 1, 2, ...
+ * terminal_obs (nullable, [n,80], 16-byte aligned): the rows of the finished slots receive the finished episode's last
+ * observation; rows of other slots are either untouched or, when a slot within the same group of 32 finished, set to that
+ * slot's obs row.  host_reset: as for kin_route_reset_sampled, every mode's waypoint range inside the route.                    */
+int kin_route_step_autoreset(void *handle, const KinRouteTable *host_route, const KinRouteResetParams *host_reset, float *state,
+                             int stride, int n_envs, const float *action, float *obs, float *reward, uint8_t *done, float *raux,
+                             float *rcomp, int sequence_mode, int reset_ready_streak_on_advance, uint64_t seed, float *terminal_obs,
+                             void *stream);
+
 /* Replaces: evaluate_sequential_route / _roll_one (eval/eval_route_curriculum.py:55-125,188-218) for n independent
  * replicas, fused with the 80-input route policy: replica r starts at start_q[r] (nullable -> waypoint(start_index-1))
  * and chains waypoints start_index..end_index, each from the actual final state of the previous one.

@@ -139,6 +139,7 @@ def lib() -> ctypes.CDLL:
     L.kin_route_reset.argtypes = [vp, vp, vp, i32, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]
     L.kin_route_reset_sampled.argtypes = [vp, vp, vp, vp, i32, i32, vp, u64, ctypes.c_uint32, vp, vp]
     L.kin_route_step.argtypes = [vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, vp]
+    L.kin_route_step_autoreset.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, u64, vp, vp]
     L.kin_route_probe.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     L.kin_route_probe_rows.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, i32, vp]
     L.kin_route_probe_tc.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]

@@ -16,11 +16,16 @@
 
 namespace kin {
 
-template <bool SEQ, bool COMP>
+// AUTORESET: a slot whose step finishes its episode (terminated or truncated) is re-seeded in the same launch with the draw
+// kin_route_reset_sampled makes for it, Philox(seed, env, state[KIN_ROW_EPISODE] + 1), and the counter is written back.
+// reward / done / raux / rcomp describe the step just taken; terminal_obs (nullable) receives the finished episode's last
+// observation, obs the next episode's first.  The trailing parameters are unused by the AUTORESET = false instances.
+template <bool SEQ, bool COMP, bool AUTORESET>
 __global__ void __launch_bounds__(RT_THREADS)
 kin_route_step_kernel(const __grid_constant__ KinEnvParams P, RouteView R, float* __restrict__ state, int stride, int n,
                       const float* __restrict__ action, float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ done,
-                      float* __restrict__ raux, float* __restrict__ rcomp, int reset_streak) {
+                      float* __restrict__ raux, float* __restrict__ rcomp, int reset_streak, const __grid_constant__ KinRouteResetParams C,
+                      uint64_t seed, float* __restrict__ terminal_obs) {
     extern __shared__ __align__(128) float smem[];
     float* tiles = smem;                                        // [RT_WARPS][ROBS_TILE_FLOATS]
     float* q_table = smem + RT_WARPS * ROBS_TILE_FLOATS;        // [min(n_wp, 1024)][7]
@@ -47,21 +52,24 @@ kin_route_step_kernel(const __grid_constant__ KinEnvParams P, RouteView R, float
     float rc[COMP ? 17 : 1];
     const float* table = R.n <= ROUTE_MAX_SMEM_WP ? q_table : R.q;
     route_step_core<SEQ, COMP>(P, R, table, s, rr, a, reset_streak != 0, so, ro, rc);
+    const bool finished = AUTORESET && active && (ro.done & (KIN_DONE_TERMINATED | KIN_DONE_TRUNCATED));
     if (active) {
-        store_env_step(state, stride, env, s);
-        if (SEQ) {   // the advance rewrote goal pose + entry metrics
+        if (!finished) {   // a finished slot's state rows are written by its reset below
+            store_env_step(state, stride, env, s);
+            if (SEQ) {   // the advance rewrote goal pose + entry metrics
 #pragma unroll
-            for (int k = 0; k < 6; ++k) st_row(state, stride, KIN_ROW_GOAL_POSE + k, env, s.goal[k]);
+                for (int k = 0; k < 6; ++k) st_row(state, stride, KIN_ROW_GOAL_POSE + k, env, s.goal[k]);
 #pragma unroll
-            for (int k = 0; k < 4; ++k) st_row(state, stride, KIN_ROW_ENTRY + k, env, s.entry[k]);
-            const float* gq = R.q + (size_t)wp_clamp(R, rr.index) * NJ;
+                for (int k = 0; k < 4; ++k) st_row(state, stride, KIN_ROW_ENTRY + k, env, s.entry[k]);
+                const float* gq = R.q + (size_t)wp_clamp(R, rr.index) * NJ;
 #pragma unroll
-            for (int i = 0; i < NJ; ++i) st_row(state, stride, KIN_ROW_GOAL_Q + i, env, __ldg(gq + i));
+                for (int i = 0; i < NJ; ++i) st_row(state, stride, KIN_ROW_GOAL_Q + i, env, __ldg(gq + i));
+            }
+            st_row_u(state, stride, KIN_ROW_ROUTE, env, (unsigned)rr.index | ((unsigned)min(rr.streak, 0xffff) << 16));
+            st_row_u(state, stride, KIN_ROW_ROUTE2, env, (unsigned)rr.last | ((unsigned)min(rr.completed, 0xffff) << 16));
         }
-        st_row_u(state, stride, KIN_ROW_ROUTE, env, (unsigned)rr.index | ((unsigned)min(rr.streak, 0xffff) << 16));
-        st_row_u(state, stride, KIN_ROW_ROUTE2, env, (unsigned)rr.last | ((unsigned)min(rr.completed, 0xffff) << 16));
         reward[env] = ro.reward;
-        done[env] = (uint8_t)ro.done;
+        done[env] = (uint8_t)(ro.done | (finished ? KIN_DONE_AUTORESET : 0u));
         if (raux) {
             raux[(size_t)KIN_RAUX_Q_ERR * stride + env] = ro.q_err;
             raux[(size_t)KIN_RAUX_NEAREST * stride + env] = ro.nearest;
@@ -78,6 +86,25 @@ kin_route_step_kernel(const __grid_constant__ KinEnvParams P, RouteView R, float
         }
     }
     float o56[OBS], o[ROBS];
+    if (AUTORESET && __ballot_sync(0xffffffffu, finished)) {
+        if (terminal_obs) {   // the whole warp's pre-reset rows through the tile; only the finished rows are meaningful to callers
+            build_obs(P, s, KIN_MODE_APPROACH, o56);
+            build_route_obs(P, R, s, rr.index, o56, o);
+            stage_route_obs_row(tile, lane, o);
+            bulk_store_tile(terminal_obs + (size_t)env0 * ROBS, tile, min(WARP, n - env0) * ROBS * 4, lane);
+            bulk_store_wait_read(lane);
+        }
+        if (finished) {
+            const unsigned episode = ld_row_u(state, stride, KIN_ROW_EPISODE, env) + 1u;
+            Philox rng(seed, (uint32_t)env, episode);
+            float gq[NJ];
+            sample_route_reset_dev(P, R, C, rng, s, rr, gq);
+            store_env_reset(state, stride, env, s, gq);
+            st_row_u(state, stride, KIN_ROW_ROUTE, env, (unsigned)rr.index);
+            st_row_u(state, stride, KIN_ROW_ROUTE2, env, (unsigned)rr.last);
+            st_row_u(state, stride, KIN_ROW_EPISODE, env, episode);
+        }
+    }
     build_obs(P, s, KIN_MODE_APPROACH, o56);   // after an advance the goal changed, so recompute the goal errors
     build_route_obs(P, R, s, rr.index, o56, o);
     stage_route_obs_row(tile, lane, o);
@@ -260,6 +287,13 @@ kin_route_probe_kernel(const __grid_constant__ KinEnvParams P, RouteView R, DevP
 
 using namespace kin;
 
+// every reset mode's target-waypoint range lies inside the route
+static bool reset_ranges_ok(const KinRouteResetParams& C, int n_waypoints) {
+    for (int m = 0; m < 5; ++m)
+        if (C.index_lo[m] < 0 || C.index_hi[m] < C.index_lo[m] || C.index_hi[m] >= n_waypoints) return false;
+    return true;
+}
+
 extern "C" int kin_route_reset(void* handle, const KinRouteTable* host_route, float* state, int stride, int n_envs, const int* env_ids,
                                int n_reset, const int* route_index, const int* start_route_index, const int* last_route_index,
                                const float* initial_q, const float* initial_dq, const float* initial_prev_action, float* obs, void* stream) {
@@ -281,38 +315,59 @@ extern "C" int kin_route_reset_sampled(void* handle, const KinRouteTable* host_r
     if (!h || !route_ok(host_route) || !host_reset) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_reset_sampled: bad handle, route table or reset parameters");
     if (!state || n_envs <= 0 || stride < n_envs || (stride % 32) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_reset_sampled: bad sizes");
     if (obs && ((uintptr_t)obs & 15u)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_reset_sampled: obs must be 16-byte aligned");
-    for (int m = 0; m < 5; ++m)
-        if (host_reset->index_lo[m] < 0 || host_reset->index_hi[m] < host_reset->index_lo[m] || host_reset->index_hi[m] >= host_route->n_waypoints)
-            return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_reset_sampled: waypoint range outside the route");
+    if (!reset_ranges_ok(*host_reset, host_route->n_waypoints)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_reset_sampled: waypoint range outside the route");
     kin_route_reset_sampled_kernel<<<(n_envs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->params, view_of(host_route), *host_reset, state, stride, n_envs,
                                                                                           done, seed, counter, obs);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_route_reset_sampled");
 }
 
-extern "C" int kin_route_step(void* handle, const KinRouteTable* host_route, float* state, int stride, int n_envs, const float* action,
-                              float* obs, float* reward, uint8_t* done, float* raux, float* rcomp, int sequence_mode,
-                              int reset_ready_streak_on_advance, void* stream) {
+// argument checks + launch shared by kin_route_step and kin_route_step_autoreset (C is only read by the AUTORESET instances)
+#define KIN_RMSG(what) (AUTORESET ? "kin_route_step_autoreset: " what : "kin_route_step: " what)
+template <bool AUTORESET>
+static int launch_route_step(void* handle, const KinRouteTable* host_route, const KinRouteResetParams& C, float* state,
+                             int stride, int n_envs, const float* action, float* obs, float* reward, uint8_t* done, float* raux, float* rcomp,
+                             int sequence_mode, int reset_ready_streak_on_advance, uint64_t seed, float* terminal_obs, void* stream) {
     KinHandle* h = kin_handle(handle);
-    if (!h || !route_ok(host_route)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_step: bad handle or route table");
-    if (!state || !action || !obs || !reward || !done || n_envs <= 0 || stride < n_envs || (stride % 32) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_step: bad buffers / sizes");
-    if (((uintptr_t)obs & 15u)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_step: obs must be 16-byte aligned");
+    if (!h || !route_ok(host_route)) return kin_fail(KIN_ERR_INVALID_ARG, KIN_RMSG("bad handle or route table"));
+    if (!state || !action || !obs || !reward || !done || n_envs <= 0 || stride < n_envs || (stride % 32) != 0) return kin_fail(KIN_ERR_INVALID_ARG, KIN_RMSG("bad buffers / sizes"));
+    if (((uintptr_t)obs & 15u) || ((uintptr_t)terminal_obs & 15u)) return kin_fail(KIN_ERR_INVALID_ARG, KIN_RMSG("obs must be 16-byte aligned"));
     const RouteView R = view_of(host_route);
     const size_t smem = (size_t)(RT_WARPS * ROBS_TILE_FLOATS + min(R.n, ROUTE_MAX_SMEM_WP) * NJ) * sizeof(float);
     const int blocks = (n_envs + RT_THREADS - 1) / RT_THREADS;
     cudaStream_t st = (cudaStream_t)stream;
-#define KIN_RLAUNCH(SEQ, COMP)                                                                                                          \
-    do {                                                                                                                                \
-        cudaError_t ea = cudaFuncSetAttribute(kin_route_step_kernel<SEQ, COMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        if (ea != cudaSuccess) return kin_fail_cuda(ea, "kin_route_step: smem attribute");                                              \
-        kin_route_step_kernel<SEQ, COMP><<<blocks, RT_THREADS, smem, st>>>(h->params, R, state, stride, n_envs, action, obs, reward, done, \
-                                                                          raux, rcomp, reset_ready_streak_on_advance);                   \
+#define KIN_RLAUNCH(SEQ, COMP)                                                                                                                  \
+    do {                                                                                                                                        \
+        cudaError_t ea = cudaFuncSetAttribute(kin_route_step_kernel<SEQ, COMP, AUTORESET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (ea != cudaSuccess) return kin_fail_cuda(ea, KIN_RMSG("smem attribute"));                                                     \
+        kin_route_step_kernel<SEQ, COMP, AUTORESET><<<blocks, RT_THREADS, smem, st>>>(h->params, R, state, stride, n_envs, action, obs, reward,  \
+                                                                                     done, raux, rcomp, reset_ready_streak_on_advance, C, seed, \
+                                                                                     terminal_obs);                                             \
     } while (0)
     if (sequence_mode) { if (rcomp) KIN_RLAUNCH(true, true); else KIN_RLAUNCH(true, false); }
     else { if (rcomp) KIN_RLAUNCH(false, true); else KIN_RLAUNCH(false, false); }
 #undef KIN_RLAUNCH
     cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_route_step");
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, AUTORESET ? "kin_route_step_autoreset" : "kin_route_step");
+}
+#undef KIN_RMSG
+
+extern "C" int kin_route_step(void* handle, const KinRouteTable* host_route, float* state, int stride, int n_envs, const float* action,
+                              float* obs, float* reward, uint8_t* done, float* raux, float* rcomp, int sequence_mode,
+                              int reset_ready_streak_on_advance, void* stream) {
+    return launch_route_step<false>(handle, host_route, KinRouteResetParams{}, state, stride, n_envs, action, obs, reward, done,
+                                    raux, rcomp, sequence_mode, reset_ready_streak_on_advance, 0, nullptr, stream);
+}
+
+extern "C" int kin_route_step_autoreset(void* handle, const KinRouteTable* host_route, const KinRouteResetParams* host_reset, float* state,
+                                        int stride, int n_envs, const float* action, float* obs, float* reward, uint8_t* done, float* raux,
+                                        float* rcomp, int sequence_mode, int reset_ready_streak_on_advance, uint64_t seed, float* terminal_obs,
+                                        void* stream) {
+    if (!host_reset) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_step_autoreset: reset parameters are required");
+    if (route_ok(host_route) && !reset_ranges_ok(*host_reset, host_route->n_waypoints))
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_step_autoreset: waypoint range outside the route");
+    return launch_route_step<true>(handle, host_route, *host_reset, state, stride, n_envs, action, obs, reward, done,
+                                   raux, rcomp, sequence_mode, reset_ready_streak_on_advance, seed, terminal_obs, stream);
 }
 
 extern "C" int kin_route_probe_rows(void* handle, const KinRouteTable* host_route, const KinPolicyWeights* w, const float* start_q, int start_index,

@@ -169,13 +169,22 @@ class BatchedRouteKinematicEnv:
     """
 
     def __init__(self, route: RouteDataset, config: RouteEnvConfig, num_envs: int, device: str | torch.device = "cuda", *,
-                 sequence_config: RouteSequenceConfig | None = None, with_components: bool = False) -> None:
+                 sequence_config: RouteSequenceConfig | None = None, with_components: bool = False, auto_reset: bool = False, seed: int = 0,
+                 graph_step: bool = False) -> None:
         if not torch.cuda.is_available():
             raise _lib.KinError("BatchedRouteKinematicEnv needs a CUDA device; there is no CPU fallback")
         self.config, self.route = config, route
         self.sequence = sequence_config if (sequence_config is not None and sequence_config.enabled) else None
         self.device = torch.device(device)
         self.num_envs = int(num_envs)
+        # auto_reset: a slot whose episode ends is re-seeded inside the step launch (kin_route_step_autoreset) with the draw
+        # reset_done(seed=seed, counter=<episodes the slot has finished>) would make; terminal_obs keeps the last observation.
+        # graph_step: step() replays a CUDA graph of [step kernel, the two done-bit ops], re-captured when the params handle, the
+        # reset window, the seed or the sequence flag changes (as BatchedArmKinematicEnv does).
+        self.auto_reset, self._seed, self.graph_step = bool(auto_reset), int(seed), bool(graph_step)
+        self._graph: Any = None
+        self._graph_key: Any = None
+        self._step_calls = 0
         self.stride = (self.num_envs + 31) // 32 * 32
         self._L = _lib.lib()
         with torch.cuda.device(self.device):
@@ -187,6 +196,7 @@ class BatchedRouteKinematicEnv:
             self.done = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
             self.raux = torch.zeros((_D("KIN_RAUX_ROWS"), self.stride), dtype=torch.float32, device=self.device)
             self.rcomp = torch.zeros((17, self.stride), dtype=torch.float32, device=self.device) if with_components else None
+            self.terminal_obs = torch.zeros_like(self.obs) if self.auto_reset else None
 
     def set_route_window(self, *, max_route_index: int, min_route_index: int = 1) -> None:
         """``RouteKinematicEnv.set_route_window`` (route_env.py:99-121): the waypoint range sampled resets draw from."""
@@ -200,6 +210,24 @@ class BatchedRouteKinematicEnv:
         ids = None if env_ids is None else torch.as_tensor(env_ids, dtype=torch.int32, device=self.device).contiguous()
         m = self.num_envs if ids is None else int(ids.numel())
         self.last_reset: dict[str, torch.Tensor] | None = None
+        if route_index is None and self.auto_reset:
+            # the draws the in-step resets continue: counter 0 here, then 1, 2, ... per slot (state row KIN_ROW_EPISODE)
+            if seed is not None:
+                self._seed = int(seed)
+            mask = None
+            if ids is not None:
+                mask = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
+                mask[ids.long()] = _D("KIN_DONE_TERMINATED")
+            with torch.cuda.device(self.device):
+                _lib.check(self._L.kin_route_reset_sampled(self._params.handle, ctypes.byref(self.table.c), ctypes.byref(self._reset_params()),
+                                                           _ptr(self.state), self.stride, self.num_envs, _ptr(mask), self._seed, 0, _ptr(self.obs),
+                                                           _stream()))
+                episode = self.state[_D("KIN_ROW_EPISODE"), :self.num_envs]
+                if ids is None:
+                    episode.zero_()
+                else:
+                    episode[ids.long()] = 0.0
+            return self.obs
         if route_index is None:      # route_env.py:60-73: no explicit waypoint -> sample_route_reset
             if seed is not None or not hasattr(self, "_gen"):
                 self._gen = torch.Generator(device=self.device)
@@ -282,24 +310,53 @@ class BatchedRouteKinematicEnv:
                                                        self.stride, self.num_envs, _ptr(d), int(seed), int(counter) & 0xFFFFFFFF, _ptr(self.obs), _stream()))
         return self.obs
 
-    def step_raw(self, actions: torch.Tensor) -> None:
-        """One ``kin_route_step`` launch with no host-side post-processing: results land in ``self.obs / reward / done / raux`` (which
-        a rollout loop may point at slices of its own buffers).  ``actions``: contiguous float32 ``[num_envs, 7]`` on this device."""
+    def _launch(self, actions: int) -> None:
+        """One step launch on the current stream: ``kin_route_step``, or ``kin_route_step_autoreset`` for an auto-reset env."""
         seq = self.sequence is not None
-        _lib.check(self._L.kin_route_step(self._params.handle, ctypes.byref(self.table.c), self.state.data_ptr(), self.stride, self.num_envs,
-                                          actions.data_ptr(), self.obs.data_ptr(), self.reward.data_ptr(), self.done.data_ptr(), _ptr(self.raux),
-                                          _ptr(self.rcomp), int(seq), int(bool(self.sequence.reset_ready_streak_on_advance)) if seq else 1, _stream()))
+        streak = int(bool(self.sequence.reset_ready_streak_on_advance)) if seq else 1
+        if self.auto_reset:
+            _lib.check(self._L.kin_route_step_autoreset(self._params.handle, ctypes.byref(self.table.c), ctypes.byref(self._reset_params()),
+                                                        _ptr(self.state), self.stride, self.num_envs, actions, _ptr(self.obs), _ptr(self.reward),
+                                                        _ptr(self.done), _ptr(self.raux), _ptr(self.rcomp), int(seq), streak, self._seed,
+                                                        _ptr(self.terminal_obs), _stream()))
+        else:
+            _lib.check(self._L.kin_route_step(self._params.handle, ctypes.byref(self.table.c), _ptr(self.state), self.stride, self.num_envs,
+                                              actions, _ptr(self.obs), _ptr(self.reward), _ptr(self.done), _ptr(self.raux), _ptr(self.rcomp),
+                                              int(seq), streak, _stream()))
+
+    def step_raw(self, actions: torch.Tensor) -> None:
+        """One step launch with no host-side post-processing: results land in ``self.obs / reward / done / raux`` (which
+        a rollout loop may point at slices of its own buffers).  ``actions``: contiguous float32 ``[num_envs, 7]`` on this device."""
+        self._launch(actions.data_ptr())
 
     def step(self, actions: torch.Tensor):
         a = torch.as_tensor(actions, dtype=torch.float32, device=self.device)
         if a.shape != (self.num_envs, 7):
             raise ValueError(f"Expected action shape {(self.num_envs, 7)}, got {tuple(a.shape)}")
         a = a.contiguous()
-        seq = self.sequence is not None
-        with torch.cuda.device(self.device):
-            _lib.check(self._L.kin_route_step(self._params.handle, ctypes.byref(self.table.c), _ptr(self.state), self.stride, self.num_envs,
-                                              _ptr(a), _ptr(self.obs), _ptr(self.reward), _ptr(self.done), _ptr(self.raux), _ptr(self.rcomp),
-                                              int(seq), int(bool(self.sequence.reset_ready_streak_on_advance)) if seq else 1, _stream()))
+        self._step_calls += 1
+        masks = getattr(self, "_done_masks", None)
+        if masks is None:
+            masks = self._done_masks = torch.tensor([[_D("KIN_DONE_TERMINATED")], [_D("KIN_DONE_TRUNCATED")]], dtype=self.done.dtype, device=self.device)
+        if self.graph_step and self._step_calls > 1:       # (the first call runs eagerly: the smem attribute is set there)
+            if self.auto_reset:
+                self._reset_params()
+            key = (id(self._params), self._reset_params_key if self.auto_reset else None, self._seed, self.sequence is not None)
+            if self._graph is None or self._graph_key != key:
+                self._g_act = torch.empty_like(a)
+                torch.cuda.synchronize(self.device)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.device(self.device), torch.cuda.graph(g):
+                    self._launch(self._g_act.data_ptr())
+                    self._g_tt = (self.done.unsqueeze(0) & masks) != 0
+                self._graph, self._graph_key = g, key
+            self._g_act.copy_(a, non_blocking=True)
+            self._graph.replay()
+            tt = self._g_tt
+        else:
+            with torch.cuda.device(self.device):
+                self._launch(a.data_ptr())
+            tt = (self.done.unsqueeze(0) & masks) != 0
         d = self.done
         n = self.num_envs
         raux, st = self.raux, self.state
@@ -317,7 +374,13 @@ class BatchedRouteKinematicEnv:
         }
         if self.rcomp is not None:
             thunks["reward_components"] = lambda: self.rcomp[:, :n]
-        return self.obs, self.reward, (d & _D("KIN_DONE_TERMINATED")) != 0, (d & _D("KIN_DONE_TRUNCATED")) != 0, LazyInfo(thunks)
+        if self.auto_reset:
+            thunks["auto_reset"] = lambda: (d & _D("KIN_DONE_AUTORESET")) != 0
+            thunks["terminal_observation"] = lambda: self.terminal_obs
+        return self.obs, self.reward, tt[0], tt[1], LazyInfo(thunks)
+
+    def close(self) -> None:
+        return None
 
 
 # SB3 flattens the Dict observation in alphabetical key order (SURVEY 8a row a17): slices of the 80-vector
@@ -328,6 +391,25 @@ ROUTE_OBS_SLICES: dict[str, slice] = {
     "route_scalar": slice(61, 64), "route_tangent": slice(64, 71), "task_type": slice(71, 74), "wp_ori_err": slice(74, 77),
     "wp_pos_err": slice(77, 80),
 }
+
+
+def build_route_observation_space(n_joints: int, include_route_keys: bool) -> Any:
+    """The route wrappers' dict observation space: the base env's keys, plus the four route keys when the observation config
+    includes them (route_observation.py:18-28)."""
+    from .env import _Box, _DictSpace, build_observation_space
+
+    base = build_observation_space(n_joints)
+    if not include_route_keys:
+        return base
+    sp = dict(base.spaces)
+    sp.update({"route_q_goal": _Box(-1.0, 1.0, (n_joints,)), "route_q_error": _Box(-1.0, 1.0, (n_joints,)),
+               "route_tangent": _Box(-1.0, 1.0, (n_joints,)), "route_scalar": _Box(0.0, 1.0, (3,))})
+    return _DictSpace(sp)
+
+
+def route_obs_keys(include_route_keys: bool) -> tuple[str, ...]:
+    """Keys of the route wrappers' dict observation, in the order of the flat 80-vector (``ROUTE_OBS_SLICES``)."""
+    return tuple(k for k in ROUTE_OBS_SLICES if include_route_keys or not k.startswith("route_"))
 
 
 class _RouteBaseEnvView:
@@ -376,14 +458,7 @@ class _SingleRouteEnv:
         n = config.base_env_config.n_joints
         self.action_space = build_action_space(n)
         self._base_observation_space = build_observation_space(n)
-        self.observation_space = self._base_observation_space
-        if config.observation_config.include_route_keys:      # route_observation.py:18-28
-            from .env import _Box, _DictSpace
-
-            sp = dict(self._base_observation_space.spaces)
-            sp.update({"route_q_goal": _Box(-1.0, 1.0, (n,)), "route_q_error": _Box(-1.0, 1.0, (n,)), "route_tangent": _Box(-1.0, 1.0, (n,)),
-                       "route_scalar": _Box(0.0, 1.0, (3,))})
-            self.observation_space = _DictSpace(sp)
+        self.observation_space = build_route_observation_space(n, config.observation_config.include_route_keys)
         self._b = BatchedRouteKinematicEnv(route, config, 1, device, sequence_config=sequence_config, with_components=True)
         self._rng = np.random.default_rng(seed)
         self._start_route_index = 0
@@ -417,8 +492,7 @@ class _SingleRouteEnv:
 
     def _obs_np(self) -> dict[str, np.ndarray]:
         flat = self._b.obs[0].detach().cpu().numpy()
-        keys = ROUTE_OBS_SLICES if self.config.observation_config.include_route_keys else {k: v for k, v in ROUTE_OBS_SLICES.items() if not k.startswith("route_")}
-        return {k: flat[sl].copy() for k, sl in keys.items()}
+        return {k: flat[ROUTE_OBS_SLICES[k]].copy() for k in route_obs_keys(self.config.observation_config.include_route_keys)}
 
     def _augment_obs(self, obs: dict[str, np.ndarray] | None = None) -> dict[str, np.ndarray]:
         """``_augment_obs`` (route_env.py:194-207): the observation of the current device state including the route keys.  Meant
