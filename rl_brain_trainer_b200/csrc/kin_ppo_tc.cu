@@ -195,7 +195,10 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
             const int u = i / (KT * 64), k = i - u * (KT * 64);
             float v = 0.0f;
             if (k < INE) v = __ldg(params + o_w0 + u * IN + (FOLD ? route_unfold_col(k) : k));
-            else if (k == INE) v = __ldg(params + o_b0 + u) + (FOLD ? __ldg(params + o_w0 + u * IN + KIN_ROUTE_ONE_A) + __ldg(params + o_w0 + u * IN + KIN_ROUTE_ONE_B) : 0.0f);
+            else if (k == INE) {    // summed left to right, as kin_ppo_pack_weights does: both weight paths round the same fp32 bias
+                v = __ldg(params + o_b0 + u);
+                if (FOLD) v = (v + __ldg(params + o_w0 + u * IN + KIN_ROUTE_ONE_A)) + __ldg(params + o_w0 + u * IN + KIN_ROUTE_ONE_B);
+            }
             st_bf16(S.W0[k >> 6], u, k & 63, v);
         }
         for (int i = tid; i < 64 * 64; i += TCG_THREADS) st_bf16(S.W1, i >> 6, i & 63, __ldg(params + o_w1 + i));
