@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define KIN_ABI_VERSION 3
+#define KIN_ABI_VERSION 4
 #define KIN_NJ 7
 #define KIN_OBS_DIM 56
 #define KIN_ROUTE_OBS_DIM 80
@@ -376,8 +376,29 @@ typedef struct KinSamplerParams {
     float dock_handoff_state_probability;
     int dock_handoff_state_count;
     const float *dock_handoff_states;
+    /* adaptive frontier targets (this project's extension, coverage.FrontierCurriculum): DEVICE pointers owned by the caller.
+     * The reference stops at per-bucket sampling priorities (workspace/adaptive_frontier_sampler.py); the rule that turns them into
+     * goals is this project's own.  Armed when frontier_probability > 0, frontier_bucket_count > 0 and every pointer is non-null,
+     * and only reached by the random-start pair sampler (approach mode, random_start_enabled).  Draw order of one armed reset:
+     *   1. u < frontier_probability                          (the coin; an UNARMED sampler draws nothing here: today's stream)
+     *   2. the start source mix, as without the table
+     *   3. coin taken:  k = integers(0, B - 1), u = uniform(), bucket b = u < alias_prob[k] ? k : alias_index[k];
+     *                   target j = integers(offset[b], offset[b + 1] - 1); goal_q = targets[j][0:7];
+     *                   stage = targets[j][7], or current_stage when it is -1 (a uniform-valid target)
+     *      otherwise:   the stage-shell target of the source (sample_target_stage + goal shell)
+     *   4. the start of the source (failure_recovery jitters the goal of step 3), dq and prev-action noise
+     *   5. min_pair_joint_l2 retries (at most 12) redraw step 3 the same way: from the table when the coin was taken.
+     * The goal pose is FK(goal_q), computed on the device as for every sampled reset.                                           */
+    float frontier_probability;
+    int frontier_bucket_count;
+    int frontier_target_count;
+    const int *frontier_bucket_offset;   /* [bucket_count + 1], CSR into frontier_targets */
+    const float *frontier_alias_prob;    /* [bucket_count] */
+    const int *frontier_alias_index;     /* [bucket_count] */
+    const float *frontier_targets;       /* [target_count][KIN_FRONTIER_TARGET_FLOATS]: goal_q 7 | stage (-1: uniform-valid) */
 } KinSamplerParams;
 #define KIN_HANDOFF_STATE_FLOATS 34
+#define KIN_FRONTIER_TARGET_FLOATS 8
 
 /* SB3 MultiInputPolicy weights, fp32, row-major [out][in] exactly as in policy.pth (SURVEY F4):
  * x[in_dim] -> tanh(W0 x + b0)[64] -> tanh(W1 h + b1)[64] -> Wa h + ba [7]; value head likewise -> [1]. */

@@ -86,6 +86,17 @@ extern "C" int kin_params_set_sampler(void* handle, const KinSamplerParams* host
     KinHandle* h = kin_handle(handle);
     if (!h || !host_sampler) return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: bad argument");
     if (host_sampler->n_stages < 0 || host_sampler->n_stages > KIN_MAX_STAGES) return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: at most 16 curriculum stages");
+    const KinSamplerParams& s = *host_sampler;
+    if (!std::isfinite(s.frontier_probability) || s.frontier_probability < 0.0f || s.frontier_probability > 1.0f)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: frontier_probability must be finite and in [0, 1]");
+    if (s.frontier_probability > 0.0f) {
+        if (s.frontier_bucket_count <= 0 || s.frontier_target_count <= 0)
+            return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: frontier_probability > 0 needs positive frontier bucket and target counts");
+        if (!s.frontier_bucket_offset || !s.frontier_alias_prob || !s.frontier_alias_index || !s.frontier_targets)
+            return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: frontier_probability > 0 needs all four frontier table pointers");
+        if (!s.random_start_enabled)
+            return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_set_sampler: frontier targets are drawn by the random-start pair sampler: enable random_start");
+    }
     if (!h->d_sampler) {
         cudaError_t e = cudaMalloc(&h->d_sampler, sizeof(KinSamplerParams));
         if (e != cudaSuccess) return kin_fail_cuda(e, "kin_params_set_sampler: cudaMalloc");

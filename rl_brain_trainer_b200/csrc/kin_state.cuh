@@ -260,10 +260,27 @@ struct ResetDraw {
     int stage;
 };
 
+// Adaptive frontier target (this project's extension, KinSamplerParams draw order step 3): alias-table bucket, uniform target in it.
+// Returns the target's stage (current for a uniform-valid target).
+__device__ __forceinline__ int sample_frontier_target(const KinSamplerParams& S, Philox& rng, int current, float* gq) {
+    const int k = rng.integers(0, S.frontier_bucket_count - 1);
+    const float u = rng.uniform();
+    const int b = u < S.frontier_alias_prob[k] ? k : S.frontier_alias_index[k];
+    const int j = rng.integers(S.frontier_bucket_offset[b], S.frontier_bucket_offset[b + 1] - 1);
+    const float* t = S.frontier_targets + (size_t)j * KIN_FRONTIER_TARGET_FLOATS;
+#pragma unroll
+    for (int i = 0; i < NJ; ++i) gq[i] = t[i];
+    const int st = (int)t[NJ];
+    return st < 0 ? current : min(st, S.n_stages - 1);
+}
+
 // reset_samplers.py:213-309.  sources: 0 home, 1 old_success, 2 random_valid, 3 frontier, 4 failure_recovery, 5 stress
 __device__ __forceinline__ void sample_random_start_pair(const KinEnvParams& P, const KinSamplerParams& S, Philox& rng, ResetDraw& d) {
     const int last = S.n_stages - 1;
     const int current = clampi(S.current_stage, 0, last);
+    // the coin is drawn only when the table is armed: an unarmed sampler consumes exactly the reference-parity stream
+    const bool from_table = S.frontier_probability > 0.0f && S.frontier_bucket_count > 0 && S.frontier_bucket_offset && S.frontier_alias_prob &&
+                            S.frontier_alias_index && S.frontier_targets && rng.uniform() < S.frontier_probability;
     float total = 0.0f;
 #pragma unroll
     for (int k = 0; k < 6; ++k) total += fmaxf(S.source_ratio[k], 0.0f);
@@ -278,8 +295,13 @@ __device__ __forceinline__ void sample_random_start_pair(const KinEnvParams& P, 
             if (!found) draw -= v;
         }
     }
-    int tstage = sample_target_stage(S, rng, source, current);
-    sample_shell(P, rng, S.goal_q + tstage * NJ, S.goal_noise + tstage * NJ, d.gq);
+    int tstage;
+    if (from_table) {
+        tstage = sample_frontier_target(S, rng, current, d.gq);
+    } else {
+        tstage = sample_target_stage(S, rng, source, current);
+        sample_shell(P, rng, S.goal_q + tstage * NJ, S.goal_noise + tstage * NJ, d.gq);
+    }
     if (source == 0) {
         int st = min(S.home_stage_index, last);
         sample_shell(P, rng, S.start_q + st * NJ, S.start_noise + st * NJ, d.iq);
@@ -312,8 +334,12 @@ __device__ __forceinline__ void sample_random_start_pair(const KinEnvParams& P, 
 #pragma unroll
             for (int i = 0; i < NJ; ++i) acc = fmaf(d.gq[i] - d.iq[i], d.gq[i] - d.iq[i], acc);
             if (sqrtf(acc) >= S.min_pair_joint_l2) break;
-            tstage = sample_target_stage(S, rng, source, current);
-            sample_shell(P, rng, S.goal_q + tstage * NJ, S.goal_noise + tstage * NJ, d.gq);
+            if (from_table) {
+                tstage = sample_frontier_target(S, rng, current, d.gq);
+            } else {
+                tstage = sample_target_stage(S, rng, source, current);
+                sample_shell(P, rng, S.goal_q + tstage * NJ, S.goal_noise + tstage * NJ, d.gq);
+            }
         }
     }
 #pragma unroll

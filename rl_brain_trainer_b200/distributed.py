@@ -52,6 +52,16 @@ def allreduce_max_(t: torch.Tensor, group: Any = None) -> torch.Tensor:
     return t
 
 
+def check_same_on_all_ranks(value: Any, what: str, group: Any = None) -> None:
+    """Raise on every rank unless every rank of ``group`` holds an equal ``value`` (a small picklable, e.g. a table checksum)."""
+    n = world(group)[1]
+    if n > 1:
+        values: list[Any] = [None] * n
+        dist.all_gather_object(values, value, group=group)
+        if any(v != values[0] for v in values):
+            raise RuntimeError(f"{what} differs between ranks: {values}")
+
+
 def reduce_eval_stats(success: torch.Tensor, final_pos: torch.Tensor, final_ori: torch.Tensor, env_steps: torch.Tensor | int,
                       group: Any = None) -> dict[str, float]:
     """Success rate / mean errors / env-steps over all ranks from per-rank episode rows (one small all-reduce)."""

@@ -103,11 +103,22 @@ class ParamsHandle:
     def handle(self) -> ctypes.c_void_p:
         return self._h
 
-    def set_sampler(self, stage_index: int, handoff_states: torch.Tensor | None = None) -> None:
+    def set_sampler(self, stage_index: int, handoff_states: torch.Tensor | None = None, frontier: Any = None) -> None:
         """Upload the reset sampler tables; ``handoff_states`` ([M, 34] float32 on the device, ``handoff.HandoffBuffer.device_rows``)
-        arms the dock reset's handoff-state replay with ``dock_reset_config.handoff_state_probability``."""
+        arms the dock reset's handoff-state replay with ``dock_reset_config.handoff_state_probability``; ``frontier`` (a
+        ``coverage.FrontierTable`` and a probability, ``(table, p)``) arms the random-start sampler's adaptive frontier targets."""
         self._sampler = _params.sampler_params(self.config, stage_index)
-        self._handoff_states = handoff_states          # keep the device buffer alive as long as the sampler points at it
+        if frontier is not None:
+            table, probability = frontier
+            if not self._sampler.random_start_enabled:
+                raise _lib.KinError("frontier targets are drawn by the random-start pair sampler: the config has random_start_pair_sampling disabled")
+            self._sampler.frontier_probability = float(probability)
+            self._sampler.frontier_bucket_count = int(table.bucket_count)
+            self._sampler.frontier_target_count = int(table.target_count)
+            self._sampler.frontier_bucket_offset = table.offsets.data_ptr()
+            self._sampler.frontier_alias_prob = table.alias_prob.data_ptr()
+            self._sampler.frontier_alias_index = table.alias_index.data_ptr()
+            self._sampler.frontier_targets = table.targets.data_ptr()
         if handoff_states is not None and handoff_states.numel() > 0:
             if handoff_states.dtype != torch.float32 or handoff_states.dim() != 2 or handoff_states.shape[1] != _D("KIN_HANDOFF_STATE_FLOATS") \
                     or not handoff_states.is_cuda or not handoff_states.is_contiguous():
@@ -116,6 +127,9 @@ class ParamsHandle:
             self._sampler.dock_handoff_state_count = int(handoff_states.shape[0])
             self._sampler.dock_handoff_states = handoff_states.data_ptr()
         _lib.check(_lib.lib().kin_params_set_sampler(self._h, ctypes.byref(self._sampler)))
+        # keep the device buffers alive as long as the sampler points at them; the ones replaced are released only now, after the
+        # synchronous upload has ordered them behind every kernel that could still read them
+        self._handoff_states, self._frontier = handoff_states, frontier
 
     def __del__(self) -> None:  # pragma: no cover - interpreter teardown order
         try:
@@ -236,13 +250,28 @@ class BatchedArmKinematicEnv:
 
     def _ensure_sampler(self) -> None:
         if self._sampler_stage != self._stage:
-            self._params.set_sampler(self._stage, getattr(self, "_handoff_rows", None))
+            self._params.set_sampler(self._stage, getattr(self, "_handoff_rows", None), getattr(self, "_frontier", None))
             self._sampler_stage = self._stage
 
     def set_handoff_states(self, rows: torch.Tensor | None) -> None:
         """Arm (or clear) the dock reset's handoff-state replay (reset_samplers.py:434-446): ``rows`` is ``[M, 34]`` float32
         (initial_q | initial_dq | initial_prev_action | goal_q | goal_pose6), e.g. ``HandoffBuffer.device_rows(device)``."""
         self._handoff_rows = None if rows is None else rows.to(self.device, torch.float32).contiguous()
+        self._sampler_stage = None
+
+    def set_frontier_targets(self, table: Any, probability: float = 0.5) -> None:
+        """Arm (or, with ``None``, clear) the adaptive frontier targets of the random-start sampler: with ``probability`` an approach
+        reset draws its goal from ``table`` (a ``coverage.FrontierTable`` on this device: alias-table bucket, uniform target in it)
+        instead of the stage shell.  Uploaded with the next reset / rollout; the env keeps the table alive while the sampler uses it."""
+        if table is not None:
+            if not _params.sampler_params(self.config, self._stage).random_start_enabled:
+                raise _lib.KinError("frontier targets are drawn by the random-start pair sampler: the config has random_start_pair_sampling disabled")
+            if not (0.0 <= float(probability) <= 1.0):
+                raise ValueError("frontier probability must be in [0, 1]")
+            here = self.device.index if self.device.index is not None else torch.cuda.current_device()
+            if not table.offsets.is_cuda or table.offsets.device.index != here:
+                raise ValueError(f"the frontier table lives on {table.offsets.device}, the env on {self.device}")
+        self._frontier = None if table is None else (table, float(probability))
         self._sampler_stage = None
 
     # ------------------------------------------------------------------ reset

@@ -132,4 +132,7 @@ def sampler_params(cfg: Phase1EnvConfig, stage_index: int = 0):
     s.dock_handoff_state_probability = 0.0      # set together with the device buffer (ParamsHandle.set_sampler(handoff_states=...))
     s.dock_handoff_state_count = 0
     s.dock_handoff_states = None
+    s.frontier_probability = 0.0                # set together with the device table (ParamsHandle.set_sampler(frontier=...))
+    s.frontier_bucket_count = 0
+    s.frontier_target_count = 0
     return s

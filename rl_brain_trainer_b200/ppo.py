@@ -20,7 +20,7 @@ import torch
 
 from . import _lib
 from .config import Phase1EnvConfig
-from .distributed import CurriculumTracker, PeerGradExchange, allreduce_sum_, world
+from .distributed import CurriculumTracker, PeerGradExchange, allreduce_sum_, check_same_on_all_ranks, world
 from .env import BatchedArmKinematicEnv, _D
 from .policy import KEYS, PolicyWeights
 
@@ -618,8 +618,19 @@ class PPOTrainer:
         return {"policy_loss": float(a[0]), "value_loss": float(a[1]), "entropy": float(a[2]), "approx_kl": float(a[3]),
                 "clip_fraction": float(a[4]), "grad_norm": float(a[5]), "minibatches": n_mb}
 
-    def learn(self, iterations: int, gate: Any = None) -> list[dict[str, float]]:
-        """``model.learn``: iterations of collect + update; curriculum promotion; optional eval gate (``gate.EvalGate``)."""
+    def _frontier_refresh(self, frontier: Any, force: bool) -> dict[str, Any] | None:
+        rec = frontier.maybe_refresh(self.num_timesteps, self.policy, self.env, force=force)
+        if rec is not None:     # every rank ran the same eval on bitwise-identical parameters: the tables must agree
+            check_same_on_all_ranks(rec["table_checksum"], "the adaptive frontier table", self.group)
+        return rec
+
+    def learn(self, iterations: int, gate: Any = None, frontier: Any = None) -> list[dict[str, float]]:
+        """``model.learn``: iterations of collect + update; curriculum promotion; optional eval gate (``gate.EvalGate``); optional
+        adaptive frontier curriculum (``coverage.FrontierCurriculum``: refreshed before the first rollout, then after every update
+        once its interval has passed; a row gets ``frontier_<field>`` entries when a refresh ran)."""
+        if frontier is not None and self.is_route:
+            raise _lib.KinError("the adaptive frontier curriculum draws arm-env goals; the route trainer has no use for it")
+        pending = self._frontier_refresh(frontier, force=True) if frontier is not None else None
         log = []
         for _ in range(int(iterations)):
             r = self.collect()
@@ -633,6 +644,11 @@ class PPOTrainer:
                 rec = gate.maybe_eval(self.num_timesteps, self.policy)
                 if rec is not None:
                     row["gate_score"] = float(rec["score"])
+            if frontier is not None:
+                rec = self._frontier_refresh(frontier, force=False) or pending
+                pending = None
+                if rec is not None:
+                    row.update({f"frontier_{k}": float(v) for k, v in rec.items() if isinstance(v, (int, float))})
             log.append(row)
         return log
 
