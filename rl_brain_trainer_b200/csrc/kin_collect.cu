@@ -8,53 +8,25 @@
 // (kinematic_phase1/envs/arm_kinematic_env.py:213-365) -- the per-step-launch path in ppo.py::collect stays as the
 // strict-fp32 restatement this kernel is tested against.
 //
-// Mapping (as in kin_rollout_tc.cu): one env <-> one thread <-> one row of the A operand <-> one TMEM lane; a CTA holds
-// TILES (1, 2 or 4) independent 128-env tiles on named barriers sharing one bf16 copy of the weights, so one tile's FP32
-// env arithmetic overlaps another's GEMMs.  Per step and tile:
-//   X  = [obs | 1 | 0]  (bf16, SWIZZLE_128B K-major image)      -> the TMA engine copies the 16 KB image straight into
-//                                                                   the rollout buffer (it IS the update kernel's operand)
-//   Z  = X [W0a;W0c]^T            128 x 128 x 64   -> tanh -> H1 (actor half overwrites the X image, critic half beside it)
-//   Z  = H1a W1a^T | H1c W1c^T    2 x (128 x 64 x 64) -> tanh(+b1) -> H2 in place
-//   O  = H2a WOa^T + H2c WOc^T    128 x 16 x 64    -> 7 action means + value
-// The observation is therefore never written as fp32: the rollout buffer holds the bf16 operand images the tensor-core
-// update (kin_ppo_grad_tc, image mode) consumes with one bulk copy per tile.  Truncated episodes append their terminal
-// observation (fp32) to a short list; kin_ppo_bootstrap_list adds gamma * V(terminal_obs) to their rewards afterwards.
-#include "kin_ppo_layout.cuh"
-#include "kin_state.cuh"
-#include "kin_umma.cuh"
+// The policy half (weights, forward, sample, bootstrap list) is kin_collect_policy.cuh, shared with K4-route; this file holds the
+// env half.  The X operand image of every step (56 obs | 1 | zeros, bf16, SWIZZLE_128B K-major) is copied by the TMA engine
+// straight into the rollout buffer: it IS the operand the tensor-core update (kin_ppo_grad_tc, image mode) consumes with one bulk
+// copy per tile, so the observation is never written as fp32.  Truncated episodes append their terminal observation (fp32) to a
+// short list; kin_ppo_bootstrap_list adds gamma * V(terminal_obs) to their rewards afterwards.
+#include "kin_collect_policy.cuh"
 
 namespace kin {
 
 using namespace umma;
 
-constexpr int CT_ROWS = 128;
-constexpr int CT_TILE_BYTES = CT_ROWS * 128;
-constexpr float kHalfLog2PiC = 0.91893853320467274178f;
-
 template <int TILES>
 struct __align__(1024) CollectSmem {
-    unsigned char XH[TILES][2][CT_TILE_BYTES];   // [.][0]: X image, then actor H1 / H2; [.][1]: critic H1 / H2
-    unsigned char W0[CT_TILE_BYTES];
-    unsigned char W1[2][64 * 128];
-    unsigned char WO[2][16 * 128];
-    float b1[128];
-    float bo[8];
-    float ls[8];
-    float sig[8];
+    unsigned char XH[TILES][2][AC_TILE_BYTES];   // [.][0]: X image, then actor H1 / H2; [.][1]: critic H1 / H2
+    AcWeights<1> w;
     unsigned long long mbar[TILES][2];           // [0]: layer 1 (MMA commit + image store drained), [1]: layers 2 / 3
     unsigned long long mbar_w;                   // weight image bulk copy
     unsigned tmem_base;
 };
-
-__device__ __forceinline__ bool elect_lane() {
-    unsigned pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0u;
-}
-__device__ __forceinline__ void tile_bar(int tile) { asm volatile("bar.sync %0, %1;" ::"r"(tile + 1), "r"(CT_ROWS) : "memory"); }
-__device__ __forceinline__ void mbar_arrive(unsigned saddr) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(saddr) : "memory");
-}
 
 struct CollectOut {
     unsigned char* ximg;      // [T][n/128][16 KB]
@@ -72,112 +44,8 @@ struct CollectOut {
     int boot_cap;
 };
 
-template <int TILES>
-struct TileState {
-    unsigned char *X, *Hc;
-    unsigned aX, aHc, aW0, aW1a, aW1c, aWOa, aWOc, mb1, mb2, tz_mma, tz_row;
-    unsigned par1, par2;
-    int tile, row;
-    bool issuer;
-};
-
-// actor + critic forward of the tile's 128 observations; collective over the tile's 128 threads.  img != nullptr: the X image
-// is also copied to global memory by the TMA engine.  Returns the 7 action means and the value in out[0..7].
-template <int TILES>
-__device__ __forceinline__ void policy_forward_tc(CollectSmem<TILES>& S, TileState<TILES>& c, const float* o, unsigned char* img, float* out) {
-    // ---- X image: 56 obs | 1 | zeros
-#pragma unroll
-    for (int ch = 0; ch < 7; ++ch)
-        *reinterpret_cast<uint4*>(c.X + sw_chunk(c.row, ch)) = make_uint4(pack_bf16(o[8 * ch], o[8 * ch + 1]), pack_bf16(o[8 * ch + 2], o[8 * ch + 3]),
-                                                                           pack_bf16(o[8 * ch + 4], o[8 * ch + 5]), pack_bf16(o[8 * ch + 6], o[8 * ch + 7]));
-    *reinterpret_cast<uint4*>(c.X + sw_chunk(c.row, 7)) = make_uint4(0x00003F80u, 0u, 0u, 0u);
-    fence_async_smem();
-    fence_before();
-    tile_bar(c.tile);
-    if (c.row < 32 && elect_lane()) {      // one lane of the tile's first (converged) warp: uniform-register descriptors
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 128, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX + k * 32), desc_k(c.aW0 + k * 32), id, k > 0);
-        commit(c.mb1);
-        if (img) {
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(img), "r"(c.aX), "r"(CT_TILE_BYTES) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the actor H1 half overwrites the image next
-        }
-        mbar_arrive(c.mb1);
-    }
-    mbar_wait(c.mb1, c.par1);
-    c.par1 ^= 1u;
-    fence_after();
-    // ---- H1 = tanh(Z): columns 0..63 actor -> X's place, 64..127 critic
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        float v[32];
-        tmem_ld32(c.tz_row + q * 32, v);
-        unsigned char* dst = (q < 2) ? c.X : c.Hc;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            unsigned p[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) p[e] = pack_bf16(tanh_fast(v[8 * j + 2 * e]), tanh_fast(v[8 * j + 2 * e + 1]));
-            *reinterpret_cast<uint4*>(dst + sw_chunk(c.row, (q & 1) * 4 + j)) = make_uint4(p[0], p[1], p[2], p[3]);
-        }
-    }
-    fence_async_smem();
-    fence_before();
-    tile_bar(c.tile);
-    if (c.row < 32 && elect_lane()) {      // one lane of the tile's first (converged) warp: uniform-register descriptors
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 64, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX + k * 32), desc_k(c.aW1a + k * 32), id, k > 0);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma + 64, desc_k(c.aHc + k * 32), desc_k(c.aW1c + k * 32), id, k > 0);
-        commit(c.mb2);
-    }
-    mbar_wait(c.mb2, c.par2);
-    c.par2 ^= 1u;
-    fence_after();
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        float v[32];
-        tmem_ld32(c.tz_row + q * 32, v);
-        unsigned char* dst = (q < 2) ? c.X : c.Hc;
-        const float* b = S.b1 + q * 32;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            unsigned p[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e)
-                p[e] = pack_bf16(tanh_fast(v[8 * j + 2 * e] + b[8 * j + 2 * e]), tanh_fast(v[8 * j + 2 * e + 1] + b[8 * j + 2 * e + 1]));
-            *reinterpret_cast<uint4*>(dst + sw_chunk(c.row, (q & 1) * 4 + j)) = make_uint4(p[0], p[1], p[2], p[3]);
-        }
-    }
-    fence_async_smem();
-    fence_before();
-    tile_bar(c.tile);
-    if (c.row < 32 && elect_lane()) {      // one lane of the tile's first (converged) warp: uniform-register descriptors
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 16, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX + k * 32), desc_k(c.aWOa + k * 32), id, k > 0);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aHc + k * 32), desc_k(c.aWOc + k * 32), id, 1u);
-        commit(c.mb2);
-    }
-    mbar_wait(c.mb2, c.par2);
-    c.par2 ^= 1u;
-    fence_after();
-    float r[16];
-    tmem_ld16(c.tz_row, r);
-    fence_before();
-#pragma unroll
-    for (int d = 0; d < 8; ++d) out[d] = r[d] + S.bo[d];
-}
-
 template <int TILES, int MODE>
-__global__ void __launch_bounds__(TILES * CT_ROWS, 1)
+__global__ void __launch_bounds__(TILES * AC_ROWS, 1)
 kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParams* __restrict__ SP, float* __restrict__ state, int stride, int n,
                    const float* __restrict__ params, const unsigned char* __restrict__ wimg, int T, uint64_t noise_seed, uint32_t step0,
                    uint64_t reset_seed, CollectOut out) {
@@ -186,85 +54,32 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
     // round up to 1024 bytes WITHOUT leaving the shared address space (pointer + offset, not an integer round trip), so every
     // access below compiles to LDS / STS rather than generic LD / ST with 64-bit address arithmetic
     CollectSmem<TILES>& S = *reinterpret_cast<CollectSmem<TILES>*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
-    const PpoOffsets O = ppo_offsets(IN);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    constexpr int NT = TILES * CT_ROWS;
+    const int tid = threadIdx.x;
+    constexpr int NT = TILES * AC_ROWS;
 
     // ---- weights -> bf16 operand tiles (both nets): one bulk copy of the prebuilt image, or converted here ---------------
     if (wimg) {
-        static_assert(offsetof(CollectSmem<TILES>, W1) == offsetof(CollectSmem<TILES>, W0) + 16384 &&
-                      offsetof(CollectSmem<TILES>, WO) == offsetof(CollectSmem<TILES>, W0) + 32768, "W0 | W1 | WO must be laid out like the image");
+        static_assert(offsetof(AcWeights<1>, W1) == offsetof(AcWeights<1>, W0) + 16384 &&
+                      offsetof(AcWeights<1>, WO) == offsetof(AcWeights<1>, W0) + 32768, "W0 | W1 | WO must be laid out like the image");
         if (tid == 0) {
             const unsigned mbw = smem_u32(&S.mbar_w);
             mbar_init(mbw, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbw), "r"(KIN_WIMG_BYTES) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(S.W0)), "l"(wimg), "r"(KIN_WIMG_BYTES), "r"(mbw) : "memory");
+            fence_mbar_init();
+            mbar_expect_tx(mbw, KIN_WIMG_BYTES);
+            bulk_load(smem_u32(S.w.W0), wimg, KIN_WIMG_BYTES, mbw);
         }
     } else {
-        {
-            uint4* zw = reinterpret_cast<uint4*>(S.WO);
-            for (int i = tid; i < 2 * 16 * 128 / 16; i += NT) zw[i] = make_uint4(0u, 0u, 0u, 0u);
-        }
-        for (int i = tid; i < 128 * 64; i += NT) {
-            const int nn = i >> 6, k = i & 63, u = nn & 63;
-            const int wbase = (nn < 64) ? O.pi_w0 : O.vf_w0, bbase = (nn < 64) ? O.pi_b0 : O.vf_b0;
-            const float v = k < IN ? __ldg(params + wbase + u * IN + k) : (k == IN ? __ldg(params + bbase + u) : 0.0f);
-            *reinterpret_cast<unsigned short*>(S.W0 + sw_elem(nn, k)) = (unsigned short)(pack_bf16(v, 0.0f) & 0xffffu);
-        }
-        for (int i = tid; i < 2 * 4096; i += NT) {
-            const int nt = i >> 12, u = (i >> 6) & 63, k = i & 63;
-            *reinterpret_cast<unsigned short*>(S.W1[nt] + sw_elem(u, k)) =
-                (unsigned short)(pack_bf16(__ldg(params + (nt ? O.vf_w1 : O.pi_w1) + u * 64 + k), 0.0f) & 0xffffu);
-        }
-        __syncthreads();
-        for (int i = tid; i < 7 * 64; i += NT)
-            *reinterpret_cast<unsigned short*>(S.WO[0] + sw_elem(i >> 6, i & 63)) = (unsigned short)(pack_bf16(__ldg(params + O.act_w + i), 0.0f) & 0xffffu);
-        if (tid < 64) *reinterpret_cast<unsigned short*>(S.WO[1] + sw_elem(7, tid)) = (unsigned short)(pack_bf16(__ldg(params + O.val_w + tid), 0.0f) & 0xffffu);
+        convert_weights<IN, 1, NT>(S.w, params, tid);
     }
-    if (tid < 128) S.b1[tid] = __ldg(params + (tid < 64 ? O.pi_b1 + tid : O.vf_b1 + tid - 64));
-    if (tid < 8) {
-        const float ls = tid < 7 ? __ldg(params + O.log_std + tid) : 0.0f;
-        S.bo[tid] = tid < 7 ? __ldg(params + O.act_b + tid) : __ldg(params + O.val_b);
-        S.ls[tid] = ls;
-        S.sig[tid] = expf(ls);
-    }
-    if (warp == 0) tmem_alloc(smem_u32(&S.tmem_base), TILES * 128);
-    if (tid < TILES) {
-        mbar_init(smem_u32(&S.mbar[tid][0]), 2);
-        mbar_init(smem_u32(&S.mbar[tid][1]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    fence_async_smem();
-    fence_before();
-    __syncthreads();
-    fence_after();
+    load_vectors<IN>(S.w, params, tid);
+    init_tiles<TILES, 2>(S, tid);
     if (wimg) mbar_wait(smem_u32(&S.mbar_w), 0u);
-
-    TileState<TILES> c;
-    c.tile = tid >> 7;
-    c.row = tid & 127;
-    c.issuer = c.row == 0;
-    c.X = S.XH[c.tile][0];
-    c.Hc = S.XH[c.tile][1];
-    c.aX = smem_u32(c.X);
-    c.aHc = smem_u32(c.Hc);
-    c.aW0 = smem_u32(S.W0);
-    c.aW1a = smem_u32(S.W1[0]);
-    c.aW1c = smem_u32(S.W1[1]);
-    c.aWOa = smem_u32(S.WO[0]);
-    c.aWOc = smem_u32(S.WO[1]);
-    c.mb1 = smem_u32(&S.mbar[c.tile][0]);
-    c.mb2 = smem_u32(&S.mbar[c.tile][1]);
-    c.tz_mma = S.tmem_base + c.tile * 128;
-    c.tz_row = c.tz_mma + ((unsigned)((warp & 3) * 32) << 16);
-    c.par1 = c.par2 = 0u;
+    AcTile<1> c = tile_of<1, 2>(S, tid);
 
     const int gtile = blockIdx.x * TILES + c.tile;            // global 128-env tile
-    const int n_tiles = n / CT_ROWS;
+    const int n_tiles = n / AC_ROWS;
     const bool live = gtile < n_tiles;                        // tile-uniform
-    const int env = (live ? gtile : 0) * CT_ROWS + c.row;
+    const int env = (live ? gtile : 0) * AC_ROWS + c.row;
 
     EnvRegs s;
     load_env<MODE != KIN_MODE_APPROACH>(state, stride, env, s);
@@ -278,22 +93,10 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
         for (int t = 0; t < T; ++t) {
             float o[OBS], mv[8];
             build_obs_from(P, s, MODE, pe, oe, margin, o);
-            policy_forward_tc<TILES>(S, c, o, out.ximg + ((size_t)t * n_tiles + gtile) * CT_TILE_BYTES, mv);
-            // ---- a = mean + sigma * eps, log N(a) (DiagGaussianDistribution), SB3 stores the unclipped sample
+            policy_forward<IN, true>(S.w, c, o, out.ximg + ((size_t)t * n_tiles + gtile) * AC_TILE_BYTES, mv);
             const size_t idx = (size_t)t * n + env;
-            float a[NJ], lp = 0.0f;
-            {
-                Philox rng(noise_seed, (unsigned)env, step0 + (uint32_t)t);
-                float eps[8];
-#pragma unroll
-                for (int k = 0; k < 8; k += 2) eps[k] = gauss_pair(rng, &eps[k + 1]);
-#pragma unroll
-                for (int k = 0; k < NJ; ++k) {
-                    a[k] = fmaf(S.sig[k], eps[k], mv[k]);
-                    lp += -0.5f * eps[k] * eps[k] - S.ls[k] - kHalfLog2PiC;
-                    out.action[idx * NJ + k] = a[k];
-                }
-            }
+            float a[NJ];
+            const float lp = sample_action(S.w, noise_seed, (unsigned)env, step0 + (uint32_t)t, mv, a, out.action + idx * NJ);
             out.logp[idx] = lp;
             out.value[idx] = mv[7];
             out.episode_start[idx] = (uint8_t)start;
@@ -303,17 +106,7 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
             unsigned done_bits = so.done;
             const bool finished = (so.done & (KIN_DONE_TERMINATED | KIN_DONE_TRUNCATED)) != 0u;
             if (finished) {
-                if ((so.done & KIN_DONE_TRUNCATED) && !(so.done & KIN_DONE_TERMINATED)) {   // TimeLimit bootstrap list
-                    const int slot = atomicAdd(out.boot_count, 1);
-                    if (slot < out.boot_cap) {
-                        float to[OBS];
-                        build_obs_from(P, s, MODE, so.pe, so.oe, so.margin, to);
-                        out.boot_index[slot] = (int)idx;
-                        float4* dst = reinterpret_cast<float4*>(out.boot_obs + (size_t)slot * OBS);
-#pragma unroll
-                        for (int k = 0; k < OBS / 4; ++k) dst[k] = make_float4(to[4 * k], to[4 * k + 1], to[4 * k + 2], to[4 * k + 3]);
-                    }
-                }
+                push_truncated<OBS>(out, so.done, idx, [&](float* to) { build_obs_from(P, s, MODE, so.pe, so.oe, so.margin, to); });
                 const unsigned episode = ld_row_u(state, stride, KIN_ROW_EPISODE, env) + 1u;
                 Philox rng(reset_seed, (unsigned)env, episode);
                 ResetDraw d;
@@ -340,14 +133,12 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
         // ---- value of the observation after the last step (GAE bootstrap)
         float o[OBS], mv[8];
         build_obs_from(P, s, MODE, pe, oe, margin, o);
-        policy_forward_tc<TILES>(S, c, o, nullptr, mv);
+        policy_forward<IN, true>(S.w, c, o, nullptr, mv);
         out.last_value[env] = mv[7];
         out.start_io[env] = (uint8_t)start;
         store_env_step(state, stride, env, s);
     }
-    fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(S.tmem_base, TILES * 128);
+    release_tiles<TILES>(S, tid);
 }
 
 // r[idx] += gamma * V(terminal_obs) for the truncated episodes the collection kernel listed (strict fp32 critic)
@@ -389,24 +180,10 @@ kin_bootstrap_list_kernel(const float* __restrict__ params, const float* __restr
 
 template <int TILES>
 static cudaError_t launch_collect(const KinHandle* h, float* state, int stride, int n, int mode, const float* params, const unsigned char* wimg, int T,
-                                  uint64_t noise_seed,
-                                  uint32_t step0, uint64_t reset_seed, const CollectOut& out, cudaStream_t st) {
-    const size_t smem = sizeof(CollectSmem<TILES>) + 1024;
-    const int n_tiles = n / CT_ROWS;
-    const int grid = (n_tiles + TILES - 1) / TILES;
-    cudaError_t e;
-    if (mode == KIN_MODE_APPROACH) {
-        e = cudaFuncSetAttribute(kin_collect_kernel<TILES, KIN_MODE_APPROACH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kin_collect_kernel<TILES, KIN_MODE_APPROACH><<<grid, TILES * CT_ROWS, smem, st>>>(h->params, h->d_sampler, state, stride, n, params, wimg, T,
-                                                                                        noise_seed, step0, reset_seed, out);
-    } else {
-        e = cudaFuncSetAttribute(kin_collect_kernel<TILES, KIN_MODE_DOCK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kin_collect_kernel<TILES, KIN_MODE_DOCK><<<grid, TILES * CT_ROWS, smem, st>>>(h->params, h->d_sampler, state, stride, n, params, wimg, T, noise_seed,
-                                                                                    step0, reset_seed, out);
-    }
-    return cudaGetLastError();
+                                  uint64_t noise_seed, uint32_t step0, uint64_t reset_seed, const CollectOut& out, cudaStream_t st) {
+    auto kernel = mode == KIN_MODE_APPROACH ? kin_collect_kernel<TILES, KIN_MODE_APPROACH> : kin_collect_kernel<TILES, KIN_MODE_DOCK>;
+    return launch_tiles<TILES>(kernel, sizeof(CollectSmem<TILES>) + 1024, n, st, h->params, h->d_sampler, state, stride, n, params, wimg, T, noise_seed,
+                               step0, reset_seed, out);
 }
 
 }  // namespace kin
@@ -424,18 +201,12 @@ extern "C" int kin_ppo_collect(void* handle, float* state, int stride, int n_env
         !boot_index || !boot_obs || boot_cap <= 0 || n_steps <= 0)
         return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_collect: null buffer or bad sizes");
     if (in_dim != 56) return kin_fail(KIN_ERR_UNSUPPORTED, "kin_ppo_collect: in_dim must be 56");
-    if (n_envs <= 0 || (n_envs % CT_ROWS) != 0 || stride < n_envs || (stride % 32) != 0)
+    if (n_envs <= 0 || (n_envs % AC_ROWS) != 0 || stride < n_envs || (stride % 32) != 0)
         return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_collect: n_envs must be a positive multiple of 128 (one GEMM tile), stride % 32 == 0");
     if (mode != KIN_MODE_APPROACH && mode != KIN_MODE_DOCK) return kin_fail(KIN_ERR_UNSUPPORTED, "kin_ppo_collect: mode must be approach (0) or dock (1)");
     if (((uintptr_t)obs_tiles & 15u) || ((uintptr_t)boot_obs & 15u)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_collect: obs_tiles / boot_obs must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
-    int tiles = tiles_per_cta;
-    if (tiles <= 0) {   // fewest tiles per CTA that still fits the batch in one wave of CTAs (one CTA per SM)
-        int sms = 148, dev = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const int n_tiles = n_envs / CT_ROWS;
-        tiles = n_tiles <= sms ? 1 : (n_tiles <= 2 * sms ? 2 : 4);
-    }
+    const int tiles = collect_tiles_per_cta(tiles_per_cta, n_envs);
     CollectOut out{(unsigned char*)obs_tiles, action, logp, value, reward, done, episode_start, start_io, last_value, boot_count, boot_index, boot_obs, boot_cap};
     cudaError_t e = cudaMemsetAsync(boot_count, 0, sizeof(int), st);
     if (e != cudaSuccess) return kin_fail_cuda(e, "kin_ppo_collect: memset");

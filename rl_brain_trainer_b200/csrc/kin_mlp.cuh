@@ -4,7 +4,7 @@
 // them) and are read as warp-uniform 128-bit loads (one LDS.128 feeds 4 FFMA); each thread's hidden
 // activations go through a private column of a shared [64][BLOCK] scratch so the output loop can stay
 // rolled (a full unroll of 64x56 FFMA would blow the instruction cache).  This is the strict-fp32 path
-// used for parity runs; the tensor-core variant (tcgen05, TMEM accumulators) lives in kin_rollout_tc.cu.
+// used for parity runs; the tensor-core variant (tcgen05, TMEM accumulators) lives in kin_rollout_tc16.cu.
 //
 // Replaces `model.predict(obs, deterministic=True)` (eval/eval_three_stage.py:25-27; SURVEY F4).
 #pragma once

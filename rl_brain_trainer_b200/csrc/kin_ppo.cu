@@ -28,7 +28,6 @@ namespace kin {
 constexpr int PPO_THREADS = 256;
 constexpr int TS = KIN_PPO_TILE;      // 64 samples per tile
 constexpr int HS = 132;               // row stride of the [TS][128] activation tiles (16-byte aligned rows)
-constexpr float kHalfLog2Pi = 0.91893853320467274178f;
 
 // ---------------------------------------------------------------------------------------------------------
 // rollout-side kernels

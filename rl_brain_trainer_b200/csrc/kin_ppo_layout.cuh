@@ -5,6 +5,8 @@
 
 namespace kin {
 
+constexpr float kHalfLog2Pi = 0.91893853320467274178f;   // 0.5 * log(2 pi): the normalising term of the policy's Gaussian log-density
+
 struct PpoOffsets {
     int pi_w0, pi_b0, pi_w1, pi_b1, act_w, act_b, vf_w0, vf_b0, vf_w1, vf_b1, val_w, val_b, log_std, total;
 };

@@ -57,7 +57,6 @@ constexpr int TCG_THREADS = TCG_EPI_THREADS + 32;   // + the MMA issuer warp
 constexpr int TCG_ISSUER_WARP = TCG_EPI_THREADS / 32;
 constexpr int TCG_ROWS = 128;
 constexpr int TILE_BYTES = TCG_ROWS * 128;        // [128][64 bf16]
-constexpr float kHalfLog2PiTc = 0.91893853320467274178f;
 
 // TMEM column map (fp32 columns)
 constexpr unsigned COL_Z = 0;         // 64 (layer 3's O aliases columns 0..15)
@@ -112,22 +111,9 @@ struct __align__(1024) TcGradSmem {
     unsigned tmem_base;
 };
 
-__device__ __forceinline__ void bulk_load(unsigned dst_saddr, const void* src, unsigned bytes, unsigned mbar_saddr) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst_saddr), "l"(src), "r"(bytes), "r"(mbar_saddr) : "memory");
-}
-__device__ __forceinline__ void st_bf16(unsigned char* tile, int row, int col, float v) {
-    *reinterpret_cast<unsigned short*>(tile + sw_elem(row, col)) = (unsigned short)(pack_bf16(v, 0.0f) & 0xffffu);
-}
-
-__device__ __forceinline__ bool elect_one() {
-    unsigned pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0u;
-}
 // named barrier 1: the epilogue threads arrive when an operand tile (or a TMEM read) is complete, the issuer warp waits for it
-__device__ __forceinline__ void ready_arrive() { asm volatile("bar.arrive 1, %0;" ::"n"(TCG_THREADS) : "memory"); }
-__device__ __forceinline__ void ready_sync() { asm volatile("bar.sync 1, %0;" ::"n"(TCG_THREADS) : "memory"); }
+__device__ __forceinline__ void ready_arrive() { bar_arrive(1, TCG_THREADS); }
+__device__ __forceinline__ void ready_sync() { bar_sync(1, TCG_THREADS); }
 
 // this thread's 32 accumulator columns [32 * half, 32 * half + 32) of its row -> f -> packed bf16 in p[16].
 // MODE 0: tanh; 1: tanh(x + b1); 2: x * (1 - h^2), h = keep[] (the packed copy of the same columns from the forward pass)
@@ -247,16 +233,13 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
     if (tid == 0) {
 #pragma unroll
         for (int i = 0; i < 6; ++i) mbar_init(smem_u32(&S.mbar[i]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
         if (wimg) {    // this net's W0 | W1 | WO blocks of the prebuilt image: three bulk copies (TMA engine) on one mbarrier
             const unsigned mbw = smem_u32(&S.mbar[4]);
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbw), "r"(8192 + 8192 + 2048) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(S.W0[0])), "l"(wimg + KIN_WIMG_W0 + net * 8192), "r"(8192), "r"(mbw) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(S.W1)), "l"(wimg + KIN_WIMG_W1 + net * 8192), "r"(8192), "r"(mbw) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(S.WO)), "l"(wimg + KIN_WIMG_WO + net * 2048), "r"(2048), "r"(mbw) : "memory");
+            mbar_expect_tx(mbw, 8192 + 8192 + 2048);
+            bulk_load(smem_u32(S.W0[0]), wimg + KIN_WIMG_W0 + net * 8192, 8192, mbw);
+            bulk_load(smem_u32(S.W1), wimg + KIN_WIMG_W1 + net * 8192, 8192, mbw);
+            bulk_load(smem_u32(S.WO), wimg + KIN_WIMG_WO + net * 2048, 2048, mbw);
         }
     }
     fence_async_smem();
@@ -289,7 +272,7 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
         auto stage = [&](int jj, int b) {       // called by the elected lane only
             const int t0 = __ldg(tile_ids + 2 * jj), t1 = __ldg(tile_ids + 2 * jj + 1);
             const unsigned mb = mb_x0 + 8 * b;
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb), "r"(stage_bytes) : "memory");
+            mbar_expect_tx(mb, stage_bytes);
             if (IMG) bulk_load(aX0 + b * TILE_BYTES, img + (size_t)(t0 >> 1) * TILE_BYTES, TILE_BYTES, mb);
             if (net == 0) {
                 bulk_load(aAct + b * 3584, action + (size_t)t0 * 448, 1792u, mb);
@@ -470,7 +453,7 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
 #pragma unroll
                     for (int d = 0; d < 7; ++d) {
                         z[d] = (act_r[d] - (o[d] + S.bo[d])) * S.inv_sig[d];
-                        lp += -0.5f * z[d] * z[d] - S.ls[d] - kHalfLog2PiTc;
+                        lp += -0.5f * z[d] * z[d] - S.ls[d] - kHalfLog2Pi;
                     }
                     if (logp_out) logp_out[g] = lp;
                     if (!forward_only) {
@@ -486,7 +469,7 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
                             dm[d] = inv_global_batch * dpl_dlp * z[d] * S.inv_sig[d];
                             dbo[d] += dm[d];
                             dls[d] += inv_global_batch * dpl_dlp * (z[d] * z[d] - 1.0f) - inv_global_batch * hp.ent_coef;
-                            ent += 0.5f + kHalfLog2PiTc + S.ls[d];
+                            ent += 0.5f + kHalfLog2Pi + S.ls[d];
                         }
                         *reinterpret_cast<uint4*>(S.DO + sw_chunk(row, 0)) =
                             make_uint4(pack_bf16(dm[0], dm[1]), pack_bf16(dm[2], dm[3]), pack_bf16(dm[4], dm[5]), pack_bf16(dm[6], 0.0f));

@@ -49,7 +49,6 @@ constexpr int ISSUER_WARP = STREAMS * EPI / 32;    // first chain-issuer warp
 constexpr int ACC_WARP = ISSUER_WARP + STREAMS;
 constexpr int ROWS = 128;
 constexpr int TILE = ROWS * 128;                   // [128][64 bf16]
-constexpr float kHalfLog2Pi = 0.91893853320467274178f;
 constexpr int DO_COL = 57;                         // X columns 57..63 hold dL/d(mean_0..6) (actor) or dL/dvalue (critic, column 57)
 constexpr int WO_ROW = DO_COL - 48;                // ... which face rows 9..15 of the WO tile (K chunk 48..63 of X)
 
@@ -103,27 +102,6 @@ __device__ unsigned long long kin_ppo_trace3_buf[4][16];
 #define T3_FLUSH(n)
 #endif
 
-__device__ __forceinline__ void bulk_load(unsigned dst_saddr, const void* src, unsigned bytes, unsigned mbar_saddr) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst_saddr), "l"(src), "r"(bytes), "r"(mbar_saddr) : "memory");
-}
-__device__ __forceinline__ void expect_tx(unsigned mbar_saddr, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar_saddr), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_test(unsigned saddr, unsigned parity) {
-    unsigned ok;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(saddr), "r"(parity) : "memory");
-    return ok != 0u;
-}
-__device__ __forceinline__ bool elect_one() {
-    unsigned pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0u;
-}
-__device__ __forceinline__ void st_bf16(unsigned char* tile, int row, int col, float v) {
-    *reinterpret_cast<unsigned short*>(tile + sw_elem(row, col)) = (unsigned short)(pack_bf16(v, 0.0f) & 0xffffu);
-}
 // an operand tile (or a TMEM read) of this warp is complete: make the generic-proxy writes visible to the tensor core, converge, and let
 // one lane arrive on the stream's "tile written" barriers (count 8 = the stream's warps): the chain issuer's, and for the tiles the
 // weight-gradient batches read (dO, G2, G1) the accumulate warp's too
@@ -133,8 +111,8 @@ __device__ __forceinline__ void tile_written(unsigned mb_rdy, int lane) {
     fence_before();
     __syncwarp();
     if (lane == 0) {
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(mb_rdy) : "memory");
-        if (ACC) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(mb_rdy + 8) : "memory");
+        mbar_arrive(mb_rdy);
+        if (ACC) mbar_arrive(mb_rdy + 8);
     }
 }
 
@@ -246,9 +224,9 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
             mbar_init(smem_u32(&S.mbar[s][7]), EPI / 32);
         }
         mbar_init(smem_u32(&S.mbar_w), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
         const unsigned mbw = smem_u32(&S.mbar_w);      // this net's W0 | W1 blocks of the prebuilt bf16 image: two bulk copies
-        expect_tx(mbw, 8192 + 8192);
+        mbar_expect_tx(mbw, 8192 + 8192);
         bulk_load(smem_u32(S.W0), wimg + KIN_WIMG_W0 + net * 8192, 8192, mbw);
         bulk_load(smem_u32(S.W1), wimg + KIN_WIMG_W1 + net * 8192, 8192, mbw);
     }
@@ -332,12 +310,12 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
             const unsigned loss_bytes = net == 0 ? 2u * 1792u + 4u * 256u : 2u * 256u;
             auto stage_x = [&](int s, int t0, int b) {           // elected lane only
                 const unsigned mb = mb0 + s * 64 + 24 + 8 * b;
-                expect_tx(mb, TILE);
+                mbar_expect_tx(mb, TILE);
                 bulk_load(aS0 + s * (unsigned)sizeof(StreamTiles) + b * TILE, img + (size_t)(t0 >> 1) * TILE, TILE, mb);
             };
             auto stage_loss = [&](int s, int t0, int t1) {       // elected lane only
                 const unsigned mb = mb0 + s * 64 + 40;
-                expect_tx(mb, loss_bytes);
+                mbar_expect_tx(mb, loss_bytes);
                 if (net == 0) {
                     bulk_load(aAct + s * 3584, action + (size_t)t0 * 448, 1792u, mb);
                     bulk_load(aAct + s * 3584 + 1792, action + (size_t)t1 * 448, 1792u, mb);
@@ -380,7 +358,7 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
                     const int si = itv[s];
                     if (k == 3 ? (ct3 != si || cs3 != s) : (k == 4 ? (ct4 != si || cs4 != s) : (ct5 != si || cs5 != s))) continue;      // not its turn
                     const unsigned mb = mb0 + s * 64;
-                    if (!mbar_test(mb + 56, pr[s])) continue;
+                    if (!mbar_test_wait(mb + 56, pr[s])) continue;
                     pr[s] ^= 1u;
                     fence_after();
                     T3_MARK(6);

@@ -1,5 +1,5 @@
 // kin_rollout_tc16.cu -- K2-TC: the fused policy-in-loop Approach -> Finisher rollout, actor MLP on the 5th-generation tensor
-// cores (tcgen05.mma kind::f16, fp16 operands, fp32 accumulators in TMEM).  Round-2 rewrite of kin_rollout_tc.cu (TF32).
+// cores (tcgen05.mma kind::f16, fp16 operands, fp32 accumulators in TMEM).  Round-2 rewrite of the earlier TF32 kernel.
 //
 // Mapping (unchanged): one episode <-> one thread <-> one row of the A operand <-> one TMEM lane; a CTA carries up to four
 // independent 128-episode tiles that share one staged copy of the policy; a batch that fits one wave is spread evenly over
@@ -107,7 +107,7 @@ __device__ __forceinline__ void tile_sync16(Tile16& c, int layer, int sid) {
             TC16_STAMP(6 + layer);
         }
     }
-    mbar_wait(c.mbar_saddr, c.parity);
+    mbar_wait_or_trap(c.mbar_saddr, c.parity);
     TC16_STAMP(3 + layer);
     c.parity ^= 1u;
 }
@@ -144,12 +144,10 @@ __device__ __forceinline__ bool mlp16(Tile16& c, const unsigned* w, float* act, 
     tile_sync16<ISS, AT>(c, 2, sid);
     umma::fence_after();
     {
-        unsigned r[8];
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(c.tmem_row) : "memory");
-        tmem_ld_wait();
+        float o[8];
+        tmem_ld8(c.tmem_row, o);
 #pragma unroll
-        for (int i = 0; i < NJ; ++i) act[i] = clampf(__uint_as_float(r[i]), -1.0f, 1.0f);
+        for (int i = 0; i < NJ; ++i) act[i] = clampf(o[i], -1.0f, 1.0f);
     }
     return true;
 }
@@ -252,7 +250,7 @@ kin_rollout_tc16_kernel(const __grid_constant__ KinEnvParams PA, const __grid_co
             S.arrive[i] = 0u;
             S.run_stamp[i] = 0;
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        umma::fence_mbar_init();
     }
     load_weights(S, pol_a, KIN_MODE_APPROACH, tid, (int)blockDim.x);
     const bool env_thread = tid < env_threads;

@@ -10,38 +10,24 @@
 // kin_ppo_bootstrap -> kin_route_reset_sampled, five launches per time step) stays as the restatement this kernel is replayed
 // against (tests/test_gpu_ppo.py::test_fused_route_collection_replays_through_the_step_kernels).
 //
-// Mapping as in kin_collect.cu: one replica <-> one thread <-> one row of the A operand <-> one TMEM lane; a CTA holds TILES
-// independent 128-replica tiles on named barriers sharing one bf16 copy of the weights.  Per step and tile:
-//   X = [obs80 | 1 | 0]  bf16, two SWIZZLE_128B K-major tiles (columns 0..63 | 64..127, 96 used)
-//   Z = X [W0a;W0c]^T            128 x 128 x 96   -> tanh -> H1 (actor half over X's first tile, critic half over its second)
-//   Z = H1a W1a^T | H1c W1c^T    2 x (128 x 64 x 64) -> tanh(+b1) -> H2 in place
-//   O = H2a WOa^T + H2c WOc^T    128 x 16 x 64    -> 7 action means + value
-// The observation goes to the rollout buffer as fp32 rows ([T + 1][n][80]: what kin_ppo_grad_tc<80> consumes).  Episodes that hit
-// the time limit append their terminal observation to a list; kin_ppo_bootstrap_list adds gamma * V(terminal_obs) afterwards.
-#include "kin_ppo_layout.cuh"
+// The policy half is kin_collect_policy.cuh, shared with K4; here X = [obs80 | 1 | 0] spans two K tiles (K = 96, 6 layer-1 MMAs)
+// and the second one is reused for the critic's activations.  The observation goes to the rollout buffer as fp32 rows
+// ([T + 1][n][80]: what kin_ppo_grad_tc<80> consumes).  Episodes that hit the time limit append their terminal observation to a
+// list; kin_ppo_bootstrap_list adds gamma * V(terminal_obs) afterwards.
+#include "kin_collect_policy.cuh"
 #include "kin_route_core.cuh"
-#include "kin_umma.cuh"
 
 namespace kin {
 
 using namespace umma;
 
-constexpr int RC_ROWS = 128;
-constexpr int RC_TILE_BYTES = RC_ROWS * 128;
 constexpr int RC_IN = KIN_ROUTE_OBS_DIM;      // 80
-constexpr float kHalfLog2PiR = 0.91893853320467274178f;
 
 template <int TILES>
 struct __align__(1024) RouteCollectSmem {
-    unsigned char XH[TILES][2][RC_TILE_BYTES];   // [.][0]: X columns 0..63, then actor H1 / H2; [.][1]: X columns 64..127, then critic H1 / H2
-    unsigned char W0[2][RC_TILE_BYTES];          // [k tile][128 rows: actor 0..63 | critic 64..127][64 cols]; column 80 (tile 1, col 16) = b0
-    unsigned char W1[2][64 * 128];
-    unsigned char WO[2][16 * 128];
-    float b1[128];
-    float bo[8];
-    float ls[8];
-    float sig[8];
-    unsigned long long mbar[TILES];
+    unsigned char XH[TILES][2][AC_TILE_BYTES];   // [.][0]: X columns 0..63, then actor H1 / H2; [.][1]: X columns 64..127, then critic H1 / H2
+    AcWeights<2> w;
+    unsigned long long mbar[TILES][1];
     unsigned tmem_base;
     alignas(16) float q_table[ROUTE_MAX_SMEM_WP * KIN_NJ];   // waypoint joint vectors for the nearest-waypoint scan (n <= 1024)
 };
@@ -63,193 +49,26 @@ struct RouteCollectOut {
     int boot_cap;
 };
 
-struct RTile {
-    unsigned char *X0, *X1;
-    unsigned aX0, aX1, aW0a, aW0b, aW1a, aW1c, aWOa, aWOc, mb, tz_mma, tz_row;
-    unsigned par;
-    int tile, row;
-};
-
-__device__ __forceinline__ bool rc_elect() {
-    unsigned pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0u;
-}
-__device__ __forceinline__ void rc_tile_bar(int tile) { asm volatile("bar.sync %0, %1;" ::"r"(tile + 1), "r"(RC_ROWS) : "memory"); }
-
-// actor + critic forward of the tile's 128 observations (80 floats each); collective over the tile's 128 threads.
-// out[0..6] = action means, out[7] = value.
-template <int TILES>
-__device__ __forceinline__ void route_policy_forward_tc(RouteCollectSmem<TILES>& S, RTile& c, const float* o, float* out) {
-    // ---- X image: 80 obs | 1 | zeros, two K tiles
-#pragma unroll
-    for (int ch = 0; ch < 8; ++ch)
-        *reinterpret_cast<uint4*>(c.X0 + sw_chunk(c.row, ch)) = make_uint4(pack_bf16(o[8 * ch], o[8 * ch + 1]), pack_bf16(o[8 * ch + 2], o[8 * ch + 3]),
-                                                                            pack_bf16(o[8 * ch + 4], o[8 * ch + 5]), pack_bf16(o[8 * ch + 6], o[8 * ch + 7]));
-#pragma unroll
-    for (int ch = 0; ch < 2; ++ch)
-        *reinterpret_cast<uint4*>(c.X1 + sw_chunk(c.row, ch)) = make_uint4(pack_bf16(o[64 + 8 * ch], o[65 + 8 * ch]), pack_bf16(o[66 + 8 * ch], o[67 + 8 * ch]),
-                                                                            pack_bf16(o[68 + 8 * ch], o[69 + 8 * ch]), pack_bf16(o[70 + 8 * ch], o[71 + 8 * ch]));
-    *reinterpret_cast<uint4*>(c.X1 + sw_chunk(c.row, 2)) = make_uint4(0x00003F80u, 0u, 0u, 0u);      // column 80 = 1 (bias carrier)
-    *reinterpret_cast<uint4*>(c.X1 + sw_chunk(c.row, 3)) = make_uint4(0u, 0u, 0u, 0u);               // columns 88..95 (the critic's H wrote here)
-    fence_async_smem();
-    fence_before();
-    rc_tile_bar(c.tile);
-    if (c.row < 32 && rc_elect()) {
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 128, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX0 + k * 32), desc_k(c.aW0a + k * 32), id, k > 0);
-#pragma unroll
-        for (int k = 0; k < 2; ++k) mma_bf16(c.tz_mma, desc_k(c.aX1 + k * 32), desc_k(c.aW0b + k * 32), id, 1u);
-        commit(c.mb);
-    }
-    mbar_wait(c.mb, c.par);
-    c.par ^= 1u;
-    fence_after();
-    // ---- H1 = tanh(Z): columns 0..63 actor -> X0's place, 64..127 critic -> X1's place
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        float v[32];
-        tmem_ld32(c.tz_row + q * 32, v);
-        unsigned char* dst = (q < 2) ? c.X0 : c.X1;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            unsigned p[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) p[e] = pack_bf16(tanh_fast(v[8 * j + 2 * e]), tanh_fast(v[8 * j + 2 * e + 1]));
-            *reinterpret_cast<uint4*>(dst + sw_chunk(c.row, (q & 1) * 4 + j)) = make_uint4(p[0], p[1], p[2], p[3]);
-        }
-    }
-    fence_async_smem();
-    fence_before();
-    rc_tile_bar(c.tile);
-    if (c.row < 32 && rc_elect()) {
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 64, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX0 + k * 32), desc_k(c.aW1a + k * 32), id, k > 0);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma + 64, desc_k(c.aX1 + k * 32), desc_k(c.aW1c + k * 32), id, k > 0);
-        commit(c.mb);
-    }
-    mbar_wait(c.mb, c.par);
-    c.par ^= 1u;
-    fence_after();
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        float v[32];
-        tmem_ld32(c.tz_row + q * 32, v);
-        unsigned char* dst = (q < 2) ? c.X0 : c.X1;
-        const float* b = S.b1 + q * 32;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            unsigned p[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e)
-                p[e] = pack_bf16(tanh_fast(v[8 * j + 2 * e] + b[8 * j + 2 * e]), tanh_fast(v[8 * j + 2 * e + 1] + b[8 * j + 2 * e + 1]));
-            *reinterpret_cast<uint4*>(dst + sw_chunk(c.row, (q & 1) * 4 + j)) = make_uint4(p[0], p[1], p[2], p[3]);
-        }
-    }
-    fence_async_smem();
-    fence_before();
-    rc_tile_bar(c.tile);
-    if (c.row < 32 && rc_elect()) {
-        fence_after();
-        constexpr unsigned id = idesc_bf16(128, 16, false, false);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX0 + k * 32), desc_k(c.aWOa + k * 32), id, k > 0);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) mma_bf16(c.tz_mma, desc_k(c.aX1 + k * 32), desc_k(c.aWOc + k * 32), id, 1u);
-        commit(c.mb);
-    }
-    mbar_wait(c.mb, c.par);
-    c.par ^= 1u;
-    fence_after();
-    float r[16];
-    tmem_ld16(c.tz_row, r);
-    fence_before();
-#pragma unroll
-    for (int d = 0; d < 8; ++d) out[d] = r[d] + S.bo[d];
-}
-
-__device__ __forceinline__ void store_obs_row80(float* dst, const float* o) {
-    float4* d4 = reinterpret_cast<float4*>(dst);
-#pragma unroll
-    for (int k = 0; k < RC_IN / 4; ++k) d4[k] = make_float4(o[4 * k], o[4 * k + 1], o[4 * k + 2], o[4 * k + 3]);
-}
-
 template <int TILES, bool SEQ>
-__global__ void __launch_bounds__(TILES * RC_ROWS, 1)
+__global__ void __launch_bounds__(TILES * AC_ROWS, 1)
 kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, const __grid_constant__ KinRouteResetParams C, float* __restrict__ state,
                          int stride, int n, const float* __restrict__ params, int T, uint64_t noise_seed, uint32_t step0, uint64_t reset_seed,
                          int reset_streak, RouteCollectOut out) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     RouteCollectSmem<TILES>& S = *reinterpret_cast<RouteCollectSmem<TILES>*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
-    const PpoOffsets O = ppo_offsets(RC_IN);
-    const int tid = threadIdx.x, warp = tid >> 5;
-    constexpr int NT = TILES * RC_ROWS;
+    const int tid = threadIdx.x;
+    constexpr int NT = TILES * AC_ROWS;
 
-    // ---- weights -> bf16 operand tiles (both nets), converted here from the flat fp32 parameters -----------------------------
-    for (int i = tid; i < 2 * 128 * 64; i += NT) {       // W0: [k tile][net row][col]
-        const int kt = i >> 13, nn = (i >> 6) & 127, kc = i & 63, k = kt * 64 + kc, u = nn & 63;
-        const int wbase = (nn < 64) ? O.pi_w0 : O.vf_w0, bbase = (nn < 64) ? O.pi_b0 : O.vf_b0;
-        const float v = k < RC_IN ? __ldg(params + wbase + u * RC_IN + k) : (k == RC_IN ? __ldg(params + bbase + u) : 0.0f);
-        *reinterpret_cast<unsigned short*>(S.W0[kt] + sw_elem(nn, kc)) = (unsigned short)(pack_bf16(v, 0.0f) & 0xffffu);
-    }
-    for (int i = tid; i < 2 * 4096; i += NT) {
-        const int nt = i >> 12, u = (i >> 6) & 63, k = i & 63;
-        *reinterpret_cast<unsigned short*>(S.W1[nt] + sw_elem(u, k)) =
-            (unsigned short)(pack_bf16(__ldg(params + (nt ? O.vf_w1 : O.pi_w1) + u * 64 + k), 0.0f) & 0xffffu);
-    }
-    {
-        uint4* zw = reinterpret_cast<uint4*>(S.WO);
-        for (int i = tid; i < 2 * 16 * 128 / 16; i += NT) zw[i] = make_uint4(0u, 0u, 0u, 0u);
-    }
-    __syncthreads();
-    for (int i = tid; i < 7 * 64; i += NT)
-        *reinterpret_cast<unsigned short*>(S.WO[0] + sw_elem(i >> 6, i & 63)) = (unsigned short)(pack_bf16(__ldg(params + O.act_w + i), 0.0f) & 0xffffu);
-    if (tid < 64) *reinterpret_cast<unsigned short*>(S.WO[1] + sw_elem(7, tid)) = (unsigned short)(pack_bf16(__ldg(params + O.val_w + tid), 0.0f) & 0xffffu);
-    if (tid < 128) S.b1[tid] = __ldg(params + (tid < 64 ? O.pi_b1 + tid : O.vf_b1 + tid - 64));
-    if (tid < 8) {
-        const float ls = tid < 7 ? __ldg(params + O.log_std + tid) : 0.0f;
-        S.bo[tid] = tid < 7 ? __ldg(params + O.act_b + tid) : __ldg(params + O.val_b);
-        S.ls[tid] = ls;
-        S.sig[tid] = expf(ls);
-    }
+    convert_weights<RC_IN, 2, NT>(S.w, params, tid);
+    load_vectors<RC_IN>(S.w, params, tid);
     load_q_table(S.q_table, R, tid, NT);
-    if (warp == 0) tmem_alloc(smem_u32(&S.tmem_base), TILES * 128);
-    if (tid < TILES) {
-        mbar_init(smem_u32(&S.mbar[tid]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    fence_async_smem();
-    fence_before();
-    __syncthreads();
-    fence_after();
-
-    RTile c;
-    c.tile = tid >> 7;
-    c.row = tid & 127;
-    c.X0 = S.XH[c.tile][0];
-    c.X1 = S.XH[c.tile][1];
-    c.aX0 = smem_u32(c.X0);
-    c.aX1 = smem_u32(c.X1);
-    c.aW0a = smem_u32(S.W0[0]);
-    c.aW0b = smem_u32(S.W0[1]);
-    c.aW1a = smem_u32(S.W1[0]);
-    c.aW1c = smem_u32(S.W1[1]);
-    c.aWOa = smem_u32(S.WO[0]);
-    c.aWOc = smem_u32(S.WO[1]);
-    c.mb = smem_u32(&S.mbar[c.tile]);
-    c.tz_mma = S.tmem_base + c.tile * 128;
-    c.tz_row = c.tz_mma + ((unsigned)((warp & 3) * 32) << 16);
-    c.par = 0u;
+    init_tiles<TILES, 1>(S, tid);
+    AcTile<2> c = tile_of<2, 1>(S, tid);
 
     const int gtile = blockIdx.x * TILES + c.tile;
-    const int n_tiles = n / RC_ROWS;
+    const int n_tiles = n / AC_ROWS;
     const bool live = gtile < n_tiles;                        // tile-uniform
-    const int env = (live ? gtile : 0) * RC_ROWS + c.row;
+    const int env = (live ? gtile : 0) * AC_ROWS + c.row;
     const float* table = R.n <= ROUTE_MAX_SMEM_WP ? S.q_table : R.q;
 
     EnvRegs s;
@@ -275,23 +94,11 @@ kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, co
             {
                 float o[RC_IN];
                 observe(o);
-                store_obs_row80(out.obs + idx * RC_IN, o);
-                route_policy_forward_tc<TILES>(S, c, o, mv);
+                store_row<RC_IN>(out.obs + idx * RC_IN, o);
+                policy_forward<RC_IN, false>(S.w, c, o, nullptr, mv);
             }
-            // ---- a = mean + sigma * eps, log N(a): the draws of kin_policy_act
-            float a[NJ], lp = 0.0f;
-            {
-                Philox rng(noise_seed, (unsigned)env, step0 + (uint32_t)t);
-                float eps[8];
-#pragma unroll
-                for (int k = 0; k < 8; k += 2) eps[k] = gauss_pair(rng, &eps[k + 1]);
-#pragma unroll
-                for (int k = 0; k < NJ; ++k) {
-                    a[k] = fmaf(S.sig[k], eps[k], mv[k]);
-                    lp += -0.5f * eps[k] * eps[k] - S.ls[k] - kHalfLog2PiR;
-                    out.action[idx * NJ + k] = a[k];
-                }
-            }
+            float a[NJ];
+            const float lp = sample_action(S.w, noise_seed, (unsigned)env, step0 + (uint32_t)t, mv, a, out.action + idx * NJ);
             out.logp[idx] = lp;
             out.value[idx] = mv[7];
             out.episode_start[idx] = (uint8_t)start;
@@ -303,15 +110,7 @@ kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, co
             if (SEQ && rr.index != index_before) goal_dirty = true;
             const bool finished = (ro.done & (KIN_DONE_TERMINATED | KIN_DONE_TRUNCATED)) != 0u;
             if (finished) {
-                if ((ro.done & KIN_DONE_TRUNCATED) && !(ro.done & KIN_DONE_TERMINATED)) {   // TimeLimit bootstrap list: the terminal observation
-                    const int slot = atomicAdd(out.boot_count, 1);
-                    if (slot < out.boot_cap) {
-                        float o[RC_IN];
-                        observe(o);
-                        out.boot_index[slot] = (int)idx;
-                        store_obs_row80(out.boot_obs + (size_t)slot * RC_IN, o);
-                    }
-                }
+                push_truncated<RC_IN>(out, ro.done, idx, observe);      // the terminal observation
                 Philox rng(reset_seed, (uint32_t)env, step0 + (uint32_t)t);
                 float gq[NJ];
                 sample_route_reset_dev(P, R, C, rng, s, rr, gq);
@@ -327,8 +126,8 @@ kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, co
         {
             float o[RC_IN], mv[8];
             observe(o);
-            store_obs_row80(out.obs + ((size_t)T * n + env) * RC_IN, o);
-            route_policy_forward_tc<TILES>(S, c, o, mv);
+            store_row<RC_IN>(out.obs + ((size_t)T * n + env) * RC_IN, o);
+            policy_forward<RC_IN, false>(S.w, c, o, nullptr, mv);
             out.last_value[env] = mv[7];
         }
         out.start_io[env] = (uint8_t)start;
@@ -345,31 +144,16 @@ kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, co
         st_row_u(state, stride, KIN_ROW_ROUTE, env, (unsigned)rr.index | ((unsigned)min(rr.streak, 0xffff) << 16));
         st_row_u(state, stride, KIN_ROW_ROUTE2, env, (unsigned)rr.last | ((unsigned)min(rr.completed, 0xffff) << 16));
     }
-    fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(S.tmem_base, TILES * 128);
+    release_tiles<TILES>(S, tid);
 }
 
 template <int TILES>
 static cudaError_t launch_route_collect(const KinHandle* h, const RouteView& R, const KinRouteResetParams& C, float* state, int stride, int n, const float* params,
                                         int T, uint64_t noise_seed, uint32_t step0, uint64_t reset_seed, int seq, int reset_streak, const RouteCollectOut& out,
                                         cudaStream_t st) {
-    const size_t smem = sizeof(RouteCollectSmem<TILES>) + 1024;
-    const int n_tiles = n / RC_ROWS;
-    const int grid = (n_tiles + TILES - 1) / TILES;
-    cudaError_t e;
-    if (seq) {
-        e = cudaFuncSetAttribute(kin_route_collect_kernel<TILES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kin_route_collect_kernel<TILES, true><<<grid, TILES * RC_ROWS, smem, st>>>(h->params, R, C, state, stride, n, params, T, noise_seed, step0, reset_seed,
-                                                                                 reset_streak, out);
-    } else {
-        e = cudaFuncSetAttribute(kin_route_collect_kernel<TILES, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        kin_route_collect_kernel<TILES, false><<<grid, TILES * RC_ROWS, smem, st>>>(h->params, R, C, state, stride, n, params, T, noise_seed, step0, reset_seed,
-                                                                                  reset_streak, out);
-    }
-    return cudaGetLastError();
+    auto kernel = seq ? kin_route_collect_kernel<TILES, true> : kin_route_collect_kernel<TILES, false>;
+    return launch_tiles<TILES>(kernel, sizeof(RouteCollectSmem<TILES>) + 1024, n, st, h->params, R, C, state, stride, n, params, T, noise_seed, step0,
+                               reset_seed, reset_streak, out);
 }
 
 }  // namespace kin
@@ -386,20 +170,14 @@ extern "C" int kin_route_collect(void* handle, const KinRouteTable* host_route, 
     if (!state || !params || !obs || !action || !logp || !value || !reward || !done || !episode_start || !route_flags || !start_io || !last_value ||
         !boot_count || !boot_index || !boot_obs || boot_cap <= 0 || n_steps <= 0)
         return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_collect: null buffer or bad sizes");
-    if (n_envs <= 0 || (n_envs % RC_ROWS) != 0 || stride < n_envs || (stride % 32) != 0)
+    if (n_envs <= 0 || (n_envs % AC_ROWS) != 0 || stride < n_envs || (stride % 32) != 0)
         return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_collect: n_envs must be a positive multiple of 128 (one GEMM tile), stride % 32 == 0");
     if (((uintptr_t)obs & 15u) || ((uintptr_t)boot_obs & 15u)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_collect: obs / boot_obs must be 16-byte aligned");
     for (int m = 0; m < 5; ++m)
         if (host_reset->index_lo[m] < 0 || host_reset->index_hi[m] >= host_route->n_waypoints || host_reset->index_lo[m] > host_reset->index_hi[m])
             return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_collect: waypoint range outside the route");
     cudaStream_t st = (cudaStream_t)stream;
-    int tiles = tiles_per_cta;
-    if (tiles <= 0) {   // fewest tiles per CTA that still fits the batch in one wave of CTAs (one CTA per SM)
-        int sms = 148, dev = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const int n_tiles = n_envs / RC_ROWS;
-        tiles = n_tiles <= sms ? 1 : (n_tiles <= 2 * sms ? 2 : 4);
-    }
+    const int tiles = collect_tiles_per_cta(tiles_per_cta, n_envs);
     RouteCollectOut out{obs, action, logp, value, reward, done, episode_start, route_flags, start_io, last_value, boot_count, boot_index, boot_obs, boot_cap};
     cudaError_t e = cudaMemsetAsync(boot_count, 0, sizeof(int), st);
     if (e != cudaSuccess) return kin_fail_cuda(e, "kin_route_collect: memset");

@@ -2,7 +2,7 @@
 // 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM); the env / route arithmetic is the code the
 // strict-fp32 probe (kin_route.cu) runs.
 //
-// One replica <-> one thread <-> one row of the A tile <-> one TMEM lane, as in kin_rollout_tc.cu.  The route observation is 80
+// One replica <-> one thread <-> one row of the A tile <-> one TMEM lane.  The route observation is 80
 // floats (+ a constant 1 that carries the layer-1 bias, zero pad to K = 96), so the A tile has three 128-byte K chunks (48 KB) and
 // layer 1 is 12 MMAs of K = 8; the hidden layers reuse the first two chunks (K = 64).  A CTA holds up to three tiles (12 warps)
 // on named barriers sharing one copy of the weights (42 KB): 186 KB of shared memory, 192 TMEM columns (256 allocated).
@@ -13,9 +13,48 @@
 // Numerics: TF32 operands + tanh.approx move actions by O(1e-3) like the Approach -> Finisher tensor-core rollout; the strict
 // probe stays the parity path (tests/test_gpu_route.py compares the two prefix distributions).
 #include "kin_route_core.cuh"
-#include "kin_tc_mlp.cuh"
+#include "kin_umma.cuh"
 
 namespace kin {
+
+using namespace umma;
+
+// ---- kind::tf32 operands: fp32 words, [rows][32 floats] = 128-byte rows per K chunk, SWIZZLE_128B, K-major
+constexpr int TC_TILE = 128;                   // replicas per tile == UMMA M == TMEM lanes
+constexpr int TC_K = 64;                       // padded reduction width of the hidden layers
+constexpr int TC_HID = 64;
+constexpr int CHUNK_FLOATS_A = TC_TILE * 32;   // one 128-byte-wide K chunk of an A tile: 128 rows x 32 floats
+constexpr int CHUNK_FLOATS_W = TC_HID * 32;    // 64 rows x 32 floats
+constexpr int W_FLOATS = 2 * CHUNK_FLOATS_W;
+constexpr int CHUNK_FLOATS_WO = 8 * 32;        // output layer: 8 rows (7 actions + zero row)
+constexpr int WO_FLOATS = 2 * CHUNK_FLOATS_WO;
+
+struct DevPolicyTc {
+    const float *w0, *b0, *w1, *b1, *wo, *bo;
+};
+
+// Round-to-nearest (ties away) TF32: cvt.rna.tf32 is "add half an ulp of the 10-bit mantissa, clear the low 13 bits"; the
+// tensor core ignores those 13 bits of a kind::tf32 operand, so the add alone feeds it the same operand (values here are finite
+// and far from overflow: observations in [-1, 1], tanh outputs, trained weights).
+__device__ __forceinline__ float to_tf32(float x) { return __uint_as_float(__float_as_uint(x) + 0x1000u); }
+
+// float offset of element (row, k) inside a K-major SWIZZLE_128B operand whose K chunks hold `rows` rows each
+__device__ __forceinline__ int sw128_offset(int row, int k, int chunk_floats) {
+    const int chunk = k >> 5, kk = k & 31;
+    return chunk * chunk_floats + row * 32 + ((((kk >> 2) ^ (row & 7)) << 2) | (kk & 3));
+}
+
+// instruction descriptor: D fp32, A/B tf32, both K-major, N>>3 at bit 17, M>>4 at bit 24
+__host__ __device__ constexpr unsigned idesc_tf32(int M, int N) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(N >> 3) << 17) | ((unsigned)(M >> 4) << 24);
+}
+
+// write 4 consecutive K elements [k4*4, k4*4+4) of this thread's A row (already TF32-rounded)
+__device__ __forceinline__ void a_store4(float* A, int row, int k4, float x0, float x1, float x2, float x3) {
+    const int chunk = k4 >> 3, j = k4 & 7;
+    float4* dst = reinterpret_cast<float4*>(A + chunk * CHUNK_FLOATS_A + row * 32 + ((j ^ (row & 7)) << 2));
+    *dst = make_float4(x0, x1, x2, x3);
+}
 
 constexpr int RTC_TILES = 3;
 constexpr int RTC_MAX_THREADS = TC_TILE * RTC_TILES;
@@ -44,14 +83,14 @@ struct RtcTile {
 
 template <int KSTEPS>
 __device__ __forceinline__ void issue_layer_k(unsigned a_saddr, unsigned w_saddr, int w_chunk_bytes, unsigned tmem_d, unsigned idesc, unsigned mbar_saddr) {
-    tc_fence_after();
+    fence_after();
 #pragma unroll
     for (int k = 0; k < KSTEPS; ++k) {
         const unsigned a_off = (k >> 2) * (CHUNK_FLOATS_A * 4) + (k & 3) * 32;
         const unsigned w_off = (k >> 2) * w_chunk_bytes + (k & 3) * 32;
-        umma_tf32(tmem_d, umma_desc(a_saddr + a_off), umma_desc(w_saddr + w_off), idesc, k > 0 ? 1u : 0u);
+        mma_tf32(tmem_d, desc_k(a_saddr + a_off), desc_k(w_saddr + w_off), idesc, k > 0 ? 1u : 0u);
     }
-    umma_commit(mbar_saddr);
+    commit(mbar_saddr);
 }
 
 // route observation [80] -> action [7]; collective over the tile's threads.  Returns false (without running the MLP) once no
@@ -68,49 +107,49 @@ __device__ __forceinline__ bool mlp_tc_route(RtcSmem& S, RtcTile& c, const float
 #pragma unroll
     for (int k4 = 21; k4 < RTC_K1 / 4; ++k4) a_store4(c.A, c.row, k4, 0.0f, 0.0f, 0.0f, 0.0f);
     fence_async_smem();
-    tc_fence_before();
-    tile_barrier(c.tile, c.tile_threads);
+    fence_before();
+    bar_sync(c.tile + 1, c.tile_threads);
     if (!(S.run_flags[fb][c.tile][0] | S.run_flags[fb][c.tile][1] | S.run_flags[fb][c.tile][2] | S.run_flags[fb][c.tile][3])) return false;
-    if (c.row < 32 && elect_one_tc()) issue_layer_k<RTC_K1 / 8>(c.a_saddr, c.w0_saddr, CHUNK_FLOATS_W * 4, c.tmem_d, umma_idesc(TC_TILE, TC_HID), c.mbar_saddr);
+    if (c.row < 32 && elect_one()) issue_layer_k<RTC_K1 / 8>(c.a_saddr, c.w0_saddr, CHUNK_FLOATS_W * 4, c.tmem_d, idesc_tf32(TC_TILE, TC_HID), c.mbar_saddr);
     mbar_wait(c.mbar_saddr, c.parity);
     c.parity ^= 1u;
-    tc_fence_after();
+    fence_after();
     float v[32];
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
         tmem_ld32(c.tmem_row + half * 32, v);
 #pragma unroll
         for (int j = 0; j < 8; ++j)
-            a_store4(c.A, c.row, half * 8 + j, to_tf32(tanh_approx(v[4 * j])), to_tf32(tanh_approx(v[4 * j + 1])),
-                     to_tf32(tanh_approx(v[4 * j + 2])), to_tf32(tanh_approx(v[4 * j + 3])));
+            a_store4(c.A, c.row, half * 8 + j, to_tf32(tanh_fast(v[4 * j])), to_tf32(tanh_fast(v[4 * j + 1])),
+                     to_tf32(tanh_fast(v[4 * j + 2])), to_tf32(tanh_fast(v[4 * j + 3])));
     }
     fence_async_smem();
-    tc_fence_before();
-    tile_barrier(c.tile, c.tile_threads);
-    if (c.row < 32 && elect_one_tc()) issue_layer_k<TC_K / 8>(c.a_saddr, c.w1_saddr, CHUNK_FLOATS_W * 4, c.tmem_d, umma_idesc(TC_TILE, TC_HID), c.mbar_saddr);
+    fence_before();
+    bar_sync(c.tile + 1, c.tile_threads);
+    if (c.row < 32 && elect_one()) issue_layer_k<TC_K / 8>(c.a_saddr, c.w1_saddr, CHUNK_FLOATS_W * 4, c.tmem_d, idesc_tf32(TC_TILE, TC_HID), c.mbar_saddr);
     mbar_wait(c.mbar_saddr, c.parity);
     c.parity ^= 1u;
-    tc_fence_after();
+    fence_after();
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
         tmem_ld32(c.tmem_row + half * 32, v);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
             const float* b = S.b1 + half * 32 + 4 * j;
-            a_store4(c.A, c.row, half * 8 + j, to_tf32(tanh_approx(v[4 * j] + b[0])), to_tf32(tanh_approx(v[4 * j + 1] + b[1])),
-                     to_tf32(tanh_approx(v[4 * j + 2] + b[2])), to_tf32(tanh_approx(v[4 * j + 3] + b[3])));
+            a_store4(c.A, c.row, half * 8 + j, to_tf32(tanh_fast(v[4 * j] + b[0])), to_tf32(tanh_fast(v[4 * j + 1] + b[1])),
+                     to_tf32(tanh_fast(v[4 * j + 2] + b[2])), to_tf32(tanh_fast(v[4 * j + 3] + b[3])));
         }
     }
     fence_async_smem();
-    tc_fence_before();
-    tile_barrier(c.tile, c.tile_threads);
-    if (c.row < 32 && elect_one_tc()) issue_layer_k<TC_K / 8>(c.a_saddr, c.wo_saddr, CHUNK_FLOATS_WO * 4, c.tmem_d, umma_idesc(TC_TILE, 8), c.mbar_saddr);
+    fence_before();
+    bar_sync(c.tile + 1, c.tile_threads);
+    if (c.row < 32 && elect_one()) issue_layer_k<TC_K / 8>(c.a_saddr, c.wo_saddr, CHUNK_FLOATS_WO * 4, c.tmem_d, idesc_tf32(TC_TILE, 8), c.mbar_saddr);
     mbar_wait(c.mbar_saddr, c.parity);
     c.parity ^= 1u;
-    tc_fence_after();
+    fence_after();
     float a8[8];
     tmem_ld8(c.tmem_row, a8);
-    tc_fence_before();
+    fence_before();
 #pragma unroll
     for (int i = 0; i < KIN_NJ; ++i) act[i] = clampf(a8[i] + S.bo[i], -1.0f, 1.0f);
     return true;
@@ -133,14 +172,11 @@ kin_route_probe_tc_kernel(const __grid_constant__ KinEnvParams P, RouteView R, D
     c.flag_buf = 0;
     const int n_tiles_cta = ((int)blockDim.x + TC_TILE - 1) / TC_TILE;
     const unsigned tmem_cols = n_tiles_cta == 1 ? 64u : (n_tiles_cta == 2 ? 128u : 256u);
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&S.tmem_base)), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc(smem_u32(&S.tmem_base), tmem_cols);
     if (tid == 0) {
 #pragma unroll
         for (int i = 0; i < RTC_TILES; ++i) mbar_init(smem_u32(&S.mbar[i]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init();
     }
     if (tid < 2 * RTC_TILES * 4) (&S.run_flags[0][0][0])[tid] = 0;
     // stage the actor into the swizzled B-operand images
@@ -160,9 +196,9 @@ kin_route_probe_tc_kernel(const __grid_constant__ KinEnvParams P, RouteView R, D
     for (int i = tid; i < TC_HID; i += (int)blockDim.x) S.b1[i] = __ldg(pol.b1 + i);
     if (tid < 8) S.bo[tid] = tid < KIN_NJ ? __ldg(pol.bo + tid) : 0.0f;
     fence_async_smem();
-    tc_fence_before();
+    fence_before();
     __syncthreads();
-    tc_fence_after();
+    fence_after();
     const unsigned tmem_base = S.tmem_base;
     c.a_saddr = smem_u32(c.A);
     c.w0_saddr = smem_u32(S.W0);
@@ -234,9 +270,9 @@ kin_route_probe_tc_kernel(const __grid_constant__ KinEnvParams P, RouteView R, D
         for (int off = 16; off > 0; off >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, off);
         if ((tid & 31) == 0 && mine) atomicAdd(env_steps, mine);
     }
-    tc_fence_before();
+    fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
+    if (warp == 0) tmem_dealloc(tmem_base, tmem_cols);
 }
 
 }  // namespace kin
@@ -253,7 +289,7 @@ extern "C" int kin_route_probe_tc(void* handle, const KinRouteTable* host_route,
     int dev = 0, sms = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    // balanced launch (as kin_rollout_tc): a batch that fits one wave gets one CTA per SM with ceil(warps / SMs) warps
+    // balanced launch: a batch that fits one wave gets one CTA per SM with ceil(warps / SMs) warps
     const int warps = (n + 31) / 32;
     int w_cta = RTC_MAX_THREADS / 32;
     if (warps <= sms * w_cta) w_cta = (warps + sms - 1) / sms;

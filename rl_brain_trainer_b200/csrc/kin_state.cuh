@@ -6,6 +6,7 @@
 #include <cstdint>
 
 #include "kin_core.cuh"
+#include "kin_umma.cuh"
 
 namespace kin {
 
@@ -111,17 +112,16 @@ __device__ __forceinline__ void stage_obs_row(float* tile, int lane, const float
 
 __device__ __forceinline__ void bulk_store_tile(float* __restrict__ gdst, const float* tile, int bytes, int lane) {
     // make the generic-proxy smem writes visible to the async proxy, then one elected lane issues the copy
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    umma::fence_async_smem();
     __syncwarp();
     if (lane == 0 && bytes > 0) {
-        unsigned saddr = (unsigned)__cvta_generic_to_shared(tile);
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(saddr), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        umma::bulk_store(gdst, umma::smem_u32(tile), bytes);
+        umma::bulk_commit();
     }
 }
 // smem may be overwritten / the CTA may exit only after the bulk engine has READ the tile
 __device__ __forceinline__ void bulk_store_wait_read(int lane) {
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+    if (lane == 0) umma::bulk_wait_read();
     __syncwarp();
 }
 

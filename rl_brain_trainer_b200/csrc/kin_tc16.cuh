@@ -21,6 +21,8 @@
 namespace kin {
 namespace tc16 {
 
+using namespace umma;
+
 constexpr int TILE = 128;                  // episodes per tile == UMMA M == TMEM lanes
 constexpr int MAX_TILES = 4;               // tiles per CTA (the last one may be partial: 1..4 warps)
 constexpr int MAX_THREADS = TILE * MAX_TILES;
@@ -61,11 +63,6 @@ __device__ __forceinline__ unsigned pack_h2(float lo, float hi) {
     unsigned r;
     asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
     return r;
-}
-__device__ __forceinline__ unsigned tanh_h2(unsigned x) {
-    unsigned y;
-    asm("tanh.approx.f16x2 %0, %1;" : "=r"(y) : "r"(x));
-    return y;
 }
 // both halves clamped to [-1, 1]
 __device__ __forceinline__ unsigned clamp1_h2(unsigned x) {
@@ -168,56 +165,6 @@ __device__ __forceinline__ void mma_f16_ts(unsigned tmem_d, unsigned a_taddr, un
         "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %3, p;\n\t}"
         ::"r"(tmem_d), "r"(a_taddr), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(DESC_HI) : "memory");
 }
-__device__ __forceinline__ void tmem_st8(unsigned taddr, const unsigned* r) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-                 ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
-}
-__device__ __forceinline__ void tmem_st4(unsigned taddr, unsigned a, unsigned b, unsigned c, unsigned d) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-__device__ __forceinline__ bool elect_one() {
-    unsigned pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0u;
-}
-// mbarrier wait with a watchdog: a protocol bug must trap (the launch fails with an error) instead of hanging the GPU
-__device__ __forceinline__ void mbar_wait(unsigned saddr, unsigned parity) {
-    unsigned done = 0u;
-    for (unsigned spins = 0u; ; ++spins) {
-        asm volatile(
-            "{\n\t.reg .pred P1;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, P1;\n\t}"
-            : "=r"(done) : "r"(saddr), "r"(parity) : "memory");
-        if (done) return;
-        if (spins > (1u << 24)) __trap();   // each failed try_wait already suspends for a bounded time: >> seconds
-    }
-}
-// non-blocking-ish probe: returns after at most ~`hint_ns` (the hardware suspends the warp meanwhile, no issue slots burnt)
-__device__ __forceinline__ bool mbar_try_wait_hint(unsigned saddr, unsigned parity, unsigned hint_ns) {
-    unsigned done;
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, P1;\n\t}"
-        : "=r"(done) : "r"(saddr), "r"(parity), "r"(hint_ns) : "memory");
-    return done != 0u;
-}
-__device__ __forceinline__ bool mbar_test_wait(unsigned saddr, unsigned parity) {
-    unsigned done;
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, P1;\n\t}"
-        : "=r"(done) : "r"(saddr), "r"(parity) : "memory");
-    return done != 0u;
-}
-__device__ __forceinline__ void mbar_arrive(unsigned saddr) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(saddr) : "memory");
-}
-
 // "My part of the operand tile is written": every lane makes its generic-proxy stores visible to the async proxy, the warp
 // converges, lane 0 bumps the tile's counter.  Returns non-zero -- to the whole warp -- on the warp that arrived last;
 // that warp issues the tile's MMAs, nobody blocks on a CTA barrier.  With `stamp` the last arriver also reports whether some
@@ -236,24 +183,6 @@ __device__ __forceinline__ int tile_arrive(unsigned cnt_saddr, unsigned target, 
     }
     return __shfl_sync(0xffffffffu, last, 0);
 }
-
-// 16 raw accumulator words of this thread's TMEM lane; the values are valid after tmem_wait16 on the same registers
-__device__ __forceinline__ void tmem_ld16_raw(unsigned taddr, unsigned* r) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr) : "memory");
-}
-// tcgen05.wait::ld with the loaded registers as in/out operands, so no consumer of them can be scheduled above the wait
-__device__ __forceinline__ void tmem_wait16(unsigned* r) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]),
-                   "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15])
-                 :: "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // 16 accumulator columns -> tanh -> two 16-byte chunks (2 * ch2, 2 * ch2 + 1) of this thread's row of the H image
 __device__ __forceinline__ void tanh_store16(const unsigned* r, unsigned char* H, int row, int ch2) {
