@@ -837,6 +837,90 @@ int kin_ppo_adam(float *params, const float *grad, float *adam_m, float *adam_v,
  * nets as SWIZZLE_128B tiles, layer-1 bias folded in as column 56).  kin_ppo_adam(weight_image != NULL) keeps it current.   */
 int kin_ppo_pack_weights(const float *params, int in_dim, void *weight_image, void *stream);
 
+/* ---- populations: K independent PPO runs through the same launches ---------------------------------------------------------------
+ * A population member is one complete single-rank 56-input trainer (kin_ppo_collect + kin_ppo_grad_tc in image mode + kin_ppo_adam):
+ * its own parameters, Adam state, env state, rollout buffers, seeds and hyper-parameters.  The kin_pop_* launches below run one phase
+ * of ALL members at once, the member index on a grid dimension; each member's CTAs run the standalone kernel's body on that member's
+ * descriptor, so member k's results are bitwise those of the standalone calls on the same buffers.  Members share the env params
+ * (KinEnvParams bytes and policy mode), n_envs, n_steps and the minibatch shape.
+ * The caller owns a DEVICE array of n_members descriptors and re-uploads it when a pointer, seed, step or hyper-parameter changes.
+ * KIN_POP_MAX bounds n_members for two reasons.  kin_pop_adam passes every member's Adam bias corrections as a by-value kernel
+ * argument (2 x 64 floats, 512 B).  kin_pop_collect resets the members' bootstrap counts from one block of KIN_POP_MAX threads.
+ * 64 is also well past the sweep sizes the population serves (8 to 32 seeds / settings); larger sweeps run as several populations.
+ * New entry points only: no existing struct, signature or behaviour changed, so KIN_ABI_VERSION stays 4.                        */
+#define KIN_POP_MAX 64
+
+typedef struct KinPopMember {
+    const KinSamplerParams *sampler;   /* the member's device sampler (kin_params_device_sampler): its curriculum stage */
+    float *state;                      /* SoA env state of the member's env handle */
+    int stride;
+    int boot_cap;
+    uint64_t noise_seed;               /* kin_ppo_collect's noise_seed / first_step / reset_seed */
+    uint64_t reset_seed;
+    uint32_t first_step;
+    int pad0;
+    float *params;                     /* flat PARAM_ORDER parameters (read by every phase, written by kin_pop_adam) */
+    void *weight_image;                /* their bf16 operand image (kin_ppo_pack_weights; kept current by kin_pop_adam) */
+    void *obs_tiles;                   /* rollout buffers, as kin_ppo_collect / kin_ppo_gae take them */
+    float *action;
+    float *logp;
+    float *value;
+    float *reward;
+    uint8_t *done;
+    uint8_t *episode_start;
+    uint8_t *start_io;
+    float *last_value;
+    int *boot_count;
+    int *boot_index;
+    float *boot_obs;
+    float *advantage;
+    float *returns;
+    double *tile_sums;
+    const int *tile_ids;               /* this epoch's tile permutation: minibatch m = tile_ids[m * n .. (m + 1) * n) */
+    float *adv_stats;                  /* [minibatches per epoch][2], kin_ppo_adv_stats' output */
+    float *partials;                   /* kin_ppo_grad_tc scratch, [grid][P + 16] */
+    float *grad;
+    float *stats;
+    float *stats_accum;
+    float *adam_m;
+    float *adam_v;
+    KinPpoHyper hyper;                 /* gamma, gae_lambda, clip_range, ent_coef, vf_coef, max_grad_norm, Adam, normalize_advantage */
+} KinPopMember;
+
+/* The device copy of the handle's sampler (NULL until kin_params_set_sampler) and a byte comparison of two handles' env params. */
+int kin_params_device_sampler(void *handle, const void **sampler);
+int kin_params_same_env(void *handle_a, void *handle_b, int *same);
+
+/* Replaces: collect_rollouts (SB3 on_policy_algorithm.py), once per member: kin_ppo_collect(handle, member.state, member.stride, n_envs,
+ * mode, member.params, member.weight_image, 56, n_steps, member.noise_seed, member.first_step, member.reset_seed, member's buffers,
+ * tiles_per_cta = 1) for every member, with member.sampler in place of the handle's.  handle supplies the shared env params.        */
+int kin_pop_collect(void *handle, const KinPopMember *members, int n_members, int n_envs, int mode, int n_steps, void *stream);
+
+/* kin_ppo_bootstrap_list(member.params, 56, member's list, member.boot_cap, member.reward, member.hyper.gamma) for every member;
+ * max_boot_cap >= every member's boot_cap sizes the grid.                                                                        */
+int kin_pop_bootstrap_list(const KinPopMember *members, int n_members, int max_boot_cap, void *stream);
+
+/* Replaces: RolloutBuffer.compute_returns_and_advantage, once per member: kin_ppo_gae on the member's buffers (last_done = the done
+ * bytes of step n_steps - 1) with its gamma / gae_lambda, tile sums included.                                                      */
+int kin_pop_gae(const KinPopMember *members, int n_members, int n_envs, int n_steps, void *stream);
+
+/* kin_ppo_adv_stats(member.tile_sums, member.tile_ids, n_tiles_per_minibatch, n_minibatches, member.hyper.normalize_advantage,
+ * member.adv_stats) for every member.                                                                                             */
+int kin_pop_adv_stats(const KinPopMember *members, int n_members, int n_tiles_per_minibatch, int n_minibatches, void *stream);
+
+/* Replaces: one minibatch of SB3 ppo.py train() (loss and backward), once per member: kin_ppo_grad_tc(member.params, 56, &member.hyper,
+ * member.obs_tiles, .., member.tile_sums, member.tile_ids + minibatch * n_tiles_per_minibatch, n_tiles_per_minibatch, global_batch,
+ * member.partials, grid, member.grad, member.stats, NULL, NULL, 0, 1, member.adv_stats + 2 * minibatch, member.weight_image) --
+ * gradient kernel and reduction, min(grid, n_tiles_per_minibatch / 2) CTAs per net and member.                                      */
+int kin_pop_grad_tc(const KinPopMember *members, int n_members, int minibatch, int n_tiles_per_minibatch, long long global_batch, int grid,
+                    void *stream);
+
+/* Replaces: clip_grad_norm_ + optimizer.step, once per member: kin_ppo_adam(member.params, member.grad, member.adam_m, member.adam_v, P,
+ * &member.hyper, host_steps[k], member.stats, member.stats_accum, member.weight_image, 56).  host_hypers / host_steps are HOST arrays
+ * [n_members]: the bias corrections 1 - beta^step are computed on the host from host_hypers[k].adam_beta1 / adam_beta2, as
+ * kin_ppo_adam computes them, so host_hypers[k] must equal member k's descriptor hyper.                                            */
+int kin_pop_adam(const KinPopMember *members, int n_members, const KinPpoHyper *host_hypers, const int *host_steps, void *stream);
+
 /* ---- gradient exchange over NVLink peer memory (the training path's one collective; SURVEY 8e(ii)) ------------------------------
  * Replaces: the per-minibatch all-reduce (sum) of the flat gradient + 5 loss statistics between the gradient kernel and Adam.
  * Every rank (one per GPU of ONE node, world <= 8) owns a receive buffer; peers open it through CUDA IPC.  Per exchange:

@@ -19,7 +19,7 @@ import os
 # KIN_B200_LIB: load another build of the same C ABI (experiment / trace builds under tools/_bin); default = the in-tree library
 LIB_PATH = Path(os.environ["KIN_B200_LIB"]).resolve() if os.environ.get("KIN_B200_LIB") else PKG_DIR / "libkin_b200.so"
 
-_SCALARS = {"float": ctypes.c_float, "int": ctypes.c_int, "double": ctypes.c_double}
+_SCALARS = {"float": ctypes.c_float, "int": ctypes.c_int, "double": ctypes.c_double, "uint32_t": ctypes.c_uint32, "uint64_t": ctypes.c_uint64}
 _structs: dict[str, type] = {}
 _defines: dict[str, int] = {}
 
@@ -45,7 +45,7 @@ def c_struct(name: str) -> type:
         if mm is None:
             raise RuntimeError(f"cannot parse field {line!r} of {name}")
         _, ctype, ptr, fname, arr = mm.groups()
-        t: Any = ctypes.c_void_p if ptr else _SCALARS[ctype]
+        t: Any = ctypes.c_void_p if ptr else (_SCALARS[ctype] if ctype in _SCALARS else c_struct(ctype))      # (a nested Kin* struct)
         if arr:
             t = t * int(arr)
         fields.append((fname, t))
@@ -161,6 +161,14 @@ def lib() -> ctypes.CDLL:
     L.kin_ppo_bootstrap_list.argtypes = [vp, i32, vp, vp, vp, i32, vp, f32, vp]
     L.kin_route_obs_images.argtypes = [vp, i64, vp, vp]
     L.kin_route_collect.argtypes = [vp, vp, vp, vp, i32, i32, vp, i32, u64, u32, u64, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp]
+    L.kin_params_device_sampler.argtypes = [vp, ctypes.POINTER(vp)]
+    L.kin_params_same_env.argtypes = [vp, vp, ctypes.POINTER(i32)]
+    L.kin_pop_collect.argtypes = [vp, vp, i32, i32, i32, i32, vp]
+    L.kin_pop_bootstrap_list.argtypes = [vp, i32, i32, vp]
+    L.kin_pop_gae.argtypes = [vp, i32, i32, i32, vp]
+    L.kin_pop_adv_stats.argtypes = [vp, i32, i32, i32, vp]
+    L.kin_pop_grad_tc.argtypes = [vp, i32, i32, i32, i64, i32, vp]
+    L.kin_pop_adam.argtypes = [vp, i32, vp, vp, vp]
     L.kin_peer_buffer_bytes.argtypes = [i32, i32]
     L.kin_peer_buffer_create.argtypes = [i32, i32, ctypes.POINTER(vp), ctypes.c_char_p]
     L.kin_peer_buffer_open.argtypes = [ctypes.c_char_p, ctypes.POINTER(vp)]

@@ -108,6 +108,21 @@ extern "C" int kin_params_set_sampler(void* handle, const KinSamplerParams* host
     return KIN_OK;
 }
 
+extern "C" int kin_params_device_sampler(void* handle, const void** sampler) {
+    KinHandle* h = kin_handle(handle);
+    if (!h || !sampler) return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_device_sampler: bad argument");
+    *sampler = h->d_sampler;
+    return KIN_OK;
+}
+
+extern "C" int kin_params_same_env(void* handle_a, void* handle_b, int* same) {
+    KinHandle* a = kin_handle(handle_a);
+    KinHandle* b = kin_handle(handle_b);
+    if (!a || !b || !same) return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_same_env: bad argument");
+    *same = std::memcmp(&a->params, &b->params, sizeof(KinEnvParams)) == 0 ? 1 : 0;
+    return KIN_OK;
+}
+
 extern "C" int kin_params_destroy(void* handle) {
     KinHandle* h = kin_handle(handle);
     if (!h) return kin_fail(KIN_ERR_INVALID_ARG, "kin_params_destroy: bad handle");

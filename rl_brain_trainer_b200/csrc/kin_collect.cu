@@ -44,11 +44,28 @@ struct CollectOut {
     int boot_cap;
 };
 
-template <int TILES, int MODE>
+// POP (population launch, kin_pop_collect): SP carries the KinPopMember table and member blockIdx.y's descriptor replaces every other
+// per-run argument; P is shared.  A CTA holds one tile of one member (TILES = 1), blockIdx.x is the member-local tile, so env indices --
+// and with them the Philox streams -- are the standalone launch's.
+template <int TILES, int MODE, bool POP = false>
 __global__ void __launch_bounds__(TILES * AC_ROWS, 1)
 kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParams* __restrict__ SP, float* __restrict__ state, int stride, int n,
                    const float* __restrict__ params, const unsigned char* __restrict__ wimg, int T, uint64_t noise_seed, uint32_t step0,
                    uint64_t reset_seed, CollectOut out) {
+    static_assert(!POP || TILES == 1, "a CTA never mixes members");
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(SP)[blockIdx.y];
+        SP = M.sampler;
+        state = M.state;
+        stride = M.stride;
+        params = M.params;
+        wimg = static_cast<const unsigned char*>(M.weight_image);
+        noise_seed = M.noise_seed;
+        step0 = M.first_step;
+        reset_seed = M.reset_seed;
+        out = CollectOut{static_cast<unsigned char*>(M.obs_tiles), M.action, M.logp, M.value, M.reward, M.done, M.episode_start, M.start_io,
+                         M.last_value, M.boot_count, M.boot_index, M.boot_obs, M.boot_cap};
+    }
     constexpr int IN = 56;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // round up to 1024 bytes WITHOUT leaving the shared address space (pointer + offset, not an integer round trip), so every
@@ -142,10 +159,21 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
 }
 
 // r[idx] += gamma * V(terminal_obs) for the truncated episodes the collection kernel listed (strict fp32 critic)
-template <int IN>
+// POP: params carries the KinPopMember table, member blockIdx.y's list, critic, rewards and gamma replace the arguments
+template <int IN, bool POP = false>
 __global__ void __launch_bounds__(128)
 kin_bootstrap_list_kernel(const float* __restrict__ params, const float* __restrict__ boot_obs, const int* __restrict__ boot_index,
                           const int* __restrict__ boot_count, int cap, float* __restrict__ reward, float gamma) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(params)[blockIdx.y];
+        params = M.params;
+        boot_obs = M.boot_obs;
+        boot_index = M.boot_index;
+        boot_count = M.boot_count;
+        cap = M.boot_cap;
+        reward = M.reward;
+        gamma = M.hyper.gamma;
+    }
     const PpoOffsets O = ppo_offsets(IN);
     const int count = min(*boot_count, cap);
     const int i = blockIdx.x * 128 + threadIdx.x;
@@ -184,6 +212,10 @@ static cudaError_t launch_collect(const KinHandle* h, float* state, int stride, 
     auto kernel = mode == KIN_MODE_APPROACH ? kin_collect_kernel<TILES, KIN_MODE_APPROACH> : kin_collect_kernel<TILES, KIN_MODE_DOCK>;
     return launch_tiles<TILES>(kernel, sizeof(CollectSmem<TILES>) + 1024, n, st, h->params, h->d_sampler, state, stride, n, params, wimg, T, noise_seed,
                                step0, reset_seed, out);
+}
+
+__global__ void kin_pop_zero_counts_kernel(const KinPopMember* __restrict__ members, int n_members) {
+    if ((int)threadIdx.x < n_members) *members[threadIdx.x].boot_count = 0;
 }
 
 }  // namespace kin
@@ -225,4 +257,33 @@ extern "C" int kin_ppo_bootstrap_list(const float* params, int in_dim, const flo
     else kin_bootstrap_list_kernel<80><<<(boot_cap + 127) / 128, 128, 0, (cudaStream_t)stream>>>(params, boot_obs, boot_index, boot_count, boot_cap, reward, gamma);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_ppo_bootstrap_list");
+}
+
+extern "C" int kin_pop_collect(void* handle, const KinPopMember* members, int n_members, int n_envs, int mode, int n_steps, void* stream) {
+    KinHandle* h = kin_handle(handle);
+    if (!h) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_collect: bad handle");
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || n_steps <= 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_collect: need a device member table, 1 <= n_members <= KIN_POP_MAX and n_steps > 0");
+    if (n_envs <= 0 || (n_envs % AC_ROWS) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_collect: n_envs must be a positive multiple of 128 (one GEMM tile)");
+    if (mode != KIN_MODE_APPROACH && mode != KIN_MODE_DOCK) return kin_fail(KIN_ERR_UNSUPPORTED, "kin_pop_collect: mode must be approach (0) or dock (1)");
+    cudaStream_t st = (cudaStream_t)stream;
+    kin_pop_zero_counts_kernel<<<1, KIN_POP_MAX, 0, st>>>(members, n_members);      // kin_ppo_collect's reset of *boot_count
+    auto kernel = mode == KIN_MODE_APPROACH ? kin_collect_kernel<1, KIN_MODE_APPROACH, true> : kin_collect_kernel<1, KIN_MODE_DOCK, true>;
+    const size_t smem = sizeof(CollectSmem<1>) + 1024;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_collect: smem attribute");
+    kernel<<<dim3((unsigned)(n_envs / AC_ROWS), (unsigned)n_members), AC_ROWS, smem, st>>>(h->params, reinterpret_cast<const KinSamplerParams*>(members), nullptr, 0,
+                                                                                          n_envs, nullptr, nullptr, n_steps, 0, 0u, 0, CollectOut{});
+    e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_collect");
+}
+
+extern "C" int kin_pop_bootstrap_list(const KinPopMember* members, int n_members, int max_boot_cap, void* stream) {
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || max_boot_cap <= 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_bootstrap_list: need a device member table, 1 <= n_members <= KIN_POP_MAX and max_boot_cap > 0");
+    // blocks past a member's own count return at once (block-uniform), so one grid sized for the largest list serves every member
+    kin_bootstrap_list_kernel<56, true><<<dim3((unsigned)((max_boot_cap + 127) / 128), (unsigned)n_members), 128, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(members), nullptr, nullptr, nullptr, 0, nullptr, 0.0f);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_bootstrap_list");
 }

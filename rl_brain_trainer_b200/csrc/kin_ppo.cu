@@ -108,11 +108,27 @@ kin_ppo_bootstrap_kernel(ActW vf, const float* __restrict__ terminal_obs, const 
     if (trunc) reward[i] = fmaf(gamma, v[0], reward[i]);
 }
 
+// POP (the kin_pop_* population launches, kin_b200.h): the kernels below take their per-run pointers and hyper-parameters from member
+// blockIdx.y's KinPopMember descriptor, whose table arrives in the first pointer argument; the body is the standalone kernel's.
+
 // buffers.py compute_returns_and_advantage: one thread per env, backwards over T; [T][n] arrays are coalesced over envs
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_ppo_gae_kernel(const float* __restrict__ reward, const float* __restrict__ value, const uint8_t* __restrict__ episode_start,
                    const float* __restrict__ last_value, const uint8_t* __restrict__ last_done, float gamma, float lam, int T, int n,
                    float* __restrict__ adv, float* __restrict__ ret) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(reward)[blockIdx.y];
+        reward = M.reward;
+        value = M.value;
+        episode_start = M.episode_start;
+        last_value = M.last_value;
+        last_done = M.done + (size_t)(T - 1) * n;
+        gamma = M.hyper.gamma;
+        lam = M.hyper.gae_lambda;
+        adv = M.advantage;
+        ret = M.returns;
+    }
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     float next_value = last_value[e];
@@ -131,8 +147,14 @@ kin_ppo_gae_kernel(const float* __restrict__ reward, const float* __restrict__ v
 }
 
 // (sum adv, sum adv^2) per 64-sample tile, in double
+template <bool POP = false>
 __global__ void __launch_bounds__(64)
 kin_ppo_tile_sums_kernel(const float* __restrict__ adv, double* __restrict__ tile_sums) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(adv)[blockIdx.y];
+        adv = M.advantage;
+        tile_sums = M.tile_sums;
+    }
     const int tile = blockIdx.x;
     const double a = (double)adv[(size_t)tile * TS + threadIdx.x];
     double s1 = a, s2 = a * a;
@@ -531,8 +553,15 @@ kin_ppo_grad_kernel(const float* __restrict__ params, KinPpoHyper hp, const floa
 
 // grad[p] = sum over CTAs of partials[c][p]; stats likewise.  A block owns 32 consecutive parameters (one 128-byte line per
 // partial row); its 8 warps take rows w, w + 8, ... with independent loads in flight, then fold in a fixed order (deterministic).
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_ppo_reduce_kernel(const float* __restrict__ partials, int n_cta, int P, float* __restrict__ grad, float* __restrict__ stats, float inv_global_batch) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(partials)[blockIdx.y];
+        partials = M.partials;
+        grad = M.grad;
+        stats = M.stats;
+    }
     __shared__ float part[8][32];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int p = blockIdx.x * 32 + lane;
@@ -559,8 +588,16 @@ kin_ppo_reduce_kernel(const float* __restrict__ partials, int n_cta, int P, floa
 
 // (mean, 1 / (std + 1e-8)) of the advantages of each minibatch (torch: mean, unbiased std) from the per-tile fp64 sums;
 // one CTA per minibatch, minibatch m = tile_ids[m * n_tiles .. (m + 1) * n_tiles)
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_ppo_adv_stats_kernel(const double* __restrict__ tile_sums, const int* __restrict__ tile_ids, int n_tiles, int normalize, float* __restrict__ out) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(tile_sums)[blockIdx.y];
+        tile_sums = M.tile_sums;
+        tile_ids = M.tile_ids;
+        normalize = M.hyper.normalize_advantage;
+        out = M.adv_stats;
+    }
     __shared__ double sh[2][8];
     const int* ids = tile_ids + (size_t)blockIdx.x * n_tiles;
     double s1 = 0.0, s2 = 0.0;
@@ -589,10 +626,32 @@ kin_ppo_adv_stats_kernel(const double* __restrict__ tile_sums, const int* __rest
 
 // clip_grad_norm_ + Adam.  Every CTA computes the global gradient norm itself (64 KB of L2-resident data, identical summation
 // order -> bitwise-identical clip coefficient in every CTA), then updates its own 1024 parameters.
+// POP: grad carries the table; bc1 / bc2 come from the one extra (by-value) argument, computed on the host from each member's betas
+// and step as kin_ppo_adam computes them.  The standalone instance has no extra argument: its parameter list is unchanged.
+struct PopBiasCorrection {
+    float bc[KIN_POP_MAX][2];
+};
+
+template <bool POP = false, class... PopArgs>
 __global__ void __launch_bounds__(1024)
 kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, float* __restrict__ m, float* __restrict__ v, int P,
                     KinPpoHyper hp, float bc1, float bc2, float* __restrict__ stats, float* __restrict__ stats_accum,
-                    unsigned short* __restrict__ wimg, int in_dim) {
+                    unsigned short* __restrict__ wimg, int in_dim, const __grid_constant__ PopArgs... pop) {
+    static_assert(sizeof...(PopArgs) == (POP ? 1 : 0), "the population instance takes its bias corrections as one extra argument");
+    if constexpr (POP) {
+        const PopBiasCorrection& B = (pop, ...);
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(grad)[blockIdx.y];
+        params = M.params;
+        grad = M.grad;
+        m = M.adam_m;
+        v = M.adam_v;
+        hp = M.hyper;
+        bc1 = B.bc[blockIdx.y][0];
+        bc2 = B.bc[blockIdx.y][1];
+        stats = M.stats;
+        stats_accum = M.stats_accum;
+        wimg = static_cast<unsigned short*>(M.weight_image);
+    }
     __shared__ float red[32];
     __shared__ float coef;
     if (stats && stats[KIN_PPO_STAT_SKIP] != 0.0f) return;      // the gradient exchange timed out (kin_peer.cu): leave the parameters alone
@@ -708,6 +767,12 @@ kin_route_obs_images_kernel(const float* __restrict__ obs, long long n_rows, uns
 
 int kin_ppo_reduce_launch(const float* partials, int n_cta, int P, float* grad, float* stats, float inv_global_batch, cudaStream_t st) {
     kin_ppo_reduce_kernel<<<(P + 5 + 31) / 32, 256, 0, st>>>(partials, n_cta, P, grad, stats, inv_global_batch);
+    return KIN_OK;
+}
+
+int kin_pop_reduce_launch(const KinPopMember* members, int n_members, int n_cta, int P, float inv_global_batch, cudaStream_t st) {
+    kin_ppo_reduce_kernel<true><<<dim3((unsigned)((P + 5 + 31) / 32), (unsigned)n_members), 256, 0, st>>>(reinterpret_cast<const float*>(members), n_cta, P,
+                                                                                                          nullptr, nullptr, inv_global_batch);
     return KIN_OK;
 }
 
@@ -916,4 +981,41 @@ extern "C" int kin_ppo_adam(float* params, const float* grad, float* adam_m, flo
                                                               static_cast<unsigned short*>(weight_image), in_dim);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_ppo_adam");
+}
+
+static bool pop_args_ok(const KinPopMember* members, int n_members) { return members && n_members > 0 && n_members <= KIN_POP_MAX; }
+
+extern "C" int kin_pop_gae(const KinPopMember* members, int n_members, int n_envs, int n_steps, void* stream) {
+    if (!pop_args_ok(members, n_members) || n_envs <= 0 || n_steps <= 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_gae: bad arguments");
+    if ((((size_t)n_steps * n_envs) % TS) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_gae: n_steps * n_envs must be a multiple of 64 for tile sums");
+    cudaStream_t st = (cudaStream_t)stream;
+    kin_ppo_gae_kernel<true><<<dim3((unsigned)((n_envs + 255) / 256), (unsigned)n_members), 256, 0, st>>>(
+        reinterpret_cast<const float*>(members), nullptr, nullptr, nullptr, nullptr, 0.0f, 0.0f, n_steps, n_envs, nullptr, nullptr);
+    kin_ppo_tile_sums_kernel<true><<<dim3((unsigned)(((size_t)n_steps * n_envs) / TS), (unsigned)n_members), TS, 0, st>>>(
+        reinterpret_cast<const float*>(members), nullptr);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_gae");
+}
+
+extern "C" int kin_pop_adv_stats(const KinPopMember* members, int n_members, int n_tiles_per_minibatch, int n_minibatches, void* stream) {
+    if (!pop_args_ok(members, n_members) || n_tiles_per_minibatch <= 0 || n_minibatches <= 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_adv_stats: bad arguments");
+    kin_ppo_adv_stats_kernel<true><<<dim3((unsigned)n_minibatches, (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const double*>(members), nullptr, n_tiles_per_minibatch, 0, nullptr);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_adv_stats");
+}
+
+extern "C" int kin_pop_adam(const KinPopMember* members, int n_members, const KinPpoHyper* host_hypers, const int* host_steps, void* stream) {
+    if (!pop_args_ok(members, n_members) || !host_hypers || !host_steps) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_adam: bad arguments");
+    PopBiasCorrection B{};
+    for (int k = 0; k < n_members; ++k) {
+        if (host_steps[k] < 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_adam: steps count optimiser steps from 1");
+        B.bc[k][0] = 1.0f - powf(host_hypers[k].adam_beta1, (float)host_steps[k]);
+        B.bc[k][1] = 1.0f - powf(host_hypers[k].adam_beta2, (float)host_steps[k]);
+    }
+    const int P = ppo_offsets(56).total;
+    kin_ppo_adam_kernel<true><<<dim3((unsigned)((P + 1023) / 1024), (unsigned)n_members), 1024, 0, (cudaStream_t)stream>>>(
+        nullptr, reinterpret_cast<const float*>(members), nullptr, nullptr, P, KinPpoHyper{}, 0.0f, 0.0f, nullptr, nullptr, nullptr, 56, B);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_adam");
 }

@@ -71,6 +71,8 @@ __host__ __device__ inline int wimg_offset(const PpoOffsets& o, int in_dim, int 
 
 // grad[p] = sum over CTAs of partials[c][p] (rows of P + KIN_PPO_STATS + 8 floats); stats (nullable) likewise, scaled
 int kin_ppo_reduce_launch(const float* partials, int n_cta, int P, float* grad, float* stats, float inv_global_batch, cudaStream_t st);
+// the same reduction for every member of a population (partials / grad / stats from member blockIdx.y's descriptor)
+int kin_pop_reduce_launch(const KinPopMember* members, int n_members, int n_cta, int P, float inv_global_batch, cudaStream_t st);
 
 
 // kin_ppo_tc3.cu: the three-streams-per-SM form of the tensor-core gradient kernel.  Returns 0 when the call is not eligible (the caller

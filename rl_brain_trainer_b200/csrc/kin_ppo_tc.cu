@@ -146,14 +146,35 @@ __device__ __forceinline__ void epilogue_store(unsigned char* tile, int row, int
 // PEER: the kernel ends with the in-kernel gradient exchange over NVLink peer memory (kin_peer.cuh::peer_exchange_tail): grid barrier,
 // per-CTA column slices reduced over the partial rows and pushed to every rank, rank-ordered sum into px.grad -- no separate push /
 // gather launches between this kernel and Adam.
-template <bool IMG, int IN, bool PEER = false>
+// POP (population launch, kin_pop_grad_tc): params carries the KinPopMember table and the one extra argument is the minibatch index;
+// member blockIdx.z's descriptor supplies every per-run pointer and hyper-parameter, its tile ids and advantage statistics are those of
+// that minibatch.  blockIdx.y stays the net and blockIdx.x the member's CTA, so the tile loop, the partial rows and their reduction
+// order are the standalone launch's.  The standalone instances have no extra argument: their parameter lists are unchanged.
+template <bool IMG, int IN, bool PEER = false, bool POP = false, class... PopArgs>
 __global__ void __launch_bounds__(TCG_THREADS, 2)
 kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const float* __restrict__ obs, const float* __restrict__ action,
                        const float* __restrict__ old_logp, const float* __restrict__ advantage, const float* __restrict__ returns,
                        const double* __restrict__ tile_sums, const int* __restrict__ tile_ids, int n_pairs, float inv_global_batch,
                        float* __restrict__ partials, float* __restrict__ logp_out, float* __restrict__ value_out, int forward_only, int net_base,
-                       const float* __restrict__ adv_stats, const unsigned char* __restrict__ wimg, const PeerFused px) {
+                       const float* __restrict__ adv_stats, const unsigned char* __restrict__ wimg, const PeerFused px, PopArgs... pop) {
     static_assert(IN == 56 || (IN == 80 && IMG), "56-input policies (fp32 observations or images) or the 80-input route policy (folded images)");
+    static_assert(sizeof...(PopArgs) == (POP ? 1 : 0) && (!POP || (IMG && IN == 56 && !PEER)), "population: 56-input images, one extra argument");
+    if constexpr (POP) {
+        const int minibatch = (pop, ...);
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(params)[blockIdx.z];
+        params = M.params;
+        hp = M.hyper;
+        obs = static_cast<const float*>(M.obs_tiles);
+        action = M.action;
+        old_logp = M.logp;
+        advantage = M.advantage;
+        returns = M.returns;
+        tile_sums = M.tile_sums;
+        tile_ids = M.tile_ids + (size_t)minibatch * 2 * n_pairs;
+        partials = M.partials;
+        adv_stats = M.adv_stats + 2 * minibatch;
+        wimg = static_cast<const unsigned char*>(M.weight_image);
+    }
     constexpr int KT = 1;                            // K tiles of layer 1
     constexpr int K1 = 64;                           // padded reduction width of layer 1 (live inputs | 1 | zeros)
     constexpr bool FOLD = IN == 80;                  // route policy: layer 1 sees its 60 live columns, the constants are folded into the bias
@@ -791,3 +812,30 @@ extern "C" int kin_ppo_grad_tc_update(const float* params, int in_dim, const Kin
                           stats, nullptr, nullptr, 0, obs_is_image, adv_stats, weight_image, px, stream);
 }
 
+
+extern "C" int kin_pop_grad_tc(const KinPopMember* members, int n_members, int minibatch, int n_tiles_per_minibatch, long long global_batch, int grid,
+                               void* stream) {
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || minibatch < 0 || n_tiles_per_minibatch <= 0 || global_batch <= 0 || grid <= 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_grad_tc: bad arguments");
+    if (n_tiles_per_minibatch & 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_grad_tc: n_tiles must be even (two 64-sample tiles per 128-row GEMM tile)");
+    auto kernel = kin_ppo_grad_tc_kernel<true, 56, false, true, int>;
+    const size_t smem = sizeof(TcGradSmem<1>) + 1024;
+    static bool attr_set[KIN_MAX_DEVICES] = {};
+    const int dev_slot = kin_device_slot();
+    if (!attr_set[dev_slot]) {
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_grad_tc: smem attribute");
+        attr_set[dev_slot] = true;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n_pairs = n_tiles_per_minibatch / 2;
+    const int g = grid < n_pairs ? grid : n_pairs;      // kin_ppo_grad_tc's clamp: the same CTAs, tiles per CTA and partial rows per member
+    const float inv = 1.0f / (float)global_batch;
+    const PeerFused none{};
+    kernel<<<dim3((unsigned)g, 2u, (unsigned)n_members), TCG_THREADS, smem, st>>>(reinterpret_cast<const float*>(members), KinPpoHyper{}, nullptr, nullptr,
+                                                                                 nullptr, nullptr, nullptr, nullptr, nullptr, n_pairs, inv, nullptr, nullptr,
+                                                                                 nullptr, 0, 0, nullptr, nullptr, none, minibatch);
+    kin_pop_reduce_launch(members, n_members, g, ppo_offsets(56).total, inv, st);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_grad_tc");
+}

@@ -436,6 +436,11 @@ class PPOTrainer:
             _lib.check(L.kin_ppo_gae(self.rew_buf.data_ptr(), self.val_buf.data_ptr(), self.start_buf.data_ptr(), self.last_val.data_ptr(),
                                      self.done_buf[self.T - 1].data_ptr(), float(hp.gamma), float(hp.gae_lambda), self.T, self.N,
                                      self.adv_buf.data_ptr(), self.ret_buf.data_ptr(), self.tile_sums.data_ptr(), stream))
+        return self._finish_fused_collect()
+
+    def _finish_fused_collect(self) -> dict[str, float]:
+        """Host bookkeeping after a fused arm collection (this trainer's own launches or a ``PPOPopulation``'s): step counters,
+        bootstrap-list overflow check, the rollout's episode outcomes and ``last_rollout``."""
         self.global_step += self.T
         self.num_timesteps += self.S * self.world
         if int(self.boot_count.item()) > self.boot_cap:       # the kernel drops entries past the capacity: returns would be biased
