@@ -827,6 +827,7 @@ int kin_ppo_bootstrap_list(const float *params, int in_dim, const float *boot_ob
                            float *reward, float gamma, void *stream);
 
 /* clip_grad_norm_(max_grad_norm) + Adam step on the flat parameter buffer (torch.optim.Adam semantics, eps = 1e-5 in SB3).
+ * max_grad_norm <= 0 skips the clip (torch's clip_grad_norm_(0) would zero the gradient instead).
  * adam_m / adam_v [P]; step = 1-based update count.  stats[5] receives the gradient norm; stats_accum (nullable, [8]) gets
  * stats[0..5] added and slot 7 incremented: running sums over the minibatches of one update without host round trips.
  * weight_image (nullable, in_dim 56): the bf16 operand image is rewritten in step with the parameters.                   */
