@@ -14,6 +14,7 @@
 #pragma once
 
 #include "kin_ppo_layout.cuh"
+#include "kin_ppo_math.cuh"
 #include "kin_state.cuh"
 #include "kin_umma.cuh"
 
@@ -251,7 +252,7 @@ __device__ __forceinline__ float sample_action(const AcWeights<KT>& W, uint64_t 
 #pragma unroll
     for (int k = 0; k < NJ; ++k) {
         a[k] = fmaf(W.sig[k], eps[k], mean[k]);
-        lp += -0.5f * eps[k] * eps[k] - W.ls[k] - kHalfLog2Pi;
+        lp += gauss_logp_term(eps[k], W.ls[k]);
         action_out[k] = a[k];
     }
     return lp;

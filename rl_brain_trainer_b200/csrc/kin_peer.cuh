@@ -17,6 +17,7 @@
 
 #include "kin_internal.h"
 #include "kin_ppo_layout.cuh"
+#include "kin_ppo_math.cuh"
 
 namespace kin {
 
@@ -273,8 +274,7 @@ __device__ __forceinline__ void peer_adam_tail(const PeerFused& px, const KinPpo
         for (int off = 16; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
         if (lane == 0) {
             const float norm = sqrtf(t);
-            const float c = hp.max_grad_norm > 0.0f ? hp.max_grad_norm / (norm + 1e-6f) : 1.0f;
-            red[32] = c < 1.0f ? c : 1.0f;
+            red[32] = clip_coef(norm, hp);
             red[33] = norm;
         }
     }
@@ -294,14 +294,11 @@ __device__ __forceinline__ void peer_adam_tail(const PeerFused& px, const KinPpo
     const float cf = red[32];
     const PpoOffsets O = ppo_offsets(A.in_dim);
     for (int p = p0 + tid; p < p1; p += (int)blockDim.x) {
-        const float g = px.grad[p] * cf;
         const bool first = p == own_p;
-        const float mm = fmaf(hp.adam_beta1, first ? own_m : A.m[p], (1.0f - hp.adam_beta1) * g);
-        const float vv = fmaf(hp.adam_beta2, first ? own_v : A.v[p], (1.0f - hp.adam_beta2) * g * g);
-        A.m[p] = mm;
-        A.v[p] = vv;
-        const float denom = sqrtf(vv) / sqrtf(A.bc2) + hp.adam_eps;
-        const float np = (first ? own_w : A.params[p]) - (hp.learning_rate / A.bc1) * (mm / denom);
+        const AdamMoments mv = adam_moments(px.grad[p], cf, first ? own_m : A.m[p], first ? own_v : A.v[p], hp);
+        A.m[p] = mv.m;
+        A.v[p] = mv.v;
+        const float np = adam_param(first ? own_w : A.params[p], mv, A.bc1, A.bc2, hp);
         A.params[p] = np;
         if (A.wimg) {
             const int off = wimg_offset(O, A.in_dim, p);

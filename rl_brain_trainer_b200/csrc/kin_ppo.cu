@@ -21,6 +21,7 @@
 #include "kin_internal.h"
 #include "kin_mlp.cuh"
 #include "kin_ppo_layout.cuh"
+#include "kin_ppo_math.cuh"
 #include "kin_state.cuh"
 
 namespace kin {
@@ -68,7 +69,7 @@ kin_policy_act_kernel(ActW pi, ActW vf, const float* __restrict__ log_std, const
             const float ls = __ldg(log_std + k);
             const float e = deterministic ? 0.0f : eps[k];
             action[(size_t)i * ACT + k] = fmaf(expf(ls), e, mean[k]);
-            lp += -0.5f * e * e - ls - kHalfLog2Pi;   // log N(a; mean, sigma) with (a - mean) / sigma == eps
+            lp += gauss_logp_term(e, ls);   // (a - mean) / sigma == eps
         }
         logp[i] = lp;
     }
@@ -189,8 +190,10 @@ struct GradSmem {
     static constexpr int H2 = H1 + TS * HS;
     static constexpr int G = H2 + TS * HS;
     static constexpr int OUT8 = G + TS * HS;          // [TS][8]
-    static constexpr int SCAL = OUT8 + TS * 8;        // adv mean, 1/(std+eps), stats accumulators [16]
+    static constexpr int SCAL = OUT8 + TS * 8;        // [0] adv mean, [1] 1/(std+eps), then RED
+    static constexpr int RED = SCAL + 8;              // [2][12] per loss warp: the 5 statistics, the 7 d log_std, summed over its tiles
     static constexpr int FLOATS = SCAL + 32;
+    static_assert(RED + 2 * 12 <= FLOATS, "the loss warps' rows fit the scalar block");
 };
 
 template <int IN>
@@ -236,24 +239,8 @@ kin_ppo_grad_kernel(const float* __restrict__ params, KinPpoHyper hp, const floa
     if (adv_stats) {
         if (tid == 0) { sm[L::SCAL + 0] = adv_stats[0]; sm[L::SCAL + 1] = adv_stats[1]; }
     } else if (tid < 32) {
-        double s1 = 0.0, s2 = 0.0;
-        for (int j = tid; j < n_tiles; j += 32) {
-            const int t = tile_ids[j];
-            s1 += tile_sums[2 * t];
-            s2 += tile_sums[2 * t + 1];
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-            s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-        }
-        if (tid == 0) {
-            const double nsamp = (double)n_tiles * TS;
-            const double mean = s1 / nsamp;
-            const double var = nsamp > 1.0 ? fmax((s2 - nsamp * mean * mean) / (nsamp - 1.0), 0.0) : 0.0;
-            sm[L::SCAL + 0] = hp.normalize_advantage ? (float)mean : 0.0f;
-            sm[L::SCAL + 1] = hp.normalize_advantage ? (float)(1.0 / (sqrt(var) + 1e-8)) : 1.0f;
-        }
+        const double2 s = warp_tile_sums(tile_sums, tile_ids, n_tiles, tid, 32);
+        if (tid == 0) adv_normaliser(s.x, s.y, (double)n_tiles * TS, hp.normalize_advantage, &sm[L::SCAL]);
     }
     __syncthreads();
 
@@ -366,23 +353,25 @@ kin_ppo_grad_kernel(const float* __restrict__ params, KinPpoHyper hp, const floa
                 const float ls = sm[L::LS + d];
                 inv_sig[d] = expf(-ls);
                 z[d] = (__ldg(action + g * 7 + d) - sm[L::OUT8 + s * 8 + d]) * inv_sig[d];
-                lp += -0.5f * z[d] * z[d] - ls - kHalfLog2Pi;
-                ent += 0.5f + kHalfLog2Pi + ls;
+                lp += gauss_logp_term(z[d], ls);
+                ent += gauss_entropy_term(ls);
             }
-            const float adv_n = (__ldg(advantage + g) - sm[L::SCAL + 0]) * sm[L::SCAL + 1];
-            const float log_ratio = lp - __ldg(old_logp + g);
-            const float ratio = expf(log_ratio);
-            const float pl1 = adv_n * ratio, pl2 = adv_n * fminf(fmaxf(ratio, 1.0f - hp.clip_range), 1.0f + hp.clip_range);
-            const float dpl_dlp = (pl1 <= pl2) ? -adv_n * ratio : 0.0f;          // d(-min(pl1, pl2)) / d logp
+            const Surrogate sur = clipped_surrogate(__ldg(advantage + g), sm[L::SCAL + 0], sm[L::SCAL + 1], lp, __ldg(old_logp + g), hp);
+            const float dpl_dlp = sur.dpl_dlp();
             const float v = sm[L::OUT8 + s * 8 + 7], rt = __ldg(returns + g);
 #pragma unroll
             for (int d = 0; d < 7; ++d) {
-                sm[L::OUT8 + s * 8 + d] = inv_global_batch * dpl_dlp * z[d] * inv_sig[d];   // dL/dmean_d
-                z[d] = inv_global_batch * dpl_dlp * (z[d] * z[d] - 1.0f) - inv_global_batch * hp.ent_coef;   // dL/dlog_std_d (per sample)
+                sm[L::OUT8 + s * 8 + d] = dloss_dmean(inv_global_batch, dpl_dlp, z[d], inv_sig[d]);
+                z[d] = dloss_dlog_std(inv_global_batch, dpl_dlp, z[d], hp);
             }
-            sm[L::OUT8 + s * 8 + 7] = inv_global_batch * hp.vf_coef * 2.0f * (v - rt);      // dL/dvalue
+            sm[L::OUT8 + s * 8 + 7] = dloss_dvalue(inv_global_batch, v, rt, hp);
             // statistics: sums over samples (divided by the global batch at the end)
-            float st[5] = {-fminf(pl1, pl2), (rt - v) * (rt - v), ent, (ratio - 1.0f) - log_ratio, fabsf(ratio - 1.0f) > hp.clip_range ? 1.0f : 0.0f};
+            float st[5];
+            st[KIN_PPO_STAT_POLICY_LOSS] = sur.loss();
+            st[KIN_PPO_STAT_VALUE_LOSS] = value_loss(v, rt);
+            st[KIN_PPO_STAT_ENTROPY] = ent;
+            st[KIN_PPO_STAT_APPROX_KL] = sur.approx_kl();
+            st[KIN_PPO_STAT_CLIP_FRACTION] = sur.clipped(hp);
 #pragma unroll
             for (int q = 0; q < 5; ++q) {
 #pragma unroll
@@ -393,11 +382,12 @@ kin_ppo_grad_kernel(const float* __restrict__ params, KinPpoHyper hp, const floa
 #pragma unroll
                 for (int off = 16; off > 0; off >>= 1) z[d] += __shfl_xor_sync(0xffffffffu, z[d], off);
             }
-            if ((tid & 31) == 0) {
+            if ((tid & 31) == 0) {      // each loss warp into its own row: the sums are taken in a fixed order
+                float* r = &sm[L::RED + (tid >> 5) * 12];
 #pragma unroll
-                for (int q = 0; q < 5; ++q) atomicAdd(&sm[L::SCAL + 2 + q], st[q]);
+                for (int q = 0; q < 5; ++q) r[q] += st[q];
 #pragma unroll
-                for (int d = 0; d < 7; ++d) atomicAdd(&sm[L::SCAL + 8 + d], z[d]);
+                for (int d = 0; d < 7; ++d) r[5 + d] += z[d];
             }
         }
         __syncthreads();
@@ -546,8 +536,8 @@ kin_ppo_grad_kernel(const float* __restrict__ params, KinPpoHyper hp, const floa
         if (tid == 7) out[O.val_b] = acc_bo;
         if (tid >= 128) { const int u = tid - 128; out[(u < 64 ? O.pi_b1 + u : O.vf_b1 + u - 64)] = acc_b1; }
         if (tid < 128) out[(tid < 64 ? O.pi_b0 + tid : O.vf_b0 + tid - 64)] = acc_b0;
-        if (tid < 7) out[O.log_std + tid] = sm[L::SCAL + 8 + tid];
-        if (tid < 5) out[P + tid] = sm[L::SCAL + 2 + tid];
+        if (tid < 7) out[O.log_std + tid] = sm[L::RED + 5 + tid] + sm[L::RED + 12 + 5 + tid];      // loss warp 0 + loss warp 1
+        if (tid < 5) out[P + tid] = sm[L::RED + tid] + sm[L::RED + 12 + tid];
     }
 }
 
@@ -586,8 +576,7 @@ kin_ppo_reduce_kernel(const float* __restrict__ partials, int n_cta, int P, floa
     }
 }
 
-// (mean, 1 / (std + 1e-8)) of the advantages of each minibatch (torch: mean, unbiased std) from the per-tile fp64 sums;
-// one CTA per minibatch, minibatch m = tile_ids[m * n_tiles .. (m + 1) * n_tiles)
+// adv_normaliser of each minibatch from the per-tile fp64 sums; one CTA per minibatch, minibatch m = tile_ids[m * n_tiles .. (m + 1) * n_tiles)
 template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_ppo_adv_stats_kernel(const double* __restrict__ tile_sums, const int* __restrict__ tile_ids, int n_tiles, int normalize, float* __restrict__ out) {
@@ -599,28 +588,13 @@ kin_ppo_adv_stats_kernel(const double* __restrict__ tile_sums, const int* __rest
         out = M.adv_stats;
     }
     __shared__ double sh[2][8];
-    const int* ids = tile_ids + (size_t)blockIdx.x * n_tiles;
-    double s1 = 0.0, s2 = 0.0;
-    for (int j = threadIdx.x; j < n_tiles; j += 256) {
-        const int t = ids[j];
-        s1 += tile_sums[2 * t];
-        s2 += tile_sums[2 * t + 1];
-    }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-        s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-    }
-    if ((threadIdx.x & 31) == 0) { sh[0][threadIdx.x >> 5] = s1; sh[1][threadIdx.x >> 5] = s2; }
+    const double2 s = warp_tile_sums(tile_sums, tile_ids + (size_t)blockIdx.x * n_tiles, n_tiles, threadIdx.x, 256);
+    if ((threadIdx.x & 31) == 0) { sh[0][threadIdx.x >> 5] = s.x; sh[1][threadIdx.x >> 5] = s.y; }
     __syncthreads();
     if (threadIdx.x == 0) {
-        s1 = 0.0; s2 = 0.0;
+        double s1 = 0.0, s2 = 0.0;
         for (int k = 0; k < 8; ++k) { s1 += sh[0][k]; s2 += sh[1][k]; }
-        const double nsamp = (double)n_tiles * TS;
-        const double mean = s1 / nsamp;
-        const double var = nsamp > 1.0 ? fmax((s2 - nsamp * mean * mean) / (nsamp - 1.0), 0.0) : 0.0;
-        out[2 * blockIdx.x] = normalize ? (float)mean : 0.0f;
-        out[2 * blockIdx.x + 1] = normalize ? (float)(1.0 / (sqrt(var) + 1e-8)) : 1.0f;
+        adv_normaliser(s1, s2, (double)n_tiles * TS, normalize, out + 2 * blockIdx.x);
     }
 }
 
@@ -682,8 +656,7 @@ kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, 
         for (int off = 16; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
         if (threadIdx.x == 0) {
             const float norm = sqrtf(t);
-            const float c = hp.max_grad_norm > 0.0f ? hp.max_grad_norm / (norm + 1e-6f) : 1.0f;
-            coef = c < 1.0f ? c : 1.0f;
+            coef = clip_coef(norm, hp);
             if (stats && blockIdx.x == 0) stats[KIN_PPO_STAT_GRAD_NORM] = norm;
             if (stats && stats_accum && blockIdx.x == 0) {          // running sums over the minibatches of an update (slot 7 counts them)
 #pragma unroll
@@ -696,14 +669,10 @@ kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, 
     __syncthreads();
     const float cf = coef;
     for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
-        const float g = __ldcg(grad + p) * cf;
-        const float m0 = has_own ? own_m : m[p], v0 = has_own ? own_v : v[p];
-        const float mm = fmaf(hp.adam_beta1, m0, (1.0f - hp.adam_beta1) * g);
-        const float vv = fmaf(hp.adam_beta2, v0, (1.0f - hp.adam_beta2) * g * g);
-        m[p] = mm;
-        v[p] = vv;
-        const float denom = sqrtf(vv) / sqrtf(bc2) + hp.adam_eps;
-        const float np = (has_own ? own_p : params[p]) - (hp.learning_rate / bc1) * (mm / denom);
+        const AdamMoments mv = adam_moments(__ldcg(grad + p), cf, has_own ? own_m : m[p], has_own ? own_v : v[p], hp);
+        m[p] = mv.m;
+        v[p] = mv.v;
+        const float np = adam_param(has_own ? own_p : params[p], mv, bc1, bc2, hp);
         params[p] = np;
         if (wimg) {      // keep the bf16 operand image of the weights in step with the parameters
             const int off = wimg_offset(ppo_offsets(in_dim), in_dim, p);
@@ -976,8 +945,8 @@ extern "C" int kin_ppo_adam(float* params, const float* grad, float* adam_m, flo
     if (weight_image && in_dim != 56)
         return kin_fail(KIN_ERR_UNSUPPORTED, "kin_ppo_adam: only the 56-input image is kept current in place; the folded route image is rebuilt with kin_ppo_pack_weights");
     if (!params || !grad || !adam_m || !adam_v || !hp || n_params <= 0 || step < 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_adam: bad arguments");
-    const float bc1 = 1.0f - powf(hp->adam_beta1, (float)step), bc2 = 1.0f - powf(hp->adam_beta2, (float)step);
-    kin_ppo_adam_kernel<<<(n_params + 1023) / 1024, 1024, 0, (cudaStream_t)stream>>>(params, grad, adam_m, adam_v, n_params, *hp, bc1, bc2, stats, stats_accum,
+    const float2 bc = adam_bias_corrections(*hp, step);
+    kin_ppo_adam_kernel<<<(n_params + 1023) / 1024, 1024, 0, (cudaStream_t)stream>>>(params, grad, adam_m, adam_v, n_params, *hp, bc.x, bc.y, stats, stats_accum,
                                                               static_cast<unsigned short*>(weight_image), in_dim);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_ppo_adam");
@@ -1010,8 +979,9 @@ extern "C" int kin_pop_adam(const KinPopMember* members, int n_members, const Ki
     PopBiasCorrection B{};
     for (int k = 0; k < n_members; ++k) {
         if (host_steps[k] < 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_adam: steps count optimiser steps from 1");
-        B.bc[k][0] = 1.0f - powf(host_hypers[k].adam_beta1, (float)host_steps[k]);
-        B.bc[k][1] = 1.0f - powf(host_hypers[k].adam_beta2, (float)host_steps[k]);
+        const float2 bc = adam_bias_corrections(host_hypers[k], host_steps[k]);
+        B.bc[k][0] = bc.x;
+        B.bc[k][1] = bc.y;
     }
     const int P = ppo_offsets(56).total;
     kin_ppo_adam_kernel<true><<<dim3((unsigned)((P + 1023) / 1024), (unsigned)n_members), 1024, 0, (cudaStream_t)stream>>>(

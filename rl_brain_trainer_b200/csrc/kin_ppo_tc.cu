@@ -44,8 +44,11 @@
 // relative per tensor (tests/test_gpu_ppo.py::test_minibatch_gradient_tc_*); log-probs move by O(1e-3), so a trainer whose
 // rollout sampled with the fp32 policy refreshes old_logp with THIS kernel's forward (forward_only); the fused collection
 // (kin_collect.cu) samples with the same bf16 arithmetic, so there the first-epoch ratio is 1 by construction.
+#include <cstdio>
+
 #include "kin_peer.cuh"
 #include "kin_ppo_layout.cuh"
+#include "kin_ppo_math.cuh"
 #include "kin_umma.cuh"
 
 namespace kin {
@@ -231,24 +234,8 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
     if (adv_stats) {
         if (tid == 0) { S.scal[0] = adv_stats[0]; S.scal[1] = adv_stats[1]; }
     } else if (tid < 32 && !forward_only && net == 0) {
-        double s1 = 0.0, s2 = 0.0;
-        for (int j = tid; j < 2 * n_pairs; j += 32) {
-            const int t = tile_ids[j];
-            s1 += tile_sums[2 * t];
-            s2 += tile_sums[2 * t + 1];
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-            s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-        }
-        if (tid == 0) {
-            const double nsamp = (double)n_pairs * TCG_ROWS;
-            const double mean = s1 / nsamp;
-            const double var = nsamp > 1.0 ? fmax((s2 - nsamp * mean * mean) / (nsamp - 1.0), 0.0) : 0.0;
-            S.scal[0] = hp.normalize_advantage ? (float)mean : 0.0f;
-            S.scal[1] = hp.normalize_advantage ? (float)(1.0 / (sqrt(var) + 1e-8)) : 1.0f;
-        }
+        const double2 s = warp_tile_sums(tile_sums, tile_ids, 2 * n_pairs, tid, 32);
+        if (tid == 0) adv_normaliser(s.x, s.y, (double)n_pairs * TCG_ROWS, hp.normalize_advantage, S.scal);
     }
     if (warp == 0) tmem_alloc(smem_u32(&S.tmem_base), TMEM_COLS_G);
     if (tid == 0) {
@@ -474,40 +461,37 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
 #pragma unroll
                     for (int d = 0; d < 7; ++d) {
                         z[d] = (act_r[d] - (o[d] + S.bo[d])) * S.inv_sig[d];
-                        lp += -0.5f * z[d] * z[d] - S.ls[d] - kHalfLog2Pi;
+                        lp += gauss_logp_term(z[d], S.ls[d]);
                     }
                     if (logp_out) logp_out[g] = lp;
                     if (!forward_only) {
-                        const float adv_n = (adv_r - S.scal[0]) * S.scal[1];
-                        const float log_ratio = lp - olp_r;
-                        const float ratio = expf(log_ratio);
-                        const float pl1 = adv_n * ratio, pl2 = adv_n * fminf(fmaxf(ratio, 1.0f - hp.clip_range), 1.0f + hp.clip_range);
-                        const float dpl_dlp = (pl1 <= pl2) ? -adv_n * ratio : 0.0f;
+                        const Surrogate sur = clipped_surrogate(adv_r, S.scal[0], S.scal[1], lp, olp_r, hp);
+                        const float dpl_dlp = sur.dpl_dlp();
                         float dm[7];
                         float ent = 0.0f;
 #pragma unroll
                         for (int d = 0; d < 7; ++d) {
-                            dm[d] = inv_global_batch * dpl_dlp * z[d] * S.inv_sig[d];
+                            dm[d] = dloss_dmean(inv_global_batch, dpl_dlp, z[d], S.inv_sig[d]);
                             dbo[d] += dm[d];
-                            dls[d] += inv_global_batch * dpl_dlp * (z[d] * z[d] - 1.0f) - inv_global_batch * hp.ent_coef;
-                            ent += 0.5f + kHalfLog2Pi + S.ls[d];
+                            dls[d] += dloss_dlog_std(inv_global_batch, dpl_dlp, z[d], hp);
+                            ent += gauss_entropy_term(S.ls[d]);
                         }
                         *reinterpret_cast<uint4*>(S.DO + sw_chunk(row, 0)) =
                             make_uint4(pack_bf16(dm[0], dm[1]), pack_bf16(dm[2], dm[3]), pack_bf16(dm[4], dm[5]), pack_bf16(dm[6], 0.0f));
-                        st[0] += -fminf(pl1, pl2);
+                        st[0] += sur.loss();
                         st[1] += ent;
-                        st[2] += (ratio - 1.0f) - log_ratio;
-                        st[3] += fabsf(ratio - 1.0f) > hp.clip_range ? 1.0f : 0.0f;
+                        st[2] += sur.approx_kl();
+                        st[3] += sur.clipped(hp);
                     }
                 } else {
                     const float v = o[7] + S.bo[7];
                     if (value_out) value_out[g] = v;
                     if (!forward_only) {
                         const float ret_r = S.ret[lb][row];
-                        const float dv = inv_global_batch * hp.vf_coef * 2.0f * (v - ret_r);
+                        const float dv = dloss_dvalue(inv_global_batch, v, ret_r, hp);
                         dbo[0] += dv;
                         *reinterpret_cast<uint4*>(S.DO + sw_chunk(row, 0)) = make_uint4(0u, 0u, 0u, pack_bf16(0.0f, dv));
-                        st[0] += (ret_r - v) * (ret_r - v);
+                        st[0] += value_loss(v, ret_r);
                     }
                 }
             }
@@ -640,10 +624,14 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
                 out[O.log_std + tid] = S.scal[8 + tid];
                 out[O.act_b + tid] = S.scal[16 + tid];
             }
-            // statistics slots: 0 policy loss, 2 entropy, 3 approx_kl, 4 clip fraction (actor CTAs); 1 value loss (critic CTAs)
-            if (tid == 0) { out[P + 0] = S.scal[2]; out[P + 2] = S.scal[3]; out[P + 3] = S.scal[4]; out[P + 4] = S.scal[5]; }
+            if (tid == 0) {
+                out[P + KIN_PPO_STAT_POLICY_LOSS] = S.scal[2];
+                out[P + KIN_PPO_STAT_ENTROPY] = S.scal[3];
+                out[P + KIN_PPO_STAT_APPROX_KL] = S.scal[4];
+                out[P + KIN_PPO_STAT_CLIP_FRACTION] = S.scal[5];
+            }
         } else if (tid == 0) {
-            out[P + 1] = S.scal[2];
+            out[P + KIN_PPO_STAT_VALUE_LOSS] = S.scal[2];
             out[O.val_b] = S.scal[16];
         }
         if constexpr (PEER) {       // every tile buffer is dead by now: the exchange borrows the X tile for its 1 KB of scratch
@@ -752,16 +740,20 @@ extern "C" int kin_ppo_grad_tc(const float* params, int in_dim, const KinPpoHype
                           stats, logp_out, value_out, forward_only, obs_is_image, adv_stats, weight_image, none, stream);
 }
 
-extern "C" int kin_ppo_grad_tc_exchange(const float* params, int in_dim, const KinPpoHyper* hp, const void* obs_any, const float* action, const float* old_logp,
-                                        const float* advantage, const float* returns, const double* tile_sums, const int* tile_ids, int n_tiles,
-                                        long long global_batch, float* partials, int grid, float* grad, float* stats, int obs_is_image,
-                                        const float* adv_stats, const void* weight_image, void* const* peer_buffers, int rank, int world, unsigned epoch,
-                                        int* timed_out, void* stream) {
-    if (!peer_buffers || !grad || !timed_out || world < 1 || world > PEER_MAX || rank < 0 || rank >= world || epoch == 0u)
-        return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_grad_tc_exchange: bad exchange arguments (epoch counts exchanges from 1)");
-    PeerFused px{};
+// the exchange arguments of kin_ppo_grad_tc_exchange / kin_ppo_grad_tc_update (`who`), checked, into px: KIN_OK or the failure
+static int peer_fused_setup(const char* who, void* const* peer_buffers, int rank, int world, unsigned epoch, float* grad, float* stats, int* timed_out,
+                            PeerFused& px) {
+    char msg[128];
+    if (!peer_buffers || !grad || !timed_out || world < 1 || world > PEER_MAX || rank < 0 || rank >= world || epoch == 0u) {
+        snprintf(msg, sizeof(msg), "%s: bad exchange arguments (epoch counts exchanges from 1)", who);
+        return kin_fail(KIN_ERR_INVALID_ARG, msg);
+    }
+    px = PeerFused{};
     for (int i = 0; i < world; ++i) {
-        if (!peer_buffers[i]) return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_grad_tc_exchange: null peer buffer");
+        if (!peer_buffers[i]) {
+            snprintf(msg, sizeof(msg), "%s: null peer buffer", who);
+            return kin_fail(KIN_ERR_INVALID_ARG, msg);
+        }
         px.peers.base[i] = static_cast<unsigned char*>(peer_buffers[i]);
     }
     px.rank = rank;
@@ -771,6 +763,17 @@ extern "C" int kin_ppo_grad_tc_exchange(const float* params, int in_dim, const K
     px.stats = stats;
     px.timed_out = timed_out;
     px.timeout_cycles = kin_peer_timeout_cycles();
+    return KIN_OK;
+}
+
+extern "C" int kin_ppo_grad_tc_exchange(const float* params, int in_dim, const KinPpoHyper* hp, const void* obs_any, const float* action, const float* old_logp,
+                                        const float* advantage, const float* returns, const double* tile_sums, const int* tile_ids, int n_tiles,
+                                        long long global_batch, float* partials, int grid, float* grad, float* stats, int obs_is_image,
+                                        const float* adv_stats, const void* weight_image, void* const* peer_buffers, int rank, int world, unsigned epoch,
+                                        int* timed_out, void* stream) {
+    PeerFused px;
+    const int rc = peer_fused_setup("kin_ppo_grad_tc_exchange", peer_buffers, rank, world, epoch, grad, stats, timed_out, px);
+    if (rc != KIN_OK) return rc;
     return grad_tc_launch(params, in_dim, hp, obs_any, action, old_logp, advantage, returns, tile_sums, tile_ids, n_tiles, global_batch, partials, grid, grad,
                           stats, nullptr, nullptr, 0, obs_is_image, adv_stats, weight_image, px, stream);
 }
@@ -783,30 +786,20 @@ extern "C" int kin_ppo_grad_tc_update(const float* params, int in_dim, const Kin
                                       const float* adv_stats, void* weight_image, void* const* peer_buffers, int rank, int world, unsigned epoch,
                                       int* timed_out, float* params_rw, float* adam_m, float* adam_v, int step, float* stats_accum, float* norm_scratch,
                                       void* stream) {
-    if (!peer_buffers || !grad || !timed_out || world < 1 || world > PEER_MAX || rank < 0 || rank >= world || epoch == 0u)
-        return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_grad_tc_update: bad exchange arguments (epoch counts exchanges from 1)");
+    PeerFused px;
+    const int rc = peer_fused_setup("kin_ppo_grad_tc_update", peer_buffers, rank, world, epoch, grad, stats, timed_out, px);
+    if (rc != KIN_OK) return rc;
     if (!params_rw || params_rw != params || !adam_m || !adam_v || !norm_scratch || !stats || step < 1 || !hp)
         return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_grad_tc_update: bad optimiser arguments (params_rw must be params; norm_scratch holds 2 * grid floats)");
-    PeerFused px{};
-    for (int i = 0; i < world; ++i) {
-        if (!peer_buffers[i]) return kin_fail(KIN_ERR_INVALID_ARG, "kin_ppo_grad_tc_update: null peer buffer");
-        px.peers.base[i] = static_cast<unsigned char*>(peer_buffers[i]);
-    }
-    px.rank = rank;
-    px.world = world;
-    px.epoch = epoch;
-    px.grad = grad;
-    px.stats = stats;
-    px.timed_out = timed_out;
-    px.timeout_cycles = kin_peer_timeout_cycles();
     px.adam.params = params_rw;
     px.adam.m = adam_m;
     px.adam.v = adam_v;
     px.adam.wimg = in_dim == 56 ? static_cast<unsigned short*>(weight_image) : nullptr;      // the folded route image is rebuilt by kin_ppo_pack_weights
     px.adam.stats_accum = stats_accum;
     px.adam.norm_part = norm_scratch;
-    px.adam.bc1 = 1.0f - powf(hp->adam_beta1, (float)step);
-    px.adam.bc2 = 1.0f - powf(hp->adam_beta2, (float)step);
+    const float2 bc = adam_bias_corrections(*hp, step);
+    px.adam.bc1 = bc.x;
+    px.adam.bc2 = bc.y;
     px.adam.in_dim = in_dim;
     return grad_tc_launch(params, in_dim, hp, obs_any, action, old_logp, advantage, returns, tile_sums, tile_ids, n_tiles, global_batch, partials, grid, grad,
                           stats, nullptr, nullptr, 0, obs_is_image, adv_stats, weight_image, px, stream);

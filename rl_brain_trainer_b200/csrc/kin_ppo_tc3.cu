@@ -34,6 +34,7 @@
 // from if the operand traffic is cut (A operands from TMEM for the four chain GEMMs would remove 52 of the 196 KB per tile).
 #include "kin_peer.cuh"
 #include "kin_ppo_layout.cuh"
+#include "kin_ppo_math.cuh"
 #include "kin_umma.cuh"
 
 namespace kin {
@@ -195,24 +196,8 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
     if (adv_stats) {
         if (tid == 0) { S.scal[0] = adv_stats[0]; S.scal[1] = adv_stats[1]; }
     } else if (tid < 32 && net == 0) {
-        double s1 = 0.0, s2 = 0.0;
-        for (int j = tid; j < 2 * n_pairs; j += 32) {
-            const int t = tile_ids[j];
-            s1 += tile_sums[2 * t];
-            s2 += tile_sums[2 * t + 1];
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-            s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-        }
-        if (tid == 0) {
-            const double nsamp = (double)n_pairs * ROWS;
-            const double mean = s1 / nsamp;
-            const double var = nsamp > 1.0 ? fmax((s2 - nsamp * mean * mean) / (nsamp - 1.0), 0.0) : 0.0;
-            S.scal[0] = hp.normalize_advantage ? (float)mean : 0.0f;
-            S.scal[1] = hp.normalize_advantage ? (float)(1.0 / (sqrt(var) + 1e-8)) : 1.0f;
-        }
+        const double2 s = warp_tile_sums(tile_sums, tile_ids, 2 * n_pairs, tid, 32);
+        if (tid == 0) adv_normaliser(s.x, s.y, (double)n_pairs * ROWS, hp.normalize_advantage, S.scal);
     }
     if (warp == 1) tmem_alloc(smem_u32(&S.tmem_base), TMEM_COLS);
     if (tid == 0) {
@@ -468,35 +453,32 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
 #pragma unroll
                     for (int d = 0; d < 7; ++d) {
                         z[d] = (act_r[d] - (o[WO_ROW + d] + S.bo[d])) * S.inv_sig[d];
-                        lp += -0.5f * z[d] * z[d] - S.ls[d] - kHalfLog2Pi;
+                        lp += gauss_logp_term(z[d], S.ls[d]);
                     }
-                    const float adv_n = (adv_r - S.scal[0]) * S.scal[1];
-                    const float log_ratio = lp - olp_r;
-                    const float ratio = expf(log_ratio);
-                    const float pl1 = adv_n * ratio, pl2 = adv_n * fminf(fmaxf(ratio, 1.0f - hp.clip_range), 1.0f + hp.clip_range);
-                    const float dpl_dlp = (pl1 <= pl2) ? -adv_n * ratio : 0.0f;
+                    const Surrogate sur = clipped_surrogate(adv_r, S.scal[0], S.scal[1], lp, olp_r, hp);
+                    const float dpl_dlp = sur.dpl_dlp();
                     float dm[7];
                     float ent = 0.0f;
 #pragma unroll
                     for (int d = 0; d < 7; ++d) {
-                        dm[d] = inv_global_batch * dpl_dlp * z[d] * S.inv_sig[d];
+                        dm[d] = dloss_dmean(inv_global_batch, dpl_dlp, z[d], S.inv_sig[d]);
                         dbo[d] += dm[d];
-                        dls[d] += inv_global_batch * dpl_dlp * (z[d] * z[d] - 1.0f) - inv_global_batch * hp.ent_coef;
-                        ent += 0.5f + kHalfLog2Pi + S.ls[d];
+                        dls[d] += dloss_dlog_std(inv_global_batch, dpl_dlp, z[d], hp);
+                        ent += gauss_entropy_term(S.ls[d]);
                     }
                     *reinterpret_cast<uint4*>(X + sw_chunk(row, 7)) =        // columns 56..63: the constant one, then dO
                         make_uint4(pack_bf16(1.0f, dm[0]), pack_bf16(dm[1], dm[2]), pack_bf16(dm[3], dm[4]), pack_bf16(dm[5], dm[6]));
-                    st[0] += -fminf(pl1, pl2);
+                    st[0] += sur.loss();
                     st[1] += ent;
-                    st[2] += (ratio - 1.0f) - log_ratio;
-                    st[3] += fabsf(ratio - 1.0f) > hp.clip_range ? 1.0f : 0.0f;
+                    st[2] += sur.approx_kl();
+                    st[3] += sur.clipped(hp);
                 } else {
                     const float v = o[WO_ROW] + S.bo[7];
                     const float ret_r = S.adv[sid][row];
-                    const float dv = inv_global_batch * hp.vf_coef * 2.0f * (v - ret_r);
+                    const float dv = dloss_dvalue(inv_global_batch, v, ret_r, hp);
                     dbo[0] += dv;
                     *reinterpret_cast<uint4*>(X + sw_chunk(row, 7)) = make_uint4(pack_bf16(1.0f, dv), 0u, 0u, 0u);
-                    st[0] += (ret_r - v) * (ret_r - v);
+                    st[0] += value_loss(v, ret_r);
                 }
             }
             tile_written<true>(mb_rdy, lane);
@@ -610,10 +592,14 @@ kin_ppo_grad_tc3_kernel(const float* __restrict__ params, KinPpoHyper hp, const 
             out[O.log_std + tid] = S.scal[8 + tid];
             out[O.act_b + tid] = S.scal[16 + tid];
         }
-        // statistics slots: 0 policy loss, 2 entropy, 3 approx_kl, 4 clip fraction (actor CTAs); 1 value loss (critic CTAs)
-        if (tid == 0) { out[P + 0] = S.scal[2]; out[P + 2] = S.scal[3]; out[P + 3] = S.scal[4]; out[P + 4] = S.scal[5]; }
+        if (tid == 0) {
+            out[P + KIN_PPO_STAT_POLICY_LOSS] = S.scal[2];
+            out[P + KIN_PPO_STAT_ENTROPY] = S.scal[3];
+            out[P + KIN_PPO_STAT_APPROX_KL] = S.scal[4];
+            out[P + KIN_PPO_STAT_CLIP_FRACTION] = S.scal[5];
+        }
     } else if (tid == 0) {
-        out[P + 1] = S.scal[2];
+        out[P + KIN_PPO_STAT_VALUE_LOSS] = S.scal[2];
         out[O.val_b] = S.scal[16];
     }
     if constexpr (PEER) {       // every tile buffer is dead by now: the exchange borrows an X tile for its 1 KB of scratch

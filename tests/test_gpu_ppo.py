@@ -116,12 +116,19 @@ def test_minibatch_gradient_matches_autograd():
     tile_ids = torch.tensor([3, 17, 0, 39, 8, 21, 22, 5, 30, 11, 12, 1], dtype=torch.int32, device="cuda")
     P = flat.numel()
     ctas = 5
-    partials = torch.zeros((ctas, P + 16), device="cuda")
-    grad, stats = torch.zeros(P, device="cuda"), torch.zeros(8, device="cuda")
     c_hp = hp.c()
-    _lib.check(_lib.lib().kin_ppo_grad(flat.data_ptr(), 56, ctypes.byref(c_hp), obs.data_ptr(), act.data_ptr(), old_logp.data_ptr(), adv.data_ptr(),
-                                       ret.data_ptr(), sums.data_ptr(), tile_ids.data_ptr(), tile_ids.numel(), tile_ids.numel() * 64,
-                                       partials.data_ptr(), ctas, grad.data_ptr(), stats.data_ptr(), None, torch.cuda.current_stream().cuda_stream))
+
+    def launch():
+        partials = torch.zeros((ctas, P + 16), device="cuda")
+        grad, stats = torch.zeros(P, device="cuda"), torch.zeros(8, device="cuda")
+        _lib.check(_lib.lib().kin_ppo_grad(flat.data_ptr(), 56, ctypes.byref(c_hp), obs.data_ptr(), act.data_ptr(), old_logp.data_ptr(), adv.data_ptr(),
+                                           ret.data_ptr(), sums.data_ptr(), tile_ids.data_ptr(), tile_ids.numel(), tile_ids.numel() * 64,
+                                           partials.data_ptr(), ctas, grad.data_ptr(), stats.data_ptr(), None, torch.cuda.current_stream().cuda_stream))
+        return grad, stats
+
+    grad, stats = launch()
+    grad2, stats2 = launch()
+    assert torch.equal(grad, grad2) and torch.equal(stats, stats2)      # every sum in a fixed order: the kernel is deterministic
     idx = (tile_ids.long()[:, None] * 64 + torch.arange(64, device="cuda")[None]).reshape(-1)
     for t in pol.tensors.values():
         t.requires_grad_(True)
