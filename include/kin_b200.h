@@ -922,6 +922,55 @@ int kin_pop_grad_tc(const KinPopMember *members, int n_members, int minibatch, i
  * kin_ppo_adam computes them, so host_hypers[k] must equal member k's descriptor hyper.                                            */
 int kin_pop_adam(const KinPopMember *members, int n_members, const KinPpoHyper *host_hypers, const int *host_steps, void *stream);
 
+/* ---- route populations: K independent 80-input route trainers (kin_route_collect + kin_ppo_grad_tc(80) on folded images +
+ * kin_ppo_adam + kin_ppo_pack_weights(80)) through the same launches.  A route member has TWO descriptors at the same index: its
+ * KinPopMember row (obs_tiles = its folded observation images [T][n/128][16 KB], weight_image = its folded weight image, sampler unused)
+ * and its KinPopRouteMember row below (fp32 observation rows, route flags, reset window).  Members share the route table, the env params,
+ * the sequence mode and reset_ready_streak_on_advance; kin_pop_gae and kin_pop_adv_stats serve route members unchanged.
+ * Every member's reset window must lie inside the route (kin_route_collect's check; the descriptors live on the device, so the caller
+ * checks them before the upload).  KinPopMember rows keep their layout; KIN_ABI_VERSION stays 4.                                    */
+typedef struct KinPopRouteMember {
+    float *obs;                        /* [T + 1][n][80] fp32 observation rows, as kin_route_collect writes them */
+    int *route_flags;                  /* [T][n] */
+    KinRouteResetParams reset;         /* the member's reset config and route window (kin_route_collect's host_reset) */
+    int pad0;
+} KinPopRouteMember;
+
+/* Replaces: collect_rollouts over the route VecEnv, once per member, for steps t0 .. t0 + n_steps of the rollout:
+ * kin_route_collect(handle, host_route, &route_member.reset, member.state, member.stride, n_envs, member.params, n_steps,
+ * member.noise_seed, member.first_step + t0, member.reset_seed, sequence_mode, reset_ready_streak_on_advance, rows t0 .. of the
+ * member's obs / action / logp / value / reward / done / episode_start / route_flags, member.start_io, member.last_value, the member's
+ * bootstrap list, tiles_per_cta = 1) -- the call a standalone trainer makes for one chunk of a chunked rollout.  Zeroes the members'
+ * bootstrap counts first, as kin_route_collect does.  handle supplies the shared env params; the route table is shared.           */
+int kin_pop_route_collect(void *handle, const KinRouteTable *host_route, const KinPopMember *members, const KinPopRouteMember *route_members,
+                          int n_members, int n_envs, int n_steps, int t0, int sequence_mode, int reset_ready_streak_on_advance, void *stream);
+
+/* kin_ppo_bootstrap_list(member.params, 80, member's list, member.boot_cap, member.reward + t0 * n_envs, member.hyper.gamma) for every
+ * member: the list indices of a chunk are relative to the chunk's first row t0.  max_boot_cap >= every member's boot_cap.          */
+int kin_pop_route_bootstrap_list(const KinPopMember *members, int n_members, int n_envs, int max_boot_cap, int t0, void *stream);
+
+/* kin_route_obs_images(route_member.obs, n_rows, member.obs_tiles) for every member; n_rows a multiple of 128.                       */
+int kin_pop_route_obs_images(const KinPopMember *members, const KinPopRouteMember *route_members, int n_members, long long n_rows,
+                             void *stream);
+
+/* The log-prob refresh of the route update (PPOTrainer.refresh_old_logp), once per member: kin_ppo_grad_tc(member.params, 80,
+ * &member.hyper, member.obs_tiles, member.action, NULL, NULL, NULL, NULL, tile_ids, n_tiles, 0, NULL, grid, NULL, NULL, member.logp,
+ * NULL, 1, 1, NULL, member.weight_image).  tile_ids: device [n_tiles], shared by all members (the refresh passes 0 .. n_tiles - 1). */
+int kin_pop_route_logp(const KinPopMember *members, int n_members, const int *tile_ids, int n_tiles, int grid, void *stream);
+
+/* Replaces: one minibatch of SB3 ppo.py train() (loss and backward), once per member: kin_pop_grad_tc's call with in_dim = 80 --
+ * kin_ppo_grad_tc(member.params, 80, &member.hyper, member.obs_tiles, .., member.tile_ids + minibatch * n_tiles_per_minibatch,
+ * n_tiles_per_minibatch, global_batch, member.partials, grid, member.grad, member.stats, NULL, NULL, 0, 1,
+ * member.adv_stats + 2 * minibatch, member.weight_image), gradient kernel and reduction.                                           */
+int kin_pop_route_grad_tc(const KinPopMember *members, int n_members, int minibatch, int n_tiles_per_minibatch, long long global_batch, int grid,
+                          void *stream);
+
+/* Replaces: clip_grad_norm_ + optimizer.step, once per member, and the rebuild of the folded weight image: kin_ppo_adam(member.params,
+ * member.grad, member.adam_m, member.adam_v, P(80), &member.hyper, host_steps[k], member.stats, member.stats_accum, NULL, 80) followed by
+ * kin_ppo_pack_weights(member.params, 80, member.weight_image).  Two launches for all members.  host_hypers / host_steps as for
+ * kin_pop_adam.                                                                                                                    */
+int kin_pop_route_adam(const KinPopMember *members, int n_members, const KinPpoHyper *host_hypers, const int *host_steps, void *stream);
+
 /* ---- gradient exchange over NVLink peer memory (the training path's one collective; SURVEY 8e(ii)) ------------------------------
  * Replaces: the per-minibatch all-reduce (sum) of the flat gradient + 5 loss statistics between the gradient kernel and Adam.
  * Every rank (one per GPU of ONE node, world <= 8) owns a receive buffer; peers open it through CUDA IPC.  Per exchange:

@@ -169,6 +169,12 @@ def lib() -> ctypes.CDLL:
     L.kin_pop_adv_stats.argtypes = [vp, i32, i32, i32, vp]
     L.kin_pop_grad_tc.argtypes = [vp, i32, i32, i32, i64, i32, vp]
     L.kin_pop_adam.argtypes = [vp, i32, vp, vp, vp]
+    L.kin_pop_route_collect.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp]
+    L.kin_pop_route_bootstrap_list.argtypes = [vp, i32, i32, i32, i32, vp]
+    L.kin_pop_route_obs_images.argtypes = [vp, vp, i32, i64, vp]
+    L.kin_pop_route_logp.argtypes = [vp, i32, vp, i32, i32, vp]
+    L.kin_pop_route_grad_tc.argtypes = [vp, i32, i32, i32, i64, i32, vp]
+    L.kin_pop_route_adam.argtypes = [vp, i32, vp, vp, vp]
     L.kin_peer_buffer_bytes.argtypes = [i32, i32]
     L.kin_peer_buffer_create.argtypes = [i32, i32, ctypes.POINTER(vp), ctypes.c_char_p]
     L.kin_peer_buffer_open.argtypes = [ctypes.c_char_p, ctypes.POINTER(vp)]

@@ -159,11 +159,13 @@ kin_collect_kernel(const __grid_constant__ KinEnvParams P, const KinSamplerParam
 }
 
 // r[idx] += gamma * V(terminal_obs) for the truncated episodes the collection kernel listed (strict fp32 critic)
-// POP: params carries the KinPopMember table, member blockIdx.y's list, critic, rewards and gamma replace the arguments
-template <int IN, bool POP = false>
+// POP: params carries the KinPopMember table, member blockIdx.y's list, critic, rewards and gamma replace the arguments.  The route
+// population passes one extra argument, the element offset of the chunk's first reward row (list indices are relative to the chunk).
+template <int IN, bool POP = false, class... PopArgs>
 __global__ void __launch_bounds__(128)
 kin_bootstrap_list_kernel(const float* __restrict__ params, const float* __restrict__ boot_obs, const int* __restrict__ boot_index,
-                          const int* __restrict__ boot_count, int cap, float* __restrict__ reward, float gamma) {
+                          const int* __restrict__ boot_count, int cap, float* __restrict__ reward, float gamma, PopArgs... pop) {
+    static_assert(sizeof...(PopArgs) <= (POP ? 1 : 0), "the chunk offset is a population argument");
     if constexpr (POP) {
         const KinPopMember& M = reinterpret_cast<const KinPopMember*>(params)[blockIdx.y];
         params = M.params;
@@ -173,6 +175,7 @@ kin_bootstrap_list_kernel(const float* __restrict__ params, const float* __restr
         cap = M.boot_cap;
         reward = M.reward;
         gamma = M.hyper.gamma;
+        if constexpr (sizeof...(PopArgs) == 1) reward += (pop, ...);
     }
     const PpoOffsets O = ppo_offsets(IN);
     const int count = min(*boot_count, cap);
@@ -216,6 +219,11 @@ static cudaError_t launch_collect(const KinHandle* h, float* state, int stride, 
 
 __global__ void kin_pop_zero_counts_kernel(const KinPopMember* __restrict__ members, int n_members) {
     if ((int)threadIdx.x < n_members) *members[threadIdx.x].boot_count = 0;
+}
+
+cudaError_t pop_zero_boot_counts(const KinPopMember* members, int n_members, cudaStream_t st) {
+    kin_pop_zero_counts_kernel<<<1, KIN_POP_MAX, 0, st>>>(members, n_members);
+    return cudaGetLastError();
 }
 
 }  // namespace kin
@@ -267,10 +275,11 @@ extern "C" int kin_pop_collect(void* handle, const KinPopMember* members, int n_
     if (n_envs <= 0 || (n_envs % AC_ROWS) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_collect: n_envs must be a positive multiple of 128 (one GEMM tile)");
     if (mode != KIN_MODE_APPROACH && mode != KIN_MODE_DOCK) return kin_fail(KIN_ERR_UNSUPPORTED, "kin_pop_collect: mode must be approach (0) or dock (1)");
     cudaStream_t st = (cudaStream_t)stream;
-    kin_pop_zero_counts_kernel<<<1, KIN_POP_MAX, 0, st>>>(members, n_members);      // kin_ppo_collect's reset of *boot_count
+    cudaError_t e = pop_zero_boot_counts(members, n_members, st);      // kin_ppo_collect's reset of *boot_count
+    if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_collect: zero counts");
     auto kernel = mode == KIN_MODE_APPROACH ? kin_collect_kernel<1, KIN_MODE_APPROACH, true> : kin_collect_kernel<1, KIN_MODE_DOCK, true>;
     const size_t smem = sizeof(CollectSmem<1>) + 1024;
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_collect: smem attribute");
     kernel<<<dim3((unsigned)(n_envs / AC_ROWS), (unsigned)n_members), AC_ROWS, smem, st>>>(h->params, reinterpret_cast<const KinSamplerParams*>(members), nullptr, 0,
                                                                                           n_envs, nullptr, nullptr, n_steps, 0, 0u, 0, CollectOut{});
@@ -286,4 +295,14 @@ extern "C" int kin_pop_bootstrap_list(const KinPopMember* members, int n_members
         reinterpret_cast<const float*>(members), nullptr, nullptr, nullptr, 0, nullptr, 0.0f);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_bootstrap_list");
+}
+
+extern "C" int kin_pop_route_bootstrap_list(const KinPopMember* members, int n_members, int n_envs, int max_boot_cap, int t0, void* stream) {
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || n_envs <= 0 || max_boot_cap <= 0 || t0 < 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_bootstrap_list: need a device member table, 1 <= n_members <= KIN_POP_MAX, n_envs > 0, "
+                                             "max_boot_cap > 0 and t0 >= 0");
+    kin_bootstrap_list_kernel<80, true, long long><<<dim3((unsigned)((max_boot_cap + 127) / 128), (unsigned)n_members), 128, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(members), nullptr, nullptr, nullptr, 0, nullptr, 0.0f, (long long)t0 * n_envs);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_bootstrap_list");
 }

@@ -281,6 +281,9 @@ __device__ __forceinline__ void push_truncated(const Out& out, unsigned done, si
 }
 
 // tiles per CTA: the requested count, or (requested <= 0) the fewest that still fit the batch in one wave of CTAs (one CTA per SM)
+// *boot_count = 0 for every member of a population (kin_collect.cu): the reset kin_ppo_collect / kin_route_collect make, one launch for all
+cudaError_t pop_zero_boot_counts(const KinPopMember* members, int n_members, cudaStream_t st);
+
 inline int collect_tiles_per_cta(int requested, int n_envs) {
     if (requested > 0) return requested;
     int sms = 148, dev = 0;

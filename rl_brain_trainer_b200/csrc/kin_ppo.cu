@@ -606,7 +606,9 @@ struct PopBiasCorrection {
     float bc[KIN_POP_MAX][2];
 };
 
-template <bool POP = false, class... PopArgs>
+// POP_IMAGE (populations only): keep member.weight_image in step in place (56 inputs); false leaves it alone (the folded route image is
+// rebuilt by kin_ppo_pack_weights_kernel<true> afterwards, as the standalone route update calls kin_ppo_adam(NULL) + kin_ppo_pack_weights)
+template <bool POP = false, bool POP_IMAGE = true, class... PopArgs>
 __global__ void __launch_bounds__(1024)
 kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, float* __restrict__ m, float* __restrict__ v, int P,
                     KinPpoHyper hp, float bc1, float bc2, float* __restrict__ stats, float* __restrict__ stats_accum,
@@ -624,7 +626,7 @@ kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, 
         bc2 = B.bc[blockIdx.y][1];
         stats = M.stats;
         stats_accum = M.stats_accum;
-        wimg = static_cast<unsigned short*>(M.weight_image);
+        wimg = POP_IMAGE ? static_cast<unsigned short*>(M.weight_image) : nullptr;
     }
     __shared__ float red[32];
     __shared__ float coef;
@@ -682,10 +684,25 @@ kin_ppo_adam_kernel(float* __restrict__ params, const float* __restrict__ grad, 
 }
 
 // full (re)build of the bf16 operand image from the flat parameters
+// POP (kin_pop_route_adam): params carries the KinPopMember table, member blockIdx.y's parameters and image replace the arguments.  The
+// standalone entry zeroes the image before the launch; here the kernel writes those zeros itself: the only image bytes no parameter
+// maps to are the padding rows of the two WO blocks (actor rows 7..15, critic rows 0..6 and 8..15).
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_ppo_pack_weights_kernel(const float* __restrict__ params, int in_dim, unsigned short* __restrict__ wimg) {
+    if constexpr (POP) {
+        const KinPopMember& M = reinterpret_cast<const KinPopMember*>(params)[blockIdx.y];
+        params = M.params;
+        wimg = static_cast<unsigned short*>(M.weight_image);
+    }
     const PpoOffsets O = ppo_offsets(in_dim);
     const int i = blockIdx.x * 256 + threadIdx.x;
+    if constexpr (POP) {
+        if (i < 2 * 16 * 64) {
+            const int blk = i >> 10, r = (i >> 6) & 15;
+            if (blk == 0 ? r >= 7 : r != 7) wimg[(KIN_WIMG_WO + blk * 2048 + wimg_elem(r, i & 63)) >> 1] = 0;
+        }
+    }
     if (in_dim == 80) {       // folded layer 1: one thread per image element of the two W0 blocks; the rest as for 56 inputs
         if (i < 2 * 64 * 64) {
             const int net = i >> 12, u = (i >> 6) & 63, k = i & 63;
@@ -715,8 +732,15 @@ kin_ppo_pack_weights_kernel(const float* __restrict__ params, int in_dim, unsign
 
 // route observations [n_rows][80] fp32 -> folded bf16 operand images [n_rows / 128][16 KB] ([60 live columns | 1 | 0 0 0] rows,
 // SWIZZLE_128B): what kin_ppo_grad_tc(in_dim = 80, obs_is_image = 1) stages with one bulk copy per tile.  One thread per 16-byte chunk.
+// POP (kin_pop_route_obs_images): obs carries the KinPopRouteMember table and img the KinPopMember table; member blockIdx.y's fp32 rows go
+// to its folded images.
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 kin_route_obs_images_kernel(const float* __restrict__ obs, long long n_rows, unsigned char* __restrict__ img) {
+    if constexpr (POP) {
+        obs = reinterpret_cast<const KinPopRouteMember*>(obs)[blockIdx.y].obs;
+        img = static_cast<unsigned char*>(reinterpret_cast<const KinPopMember*>(img)[blockIdx.y].obs_tiles);
+    }
     const long long i = (long long)blockIdx.x * 256 + threadIdx.x;      // row * 8 + chunk
     if (i >= n_rows * 8) return;
     const long long row = i >> 3;
@@ -988,4 +1012,32 @@ extern "C" int kin_pop_adam(const KinPopMember* members, int n_members, const Ki
         nullptr, reinterpret_cast<const float*>(members), nullptr, nullptr, P, KinPpoHyper{}, 0.0f, 0.0f, nullptr, nullptr, nullptr, 56, B);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_adam");
+}
+
+extern "C" int kin_pop_route_obs_images(const KinPopMember* members, const KinPopRouteMember* route_members, int n_members, long long n_rows, void* stream) {
+    if (!pop_args_ok(members, n_members) || !route_members || n_rows <= 0 || (n_rows % 128) != 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_obs_images: bad arguments (n_rows must be a positive multiple of 128)");
+    const long long chunks = n_rows * 8;
+    kin_route_obs_images_kernel<true><<<dim3((unsigned)((chunks + 255) / 256), (unsigned)n_members), 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(route_members), n_rows, reinterpret_cast<unsigned char*>(const_cast<KinPopMember*>(members)));
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_obs_images");
+}
+
+extern "C" int kin_pop_route_adam(const KinPopMember* members, int n_members, const KinPpoHyper* host_hypers, const int* host_steps, void* stream) {
+    if (!pop_args_ok(members, n_members) || !host_hypers || !host_steps) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_adam: bad arguments");
+    PopBiasCorrection B{};
+    for (int k = 0; k < n_members; ++k) {
+        if (host_steps[k] < 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_adam: steps count optimiser steps from 1");
+        const float2 bc = adam_bias_corrections(host_hypers[k], host_steps[k]);
+        B.bc[k][0] = bc.x;
+        B.bc[k][1] = bc.y;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int P = ppo_offsets(80).total;
+    kin_ppo_adam_kernel<true, false><<<dim3((unsigned)((P + 1023) / 1024), (unsigned)n_members), 1024, 0, st>>>(
+        nullptr, reinterpret_cast<const float*>(members), nullptr, nullptr, P, KinPpoHyper{}, 0.0f, 0.0f, nullptr, nullptr, nullptr, 80, B);
+    kin_ppo_pack_weights_kernel<true><<<dim3((unsigned)((P + 255) / 256), (unsigned)n_members), 256, 0, st>>>(reinterpret_cast<const float*>(members), 80, nullptr);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_adam");
 }

@@ -161,8 +161,9 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
                        float* __restrict__ partials, float* __restrict__ logp_out, float* __restrict__ value_out, int forward_only, int net_base,
                        const float* __restrict__ adv_stats, const unsigned char* __restrict__ wimg, const PeerFused px, PopArgs... pop) {
     static_assert(IN == 56 || (IN == 80 && IMG), "56-input policies (fp32 observations or images) or the 80-input route policy (folded images)");
-    static_assert(sizeof...(PopArgs) == (POP ? 1 : 0) && (!POP || (IMG && IN == 56 && !PEER)), "population: 56-input images, one extra argument");
+    static_assert(sizeof...(PopArgs) == (POP ? 1 : 0) && (!POP || (IMG && !PEER)), "population: images, no peer exchange, one extra argument");
     if constexpr (POP) {
+        const int* const shared_ids = tile_ids;
         const int minibatch = (pop, ...);
         const KinPopMember& M = reinterpret_cast<const KinPopMember*>(params)[blockIdx.z];
         params = M.params;
@@ -177,6 +178,15 @@ kin_ppo_grad_tc_kernel(const float* __restrict__ params, KinPpoHyper hp, const f
         partials = M.partials;
         adv_stats = M.adv_stats + 2 * minibatch;
         wimg = static_cast<const unsigned char*>(M.weight_image);
+        if constexpr (IN == 80) {
+            if (forward_only) {      // kin_pop_route_logp: refresh_old_logp's launch -- the shared tile list, log-probs into member.logp
+                old_logp = advantage = returns = adv_stats = nullptr;
+                tile_sums = nullptr;
+                partials = nullptr;
+                tile_ids = shared_ids;
+                logp_out = M.logp;
+            }
+        }
     }
     constexpr int KT = 1;                            // K tiles of layer 1
     constexpr int K1 = 64;                           // padded reduction width of layer 1 (live inputs | 1 | zeros)
@@ -806,6 +816,16 @@ extern "C" int kin_ppo_grad_tc_update(const float* params, int in_dim, const Kin
 }
 
 
+// the dynamic shared-memory attribute of a population gradient instance, once per device
+template <class Kernel>
+static cudaError_t pop_smem_attr(Kernel kernel, bool* attr_set) {
+    const int dev_slot = kin_device_slot();
+    if (attr_set[dev_slot]) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(TcGradSmem<1>) + 1024));
+    attr_set[dev_slot] = e == cudaSuccess;
+    return e;
+}
+
 extern "C" int kin_pop_grad_tc(const KinPopMember* members, int n_members, int minibatch, int n_tiles_per_minibatch, long long global_batch, int grid,
                                void* stream) {
     if (!members || n_members <= 0 || n_members > KIN_POP_MAX || minibatch < 0 || n_tiles_per_minibatch <= 0 || global_batch <= 0 || grid <= 0)
@@ -814,12 +834,8 @@ extern "C" int kin_pop_grad_tc(const KinPopMember* members, int n_members, int m
     auto kernel = kin_ppo_grad_tc_kernel<true, 56, false, true, int>;
     const size_t smem = sizeof(TcGradSmem<1>) + 1024;
     static bool attr_set[KIN_MAX_DEVICES] = {};
-    const int dev_slot = kin_device_slot();
-    if (!attr_set[dev_slot]) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_grad_tc: smem attribute");
-        attr_set[dev_slot] = true;
-    }
+    const cudaError_t ea = pop_smem_attr(kernel, attr_set);
+    if (ea != cudaSuccess) return kin_fail_cuda(ea, "kin_pop_grad_tc: smem attribute");
     cudaStream_t st = (cudaStream_t)stream;
     const int n_pairs = n_tiles_per_minibatch / 2;
     const int g = grid < n_pairs ? grid : n_pairs;      // kin_ppo_grad_tc's clamp: the same CTAs, tiles per CTA and partial rows per member
@@ -831,4 +847,45 @@ extern "C" int kin_pop_grad_tc(const KinPopMember* members, int n_members, int m
     kin_pop_reduce_launch(members, n_members, g, ppo_offsets(56).total, inv, st);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_grad_tc");
+}
+
+extern "C" int kin_pop_route_grad_tc(const KinPopMember* members, int n_members, int minibatch, int n_tiles_per_minibatch, long long global_batch, int grid,
+                                     void* stream) {
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || minibatch < 0 || n_tiles_per_minibatch <= 0 || global_batch <= 0 || grid <= 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_grad_tc: bad arguments");
+    if (n_tiles_per_minibatch & 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_grad_tc: n_tiles must be even (two 64-sample tiles per 128-row GEMM tile)");
+    auto kernel = kin_ppo_grad_tc_kernel<true, 80, false, true, int>;
+    static bool attr_set[KIN_MAX_DEVICES] = {};
+    const cudaError_t ea = pop_smem_attr(kernel, attr_set);
+    if (ea != cudaSuccess) return kin_fail_cuda(ea, "kin_pop_route_grad_tc: smem attribute");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n_pairs = n_tiles_per_minibatch / 2;
+    const int g = grid < n_pairs ? grid : n_pairs;
+    const float inv = 1.0f / (float)global_batch;
+    const PeerFused none{};
+    kernel<<<dim3((unsigned)g, 2u, (unsigned)n_members), TCG_THREADS, sizeof(TcGradSmem<1>) + 1024, st>>>(
+        reinterpret_cast<const float*>(members), KinPpoHyper{}, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n_pairs, inv, nullptr, nullptr,
+        nullptr, 0, 0, nullptr, nullptr, none, minibatch);
+    kin_pop_reduce_launch(members, n_members, g, ppo_offsets(80).total, inv, st);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_grad_tc");
+}
+
+extern "C" int kin_pop_route_logp(const KinPopMember* members, int n_members, const int* tile_ids, int n_tiles, int grid, void* stream) {
+    if (!members || n_members <= 0 || n_members > KIN_POP_MAX || !tile_ids || n_tiles <= 0 || grid <= 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_logp: bad arguments");
+    if (n_tiles & 1) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_logp: n_tiles must be even (two 64-sample tiles per 128-row GEMM tile)");
+    auto kernel = kin_ppo_grad_tc_kernel<true, 80, false, true, int>;
+    static bool attr_set[KIN_MAX_DEVICES] = {};
+    const cudaError_t ea = pop_smem_attr(kernel, attr_set);
+    if (ea != cudaSuccess) return kin_fail_cuda(ea, "kin_pop_route_logp: smem attribute");
+    const int n_pairs = n_tiles / 2;
+    const int g = grid < n_pairs ? grid : n_pairs;
+    const PeerFused none{};
+    // forward-only, log-prob only: the actor CTAs alone (net_base 0, one net), as kin_ppo_grad_tc launches refresh_old_logp
+    kernel<<<dim3((unsigned)g, 1u, (unsigned)n_members), TCG_THREADS, sizeof(TcGradSmem<1>) + 1024, (cudaStream_t)stream>>>(
+        reinterpret_cast<const float*>(members), KinPpoHyper{}, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, tile_ids, n_pairs, 0.0f, nullptr, nullptr,
+        nullptr, 1, 0, nullptr, nullptr, none, 0);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_logp");
 }

@@ -49,11 +49,39 @@ struct RouteCollectOut {
     int boot_cap;
 };
 
-template <int TILES, bool SEQ>
+// POP (population launch, kin_pop_route_collect): the one extra argument carries the two member tables and the chunk offset t0; member
+// blockIdx.y's descriptors replace every other per-run argument (its reset window included) and its buffers are offset to row t0, the
+// step counter to first_step + t0 -- what a standalone trainer passes for that chunk.  P, R and reset_streak are shared.  A CTA holds
+// one tile of one member (TILES = 1), blockIdx.x is the member-local tile, so env indices and Philox streams are the standalone launch's.
+struct PopRouteCollect {
+    const KinPopMember* members;
+    const KinPopRouteMember* route_members;
+    int t0;
+};
+
+template <int TILES, bool SEQ, bool POP = false, class... PopArgs>
 __global__ void __launch_bounds__(TILES * AC_ROWS, 1)
-kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, const __grid_constant__ KinRouteResetParams C, float* __restrict__ state,
+kin_route_collect_kernel(const __grid_constant__ KinEnvParams P, RouteView R, const __grid_constant__ KinRouteResetParams C_arg, float* __restrict__ state,
                          int stride, int n, const float* __restrict__ params, int T, uint64_t noise_seed, uint32_t step0, uint64_t reset_seed,
-                         int reset_streak, RouteCollectOut out) {
+                         int reset_streak, RouteCollectOut out, const __grid_constant__ PopArgs... pop) {
+    static_assert(sizeof...(PopArgs) == (POP ? 1 : 0) && (!POP || TILES == 1), "population: one extra argument, a CTA never mixes members");
+    const KinRouteResetParams* Cp = &C_arg;
+    if constexpr (POP) {
+        const PopRouteCollect& A = (pop, ...);
+        const KinPopMember& M = A.members[blockIdx.y];
+        const KinPopRouteMember& RM = A.route_members[blockIdx.y];
+        const size_t r0 = (size_t)A.t0 * n;
+        Cp = &RM.reset;
+        state = M.state;
+        stride = M.stride;
+        params = M.params;
+        noise_seed = M.noise_seed;
+        step0 = M.first_step + (uint32_t)A.t0;
+        reset_seed = M.reset_seed;
+        out = RouteCollectOut{RM.obs + r0 * RC_IN, M.action + r0 * NJ, M.logp + r0, M.value + r0, M.reward + r0, M.done + r0, M.episode_start + r0,
+                              RM.route_flags + r0, M.start_io, M.last_value, M.boot_count, M.boot_index, M.boot_obs, M.boot_cap};
+    }
+    const KinRouteResetParams& C = *Cp;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     RouteCollectSmem<TILES>& S = *reinterpret_cast<RouteCollectSmem<TILES>*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
     const int tid = threadIdx.x;
@@ -187,4 +215,25 @@ extern "C" int kin_route_collect(void* handle, const KinRouteTable* host_route, 
     else if (tiles == 4) e = launch_route_collect<4>(h, R, *host_reset, state, stride, n_envs, params, n_steps, noise_seed, first_step, reset_seed, sequence_mode, reset_ready_streak_on_advance, out, st);
     else return kin_fail(KIN_ERR_INVALID_ARG, "kin_route_collect: tiles_per_cta must be 0 (auto), 1, 2 or 4");
     return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_route_collect");
+}
+
+extern "C" int kin_pop_route_collect(void* handle, const KinRouteTable* host_route, const KinPopMember* members, const KinPopRouteMember* route_members,
+                                     int n_members, int n_envs, int n_steps, int t0, int sequence_mode, int reset_ready_streak_on_advance, void* stream) {
+    KinHandle* h = kin_handle(handle);
+    if (!h || !route_ok(host_route)) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_collect: bad handle or route table");
+    if (!members || !route_members || n_members <= 0 || n_members > KIN_POP_MAX || n_steps <= 0 || t0 < 0)
+        return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_collect: need device member tables, 1 <= n_members <= KIN_POP_MAX, n_steps > 0 and t0 >= 0");
+    if (n_envs <= 0 || (n_envs % AC_ROWS) != 0) return kin_fail(KIN_ERR_INVALID_ARG, "kin_pop_route_collect: n_envs must be a positive multiple of 128 (one GEMM tile)");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = pop_zero_boot_counts(members, n_members, st);      // kin_route_collect's reset of *boot_count
+    if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_route_collect: zero counts");
+    auto kernel = sequence_mode ? kin_route_collect_kernel<1, true, true, PopRouteCollect> : kin_route_collect_kernel<1, false, true, PopRouteCollect>;
+    const size_t smem = sizeof(RouteCollectSmem<1>) + 1024;
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return kin_fail_cuda(e, "kin_pop_route_collect: smem attribute");
+    kernel<<<dim3((unsigned)(n_envs / AC_ROWS), (unsigned)n_members), AC_ROWS, smem, st>>>(h->params, view_of(host_route), KinRouteResetParams{}, nullptr, 0,
+                                                                                          n_envs, nullptr, n_steps, 0, 0u, 0, reset_ready_streak_on_advance,
+                                                                                          RouteCollectOut{}, PopRouteCollect{members, route_members, t0});
+    e = cudaGetLastError();
+    return e == cudaSuccess ? KIN_OK : kin_fail_cuda(e, "kin_pop_route_collect");
 }

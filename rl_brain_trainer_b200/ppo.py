@@ -369,17 +369,11 @@ class PPOTrainer:
         chunk starts, so a promotion widens the reset window at most ``route_chunk_steps`` steps after the step that triggered it
         (the reference's callback widens it at that very step, route/route_curriculum.py:85-99; chunk 1 reproduces that)."""
         L, env, hp = self._L, self.env, self.hp
-        done_bits = _D("KIN_DONE_TERMINATED") | _D("KIN_DONE_TRUNCATED")
-        if not hasattr(self, "_route_raw"):
-            self._route_raw = torch.zeros((self.T, self.N), dtype=torch.int32, device=self.device)
-        chunk = self.T if self.route_curriculum is None else max(1, min(int(self.route_chunk_steps), self.T))
         seq = env.sequence is not None
-        episodes = successes = 0.0
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream(self.device).cuda_stream
             t0 = 0
-            while t0 < self.T:
-                tc = min(chunk, self.T - t0)
+            for tc in self._route_chunks():
                 _lib.check(L.kin_route_collect(
                     env._params.handle, ctypes.byref(env.table.c), ctypes.byref(env._reset_params()), env.state.data_ptr(), env.stride, self.N,
                     self.params.data_ptr(), tc, self.seed, self.global_step, self.seed ^ 0x5EED, int(seq),
@@ -390,26 +384,52 @@ class PPOTrainer:
                 # time-limit episodes of this chunk: r += gamma * V(terminal observation); indices are relative to the chunk's first row
                 _lib.check(L.kin_ppo_bootstrap_list(self.params.data_ptr(), 80, self.boot_obs.data_ptr(), self.boot_index.data_ptr(), self.boot_count.data_ptr(),
                                                     self.boot_cap, self.rew_buf[t0].data_ptr(), float(hp.gamma), stream))
-                self.global_step += tc
-                if self.route_curriculum is not None:
-                    d, raw = self.done_buf[t0:t0 + tc], self._route_raw[t0:t0 + tc]
-                    fin = (d & done_bits) != 0
-                    flags = torch.stack([fin, (d & _D("KIN_DONE_SUCCESS")) != 0, (raw & 1) != 0, (raw & 4) != 0, (raw & 2) != 0], dim=1).cpu().numpy()
-                    promoted = False
-                    for t in range(tc):
-                        ids = np.nonzero(flags[t, 0])[0]
-                        if ids.size:
-                            promoted |= self.route_curriculum.record(flags[t, 1, ids], flags[t, 2, ids], flags[t, 3, ids], flags[t, 4, ids],
-                                                                    total_timesteps=self.num_timesteps + (t0 + t + 1) * self.N * self.world)
-                    if promoted:
-                        env.set_route_window(max_route_index=self.route_curriculum.prefix_end_index)
-                if int(self.boot_count.item()) > self.boot_cap:
-                    raise _lib.KinError("TimeLimit bootstrap list overflow in the fused route collection: rebuild the trainer")
+                flags = self._route_chunk_flags(t0, tc).cpu().numpy() if self.route_curriculum is not None else None
+                self._route_chunk_done(t0, tc, flags, int(self.boot_count.item()))
                 t0 += tc
             _lib.check(L.kin_ppo_gae(self.rew_buf.data_ptr(), self.val_buf.data_ptr(), self.start_buf.data_ptr(), self.last_val.data_ptr(),
                                      self.done_buf[self.T - 1].data_ptr(), float(hp.gamma), float(hp.gae_lambda), self.T, self.N,
                                      self.adv_buf.data_ptr(), self.ret_buf.data_ptr(), self.tile_sums.data_ptr(), stream))
-            env.obs.copy_(self.obs_buf[self.T])
+        return self._finish_route_collect()
+
+    # Host bookkeeping of the fused route collection, shared by this trainer's own launches and a ``PPOPopulation``'s.
+    def _route_chunks(self) -> list[int]:
+        """Step counts of the collection launches of one rollout: the whole rollout, or ``route_chunk_steps`` per launch under a prefix
+        curriculum."""
+        if not hasattr(self, "_route_raw"):
+            self._route_raw = torch.zeros((self.T, self.N), dtype=torch.int32, device=self.device)      # KIN_RAUX_FLAGS word per step
+        chunk = self.T if self.route_curriculum is None else max(1, min(int(self.route_chunk_steps), self.T))
+        return [min(chunk, self.T - t0) for t0 in range(0, self.T, chunk)]
+
+    def _route_chunk_flags(self, t0: int, tc: int) -> torch.Tensor:
+        """[tc, 5, N] bool on the device for steps t0 .. t0 + tc: finished, success, route_ready, orientation_hit, regression."""
+        d, raw = self.done_buf[t0:t0 + tc], self._route_raw[t0:t0 + tc]
+        fin = (d & (_D("KIN_DONE_TERMINATED") | _D("KIN_DONE_TRUNCATED"))) != 0
+        return torch.stack([fin, (d & _D("KIN_DONE_SUCCESS")) != 0, (raw & 1) != 0, (raw & 4) != 0, (raw & 2) != 0], dim=1)
+
+    def _route_chunk_done(self, t0: int, tc: int, flags: np.ndarray | None, boot_count: int) -> bool:
+        """After the chunk of steps t0 .. t0 + tc: advance the step counter, feed the chunk's finished episodes to the prefix curriculum in
+        time order (``flags``: ``_route_chunk_flags`` on the host), widen the reset window on a promotion and check the bootstrap list.
+        Returns True when the window changed."""
+        self.global_step += tc
+        promoted = False
+        if self.route_curriculum is not None:
+            for t in range(tc):
+                ids = np.nonzero(flags[t, 0])[0]
+                if ids.size:
+                    promoted |= self.route_curriculum.record(flags[t, 1, ids], flags[t, 2, ids], flags[t, 3, ids], flags[t, 4, ids],
+                                                            total_timesteps=self.num_timesteps + (t0 + t + 1) * self.N * self.world)
+            if promoted:
+                self.env.set_route_window(max_route_index=self.route_curriculum.prefix_end_index)
+        if boot_count > self.boot_cap:
+            raise _lib.KinError("TimeLimit bootstrap list overflow in the fused route collection: rebuild the trainer")
+        return promoted
+
+    def _finish_route_collect(self) -> dict[str, float]:
+        """After the last chunk and GAE: the env's observation, the rollout's episode outcomes, ``num_timesteps`` and ``last_rollout``."""
+        done_bits = _D("KIN_DONE_TERMINATED") | _D("KIN_DONE_TRUNCATED")
+        with torch.cuda.device(self.device):
+            self.env.obs.copy_(self.obs_buf[self.T])
         finished = (self.done_buf & done_bits) != 0
         succ = ((self.done_buf & _D("KIN_DONE_SUCCESS")) != 0) & finished
         self._finished, self._success = finished, succ

@@ -1,9 +1,12 @@
 """Population vs standalone PPO training at the reference's own small-batch shape.
 
-  python tools/population_bench.py [--members 1 8 32] [--iters 5]
+  python tools/population_bench.py [--route] [--members 1 8 32] [--iters 5]
 
 Every member: 128 envs x 256 steps (the 32 768 samples of 16 x 2048), batch_size 512, 8 epochs, approach_dynamic_scale_big's
-learning rate / clip / entropy / gamma / lambda, Stage 10.  For each K it times, per iteration (collect + update):
+learning rate / clip / entropy / gamma / lambda, Stage 10.  With --route every member trains the 80-input route policy at the
+route_prefix120 shape instead: 128 envs x 128 steps (the 16 384 samples of 16 x 1024), batch_size 512, 6 epochs, the preset's
+learning rate / clip / entropy / gamma / lambda, the synthetic 483-waypoint route and the sequence wrapper, no prefix curriculum (one
+collection launch per rollout).  For each K it times, per iteration (collect + update):
   (a) a PPOPopulation of K members, (b) one standalone PPOTrainer with a member's arguments, (c) K members one after another = K x (b).
 Device work is timed with CUDA events and a synchronise; one warm-up iteration of each is excluded; population and standalone
 iterations alternate in the same process and the median over --iters is reported.  Prints one JSON line.
@@ -25,7 +28,8 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--members", type=int, nargs="+", default=[1, 8, 32])
 ap.add_argument("--iters", type=int, default=5)
 ap.add_argument("--envs", type=int, default=128)
-ap.add_argument("--n-steps", type=int, default=256)
+ap.add_argument("--n-steps", type=int, default=None, help="default 256, or 128 with --route")
+ap.add_argument("--route", action="store_true", help="route_prefix120 route members instead of Approach members")
 ap.add_argument("--stage", type=int, default=10)
 a = ap.parse_args()
 if not torch.cuda.is_available():
@@ -45,13 +49,24 @@ def device_info() -> dict:
     return info
 
 
-cfg = kcfg.load_preset("approach_dynamic_scale_big")
-ref = kcfg.preset_dict("approach_dynamic_scale_big")["algorithms"]["ppo"]
+a.n_steps = a.n_steps or (128 if a.route else 256)
+preset = "route_prefix120" if a.route else "approach_dynamic_scale_big"
+ref = kcfg.preset_dict(preset)["algorithms"]["ppo"]
+if a.route:
+    from rl_brain_trainer_b200.route import synthetic_route
+
+    route = synthetic_route(483, seed=7)
+    cfg, seq = kcfg.to_route_env_config(kcfg.preset_dict(preset), max_route_index=len(route) - 1)
+else:
+    cfg = kcfg.load_preset(preset)
 hp = dict(learning_rate=ref["learning_rate"], n_steps=a.n_steps, batch_size=ref["batch_size"], n_epochs=ref["n_epochs"], gamma=ref["gamma"],
           gae_lambda=ref["gae_lambda"], clip_range=ref["clip_range"], ent_coef=ref["ent_coef"])
 
 
 def trainer(seed: int) -> ppo.PPOTrainer:
+    if a.route:
+        return ppo.PPOTrainer(cfg, ppo.random_policy(80, seed=seed, log_std_init=-1.0, device=dev), num_envs=a.envs, hyper=ppo.PPOHyper(**hp),
+                              device=dev, seed=seed, route=route, route_sequence_config=seq)
     return ppo.PPOTrainer(cfg, ppo.random_policy(56, seed=seed, log_std_init=-1.0, device=dev), num_envs=a.envs, hyper=ppo.PPOHyper(**hp), device=dev,
                           seed=seed, stage_index=a.stage)
 
@@ -69,8 +84,9 @@ def timed(collect, update) -> tuple[float, float]:
 
 
 S = a.envs * a.n_steps
-result = {"bench": "population", **device_info(), "envs_per_member": a.envs, "n_steps": a.n_steps, "batch_size": hp["batch_size"],
-          "n_epochs": hp["n_epochs"], "stage": a.stage, "iters": a.iters, "results": []}
+result = {"bench": "route_population" if a.route else "population", **device_info(), "envs_per_member": a.envs, "n_steps": a.n_steps,
+          "batch_size": hp["batch_size"], "n_epochs": hp["n_epochs"], **({"preset": preset, "waypoints": len(route)} if a.route else {"stage": a.stage}),
+          "iters": a.iters, "results": []}
 for K in a.members:
     pop = PPOPopulation([trainer(1000 + k) for k in range(K)])
     alone = trainer(1000)
